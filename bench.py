@@ -90,7 +90,18 @@ def parse_args():
                     help="N > 1: sites = one site shard per GPU (the north-star layout: one all-reduce per "
                          "evaluation batch); roots = a replica per GPU, root placements in chunks; auto = fewest "
                          "site shards that fit HBM, rest over root placements (exhaustive mode's rule)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step computed to DIR/<name>.npy (float64): logl_root0 (the "
+                         "full evaluation at root 0) and placement_logl (all 2n-3 placements, in root-id order); "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir: str, **arrays):
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / (name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def peaks():
@@ -451,6 +462,8 @@ def run_ours(args):
         lh0, sweep_lh = step()
     ev1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, logl_root0=np.array([lh0]), placement_logl=sweep_lh)
     ms = ev0.elapsed_time(ev1)
     st = g.stats()
     g.set_timing(False)

@@ -1,8 +1,8 @@
-// lbfgsb_driver.cpp -- binds the reference's own L-BFGS-B 3.0 (lib/lbfgsb,
-// setulb(): lbfgsb.c:44) at run time.  The C sources stay in the reference
-// tree; lib/liblbfgsb.so is compiled from them by root_digger_b200/_build.py
-// and loaded here from the directory of this library.  There is no substitute
-// optimiser: if the library is missing, parameter optimisation fails loudly.
+// lbfgsb_driver.cpp -- binds L-BFGS-B 3.0 (setulb(), root_digger_b200/lbfgsb/lbfgsb.c,
+// the interface of the C translation RootDigger vendors under lib/lbfgsb) at run time:
+// lib/liblbfgsb.so is compiled by root_digger_b200/_build.py and loaded here from the
+// directory of this library.  There is no substitute optimiser: if the library is
+// missing, parameter optimisation fails loudly.
 #include "lbfgsb_driver.hpp"
 
 #include <dlfcn.h>
@@ -35,7 +35,7 @@ setulb_fn load_setulb() {
     h = dlopen(c.c_str(), RTLD_NOW | RTLD_LOCAL);
     if (h) break;
   }
-  if (!h) throw std::runtime_error("liblbfgsb.so (the reference's lib/lbfgsb) could not be loaded");
+  if (!h) throw std::runtime_error("liblbfgsb.so (L-BFGS-B 3.0) could not be loaded");
   g_setulb = (setulb_fn)dlsym(h, "setulb");
   if (!g_setulb) throw std::runtime_error("setulb not found in liblbfgsb.so");
   return g_setulb;

@@ -1,7 +1,7 @@
 #ifndef RD_HOST_LBFGSB_DRIVER_HPP_
 #define RD_HOST_LBFGSB_DRIVER_HPP_
 namespace rd {
-// signature of setulb in the reference's lib/lbfgsb/lbfgsb.h (logical == int)
+// signature of setulb (root_digger_b200/lbfgsb/lbfgsb.c; RootDigger's lib/lbfgsb/lbfgsb.h, logical == int)
 typedef int (*setulb_fn)(int *n, int *m, double *x, double *l, double *u, int *nbd, double *f, double *g,
                          double *factr, double *pgtol, double *wa, int *iwa, int *task, int *iprint,
                          int *csave, int *lsave, int *isave, double *dsave);

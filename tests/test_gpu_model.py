@@ -159,3 +159,38 @@ def test_batched_root_only_evaluations_on_the_engine(libs):
     c = g.probe_counters()
     assert c["fused_batches"] > 0 and c["fused_evaluations"] >= 2 * c["fused_batches"]
     g.close()
+
+
+# bench.py's exhaustive-mode sample (cfg2: 500 taxa x 100 000 sites, UNREST+G4, root branch 0 optimised to
+# convergence) as recorded on a B200 with RootDigger's own vendored L-BFGS-B (lib/lbfgsb) linked into the host:
+# profiles/r02_bench_final2_n1.json, e2e.exhaustive.  Thousands of L-BFGS-B steps lead to this value, so
+# its bits and the number of root evaluations pin the optimiser's trajectory.
+RECORDED_EXHAUSTIVE_BEST_LLH = -9474150.440101244
+RECORDED_EXHAUSTIVE_ROOT_EVALUATIONS = 57553
+
+
+def test_exhaustive_branch_reproduces_the_run_recorded_with_the_reference_lbfgsb():
+    import ctypes as C
+    from cases import Case
+    case = Case(500, 100000, 4, seed=0x5EED0002, data="evolved", alpha=1.0, gamma_cats=capi.gamma_cats)
+    m = capi.Model(capi.RootedTree(case.newick), case.aln, 4)
+    m.initialize_partitions()
+    m.set_params(rates=case.rates, freqs=case.freqs)
+    m.set_sweep_mode(m.SWEEP_DIRECTED)
+    m.compute_lh(0, 0.5)
+    m.sweep_root_lh()
+    part = C.cast(m.L.rdh_model_partition(m.h, 0), C.POINTER(capi.PartitionStruct))
+    L = capi.load_engine()
+
+    def root_evals():
+        s = capi.Stats()
+        L.rdk_partition_stats(part, C.byref(s))
+        return s.asdict()["root_evals"]
+
+    before = root_evals()
+    ids, llh, _ = m.exhaustive_search(1e-7, 1e-7, 1e-12, 1e4, rank=0, num_tasks=m.root_count)
+    evaluations = root_evals() - before
+    m.close()
+    assert list(ids) == [0]
+    assert float(llh[0]).hex() == RECORDED_EXHAUSTIVE_BEST_LLH.hex()
+    assert evaluations == RECORDED_EXHAUSTIVE_ROOT_EVALUATIONS

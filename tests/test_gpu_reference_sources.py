@@ -1,7 +1,8 @@
 """tests/test_reference_sources.py on the CUDA engine: RootDigger's own src/model.cpp, src/tree.cpp,
 src/msa.cpp (unchanged, compiled against root_digger_b200/compat/corax/corax.h + librdk_b200.so) next
 to the engine host's model_t mirror (librd_host.so), both on cuda:0 through include/rdk.h: search with
-4 and 3 rate categories, exhaustive mode with its LWR inputs, every root of 101.phy -- bit for bit."""
+4 and 3 rate categories, exhaustive mode with its LWR inputs, every root of 101.phy -- bit for bit.
+Without a RootDigger checkout the reference's side is its recorded results (t.RecordedReference)."""
 import pytest
 
 import test_reference_sources as t
@@ -12,7 +13,7 @@ pytestmark = pytest.mark.gpu
 
 @pytest.fixture(scope="module")
 def ref():
-    return t.ReferenceBuild("engine")
+    return t.reference("engine")
 
 
 @pytest.fixture(scope="module")

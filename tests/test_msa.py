@@ -140,24 +140,16 @@ def test_the_reference_sources_read_every_form_through_the_compat_header(lib, ca
     """RootDigger's own src/msa.cpp, compiled unchanged against root_digger_b200/compat/corax/corax.h,
     reads each form through the compat readers (corax_phylip_parse_interleaved / _sequential,
     corax_fasta_getnext in compat/corax_compat.cpp) and its model_t gives, for every root, the bits
-    this repository's host gives for the same file"""
-    import ctypes as C
-    import os
-    from test_reference_sources import ReferenceBuild
-    ref = ReferenceBuild("oracle")  # skips when neither the checkout nor a built library is here
+    this repository's host gives for the same file.  Compared with the recorded results instead (no
+    checkout), neither msa.cpp nor the compat readers run: every form read by this host must then give
+    the reference's record of the fixture file."""
+    from test_reference_sources import reference
+    ref = reference("oracle")  # RootDigger's sources, else their recorded results (reported as a warning)
     fx, labels, seqs = case
-    dp = C.POINTER(C.c_double)
     for name, write in writers().items():
         path = tmp_path / (name + ".aln")
         path.write_text(write(labels, seqs), newline="")
-        h = ref.L.rdref_create(str(fx["tree_path"]).encode(), str(path).encode(), 2, 5, 1,
-                               os.path.join(str(tmp_path), "ref_" + name).encode())
-        assert h, (name, ref.L.rdref_last_error().decode())
-        h = C.c_void_p(h)
-        n = ref.L.rdref_root_count(h)
-        theirs = np.zeros(n)
-        ref.check(ref.L.rdref_all_root_lh(h, theirs.ctypes.data_as(dp), n))
-        ref.L.rdref_destroy(h)
+        theirs = ref.all_root_lh("10.fasta", 2, 5, alignment=path)
         m = model_from(lib, fx, path)
         ours = m.compute_all_root_lh()
         m.close()

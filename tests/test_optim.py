@@ -273,3 +273,60 @@ def test_minimize_in_box_is_the_reference_driver(lib, name, pgtol, factr):
     as_bits = lambda rows: [[bits(a) for a in r] for r in rows]  # noqa: E731
     assert calls == len(want_trace) and as_bits(seen) == as_bits(want_trace), name
     assert bits(f_end) == bits(want_f) and [bits(a) for a in x] == [bits(a) for a in want_x], name
+
+
+# ---------------------------------------------------------------------------------------------
+# setulb itself (root_digger_b200/lbfgsb) against an independent L-BFGS-B 3.0: scipy's
+# ---------------------------------------------------------------------------------------------
+def _rosenbrock(x):
+    f = np.sum(100.0 * (x[1:] - x[:-1] ** 2) ** 2 + (1.0 - x[:-1]) ** 2)
+    g = np.zeros_like(x)
+    g[:-1] = -400.0 * x[:-1] * (x[1:] - x[:-1] ** 2) - 2.0 * (1.0 - x[:-1])
+    g[1:] += 200.0 * (x[1:] - x[:-1] ** 2)
+    return f, g
+
+
+def _run_setulb(path, fg, x0, lo, hi, m, factr, pgtol):
+    """setulb driven to its end with the analytic gradient -> every point it asked f and g at"""
+    import ctypes as C
+    L = C.CDLL(str(path))
+    dp, ip = C.POINTER(C.c_double), C.POINTER(C.c_int)
+    L.setulb.argtypes = [ip, ip, dp, dp, dp, ip, dp, dp, dp, dp, dp, ip, ip, ip, ip, ip, ip, dp]
+    n = len(x0)
+    x, lower, upper = (C.c_double * n)(*x0), (C.c_double * n)(*([lo] * n)), (C.c_double * n)(*([hi] * n))
+    nbd, f, g = (C.c_int * n)(*([2] * n)), C.c_double(0.0), (C.c_double * n)()
+    wa, iwa = (C.c_double * (2 * m * n + 5 * n + 11 * m * m + 8 * m))(), (C.c_int * (3 * n))()
+    task, csave, iprint = C.c_int(bfgs_oracle.START), C.c_int(0), C.c_int(-1)
+    lsave, isave, dsave = (C.c_int * 4)(), (C.c_int * 44)(), (C.c_double * 29)()
+    n_c, m_c, factr_c, pgtol_c = C.c_int(n), C.c_int(m), C.c_double(factr), C.c_double(pgtol)
+    points = []
+    while True:
+        L.setulb(C.byref(n_c), C.byref(m_c), x, lower, upper, nbd, C.byref(f), g, C.byref(factr_c), C.byref(pgtol_c),
+                 wa, iwa, C.byref(task), C.byref(iprint), C.byref(csave), lsave, isave, dsave)
+        if bfgs_oracle.FG <= task.value <= bfgs_oracle.FG_END:
+            points.append(np.array(x[:]))
+            fv, gv = fg(points[-1])
+            f.value, g[:] = fv, gv.tolist()
+        elif task.value != bfgs_oracle.NEW_X:
+            return points
+
+
+@pytest.mark.parametrize("n,lo,hi,m,seed", [(2, -2.0, 2.0, 10, 1), (8, 0.2, 5.0, 20, 2), (12, 0.0, 0.9, 20, 3),
+                                            (25, -0.5, 2.0, 3, 4)])
+def test_setulb_follows_an_independent_lbfgsb(n, lo, hi, m, seed):
+    """bounded Rosenbrock from a seeded start: the same number of evaluations as scipy's L-BFGS-B and
+    the same points up to rounding (scipy sums through LAPACK / BLAS in another order)"""
+    optimize = pytest.importorskip("scipy.optimize")
+    from root_digger_b200 import _build
+    x0 = np.random.default_rng(seed).uniform(lo, hi, n)
+    ours = _run_setulb(_build.build_lbfgsb(), _rosenbrock, x0, lo, hi, m, 1e7, 1e-5)
+    theirs = []
+
+    def logged(x):
+        theirs.append(x.copy())
+        return _rosenbrock(x)
+
+    optimize.fmin_l_bfgs_b(logged, x0.copy(), bounds=[(lo, hi)] * n, m=m, factr=1e7, pgtol=1e-5, maxiter=10 ** 5,
+                           maxfun=10 ** 5)
+    assert len(ours) == len(theirs) > 5
+    assert max(np.max(np.abs(a - b)) for a, b in zip(ours, theirs)) < 1e-8
