@@ -58,23 +58,21 @@ def _run(cmd, **kw):
 PROGRAM_KS = (1, 2, 4, 8, 16, 32)  # rate-category counts the program kernel is instantiated for
 
 
-def build_engine(force: bool = False, verbose: bool = False, out: Path | None = None, defines=()) -> Path:
+def build_engine(force: bool = False, verbose: bool = False) -> Path:
     """nvcc -> lib/librdk_b200.so (sm_100a, -lineinfo).  The ABI, the host math and one
     translation unit per rate-category count (rdk_program_inst.cu, -DRDK_INST_K=K) are compiled
     in parallel and linked into one shared library."""
     from concurrent.futures import ThreadPoolExecutor
 
     LIBDIR.mkdir(exist_ok=True)
-    out = Path(out) if out else LIBDIR / "librdk_b200.so"
-    out.parent.mkdir(parents=True, exist_ok=True)
+    out = LIBDIR / "librdk_b200.so"
     srcs = [CSRC / "rdk_abi.cu", CSRC / "rdk_host_math.cpp", CSRC / "rdk_lower_debug.cpp", CSRC / "rdk_program_inst.cu"]
     deps = srcs + [CSRC / "rdk_kernels.cuh", CSRC / "rdk_lower.hpp", INCLUDE / "rdk.h"]
     if not force and _newer(out, deps):
         return out
-    objdir = out.parent / ("obj_" + out.stem)
+    objdir = LIBDIR / "obj_librdk_b200"
     objdir.mkdir(exist_ok=True)
-    defs = ["-D" + d for d in list(defines) + os.environ.get("RDK_NVCC_DEFINES", "").split()]  # experiment switches
-    base = [_nvcc(), *defs, *NVCC_ARCH, "-lineinfo", "-O3", "-std=c++17", "--fmad=false", "-ccbin", _cxx(),
+    base = [_nvcc(), *NVCC_ARCH, "-lineinfo", "-O3", "-std=c++17", "--fmad=false", "-ccbin", _cxx(),
             "-Xcompiler", "-fPIC,-ffp-contract=off,-Wall", "-I", INCLUDE]
     if verbose:
         base.insert(1, "-Xptxas=-v")
@@ -83,8 +81,6 @@ def build_engine(force: bool = False, verbose: bool = False, out: Path | None = 
             (base + ["-c", CSRC / "rdk_lower_debug.cpp", "-o", objdir / "rdk_lower_debug.o"])]
     for k in PROGRAM_KS:
         jobs.append(base + ["-DRDK_INST_K=%d" % k, "-c", CSRC / "rdk_program_inst.cu", "-o", objdir / ("rdk_program_k%d.o" % k)])
-    # heaviest translation units first (K = 4 carries the optional per-kind copies)
-    jobs.sort(key=lambda c: 0 if any(str(x) == "-DRDK_INST_K=4" for x in c) else 1)
     with ThreadPoolExecutor(max_workers=max(1, min(len(jobs), os.cpu_count() or 1))) as pool:
         logs = list(pool.map(_run, jobs))
     objs = [j[-1] for j in jobs]

@@ -82,7 +82,8 @@ def _ptr(a, t):
 
 def engine_lib_path() -> Path:
     import os
-    override = os.environ.get("RDK_ENGINE_LIB")  # kernel experiments: a variant build of the same ABI
+    # another build of the same ABI, e.g. the parent commit's, to compare outputs (bench.py --dump-outputs)
+    override = os.environ.get("RDK_ENGINE_LIB")
     return Path(override) if override else _build.LIBDIR / "librdk_b200.so"
 
 

@@ -212,7 +212,6 @@ struct Engine {
   };
   std::vector<KeptProgram> kept_programs;
   unsigned long long       kept_clock = 0;
-  bool                     keep_programs = true;
 
   // launch config
   int ctas_per_sm = 0, threads = 0, elems = 0;
@@ -765,7 +764,7 @@ int flush(rdk_partition_t *p) {
   for (size_t i = 0; i < e->pend_prog.size(); ++i) e->pend_prog[i].id = (unsigned)i;
   Engine::KeptProgram  scratch_entry;  // programs that are not kept are lowered into this one
   Engine::KeptProgram *kp = nullptr;
-  const bool           keepable = e->keep_programs && e->pend_prog.size() >= kKeptMinOps;
+  const bool           keepable = e->pend_prog.size() >= kKeptMinOps;
   if (keepable) kp = find_kept_program(e, lazy, chunked);
   if (kp) {
     e->stats.programs_reused++;
@@ -1048,7 +1047,6 @@ static int engine_init(rdk_partition_t *p, Engine *e) {
   e->clv_buffers = p->clv_buffers;
   e->S = p->sites;
   if (const char *env = getenv("RDK_LAZY")) e->lazy_enabled = atoi(env) != 0;
-  if (const char *env = getenv("RDK_KEEP_PROGRAMS")) e->keep_programs = atoi(env) != 0;  // experiments
   if (const char *env = getenv("RDK_SUBTREE_GROUPS")) e->subtree_groups = std::max(0, std::min(kMaxChunks, atoi(env)));
   e->Kreal = p->rate_cats;
   e->K = 1;

@@ -17,37 +17,6 @@
 // by instruction issue and the half-rate fp64 pipe instead (DESIGN.md section 5.1).
 #pragma once
 #include <cuda_runtime.h>
-#ifndef RDK_L2_PREFETCH_DIST
-// > 0: while instruction j computes, the CLV operand of instruction j + DIST is pulled into L2
-// (prefetch.global.L2, no registers).  Measured on B200 (cfg2 step, distances 2 and 3): 8.46 ->
-// 9.0 ms -- the walk is not waiting on DRAM, the prefetches only take issue slots.  Off.
-#define RDK_L2_PREFETCH_DIST 0
-#endif
-// timing experiments only (tools/build_variant.sh): each removes one piece of the kernel -- the
-// results are WRONG when any is set
-#ifndef RDK_X_NOTABLES
-#define RDK_X_NOTABLES 0  // the producer moves no tables
-#endif
-#ifndef RDK_X_NOSTORE
-#define RDK_X_NOSTORE 0  // no CLV is stored
-#endif
-#ifndef RDK_X_NOLOAD
-#define RDK_X_NOLOAD 0  // the consumers load no CLV
-#endif
-#ifndef RDK_PRODUCER_SLEEP_NS
-// back-off of the producer warp while its ring is full (measured: 200 / 1000 / 4000 ns, no difference)
-#define RDK_PRODUCER_SLEEP_NS 200
-#endif
-#ifndef RDK_A_FIRST
-// 1: an instruction starts with the child-1 term (the operand LOADED for it), so that the loads
-//    of the next instruction's operand are issued before the child-2 mat-vec and everything
-//    after it -- the longest flight time a one-instruction look-ahead can give them; the result
-//    is then moved into v (8 E register moves).
-// 0: the child-2 term first (computed from v), the product lands directly in v; the next
-//    instruction's loads are issued only after both mat-vecs.
-// Measured on B200 (cfg2 step): 8.46 ms (1) against 8.69 ms (0).
-#define RDK_A_FIRST 1
-#endif
 #include "rdk_lower.hpp"
 #include <stdint.h>
 #include <type_traits>
@@ -516,12 +485,11 @@ struct ProgArgs {
 // the table ring of one CTA
 template <int K>
 struct Ring {
-#ifdef RDK_RING_DEPTH
-  static constexpr int      kDepth = RDK_RING_DEPTH;
-#else
+  // 8 slots, fewer for K = 16 / 32 so that the ring stays at about 66 KB of shared memory (a slot
+  // holds two K-sized tables); depths 4 / 8 / 16 measured the same on B200: the ring is not the
+  // limiter (DESIGN.md section 5.1)
   static constexpr int      kDepth = K <= 8 ? 8 : (K == 16 ? 4 : 2);
-#endif
-  static constexpr int      kLogDepth = kDepth == 16 ? 4 : (kDepth == 8 ? 3 : (kDepth == 4 ? 2 : 1));
+  static constexpr int      kLogDepth = kDepth == 8 ? 3 : (kDepth == 4 ? 2 : 1);
   static constexpr unsigned kTabBytes = kTabDoubles * K * 8;      // one child's table (the larger kind)
   static constexpr unsigned kPBytes = kPTabDoubles * K * 8;       // P of an inner child
   static constexpr unsigned kInstrBytes = 128;                    // the instruction, padded
@@ -549,9 +517,6 @@ __device__ __forceinline__ void st_clv(double* base, unsigned e, const d4& x) {
   asm volatile("st.global.cg.v4.f64 [%0], {%1,%2,%3,%4};\n" ::"l"(q), "d"(x.v[0]), "d"(x.v[1]), "d"(x.v[2]),
                "d"(x.v[3])
                : "memory");
-}
-__device__ __forceinline__ void prefetch_l2(const void* p) {
-  asm volatile("prefetch.global.L2 [%0];\n" ::"l"(p));
 }
 
 // ---- mbarrier + bulk async copy (one elected thread moves a whole table) ----
@@ -604,6 +569,9 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned by
 // 2^-256 is zero) -- the underflow test then runs on the integer pipe, not the fp64 pipe
 __device__ __forceinline__ int hi_word(double x) { return __double2hiint(x); }
 constexpr int kScaleThresholdHi = (1023 - 256) << 20;
+
+// back-off of the producer warp while its ring is full (200 / 1000 / 4000 ns measured the same on B200)
+constexpr unsigned kProducerSleepNs = 200;
 
 template <int K, int E, int MAXT, int MINB>
 __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_constant__ ProgArgs a) {
@@ -668,7 +636,7 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
           const unsigned s = j & (D - 1u);
           // the producer runs kDepth instructions ahead: it is nearly always waiting here, and a
           // busy wait would take issue slots from the consumer warps of its sub-partition
-          while (!mbar_try_wait(&s_empty[s], ((j >> R::kLogDepth) & 1u) ^ 1u)) __nanosleep(RDK_PRODUCER_SLEEP_NS);
+          while (!mbar_try_wait(&s_empty[s], ((j >> R::kLogDepth) & 1u) ^ 1u)) __nanosleep(kProducerSleepNs);
           unsigned char* slot = smem_raw + s * R::kSlotBytes;
           int4*          dst = reinterpret_cast<int4*>(slot);
           dst[0] = w0;
@@ -678,7 +646,7 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
           dst[4] = w4;
           const unsigned fl = (unsigned)w4.x;
           unsigned       b1 = 0, b2 = 0;
-          if (!(fl & (fLoadV | fNop)) && !RDK_X_NOTABLES) {
+          if (!(fl & (fLoadV | fNop))) {
             b1 = (fl & fTip1) ? R::kTabBytes : R::kPBytes;
             b2 = (fl & fTip2) ? R::kTabBytes : R::kPBytes;
           }
@@ -763,7 +731,7 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
         const unsigned char* t = reinterpret_cast<const unsigned char*>(in.c1);
 #pragma unroll
         for (int u = 0; u < E; ++u) m1[u] = __ldg(t + site[u]);
-      } else if (!(fl & fNop) && !RDK_X_NOLOAD) {
+      } else if (!(fl & fNop)) {
         const void* g = in.c1;
 #pragma unroll
         for (int u = 0; u < E; ++u) c1r[u] = ld_clv(g, e[u]);
@@ -920,8 +888,10 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
         cnt[u] = cnt1[u] + ((fl & fCnt2V) ? vcnt[u] : 0u);
       }
 
-#if RDK_A_FIRST
       // ---- phase 1: y = A(child 1); c1r / m1 are dead afterwards ---------------------------
+      // child-1 term first: its operands are dead before the second mat-vec, so the next
+      // instruction's loads fly longer; the other order measured 8.69 vs 8.46 ms on B200
+      // (DESIGN.md section 5.1)
       if (main_op) {
         if (fl & fTip1) {
 #pragma unroll
@@ -960,17 +930,6 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
       if (ii + 1 < n_instr) {
         wait_full(jg + 1);
         load_operands(*reinterpret_cast<const Instr*>(slot_of(jg + 1)));
-#if RDK_L2_PREFETCH_DIST > 1
-        if (ii + RDK_L2_PREFETCH_DIST < n_instr && RDK_L2_PREFETCH_DIST < (int)D) {
-          wait_full(jg + RDK_L2_PREFETCH_DIST);
-          const Instr& fx = *reinterpret_cast<const Instr*>(slot_of(jg + RDK_L2_PREFETCH_DIST));
-          if (!(fx.flags & (fTip1 | fNop))) {
-            const char* g = reinterpret_cast<const char*>(fx.c1);
-#pragma unroll
-            for (int u = 0; u < E; ++u) prefetch_l2(g + (size_t)e[u] * 32u);
-          }
-        }
-#endif
       }
 
       // ---- phase 2: r = y o B(child 2), in place ------------------------------------------
@@ -1009,7 +968,7 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
         if (keep_v) {
           evaluate(in, fl, y, cnt);
         } else {
-          if ((fl & fWrite) && !RDK_X_NOSTORE) {
+          if (fl & fWrite) {
             double* par = in.parent;
 #pragma unroll
             for (int u = 0; u < E; ++u) st_clv(par, e[u], y[u]);
@@ -1026,121 +985,6 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
           }
         }
       }
-#else
-      // ---- phase 1: y = B(child 2) ------------------------------------------------------
-      if (main_op) {
-        if (fl & fTip2) {
-#pragma unroll
-          for (int u = 0; u < E; ++u) {
-            const double2* t = reinterpret_cast<const double2*>(tab2 + (m2c[u] * K + k) * 32u);
-            const double2  lo = t[0], hi = t[1];
-            y[u].v[0] = lo.x;
-            y[u].v[1] = lo.y;
-            y[u].v[2] = hi.x;
-            y[u].v[3] = hi.y;
-          }
-        } else {
-          const double2* p = reinterpret_cast<const double2*>(tab2 + k * (kPTabDoubles * 8));
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const double2 p01 = p[i * 2], p23 = p[i * 2 + 1];
-#pragma unroll
-            for (int u = 0; u < E; ++u) {
-              double s = dmul(p01.x, v[u].v[0]);
-              s = dfma(p01.y, v[u].v[1], s);
-              s = dfma(p23.x, v[u].v[2], s);
-              s = dfma(p23.y, v[u].v[3], s);
-              y[u].v[i] = s;
-            }
-          }
-        }
-      }
-
-      // ---- phase 2: r = A(child 1) o y, into v (regular operation) or y (evaluation) -----
-      const bool keep_v = (fl & fEval) != 0;
-      if (main_op) {
-        if (fl & fTip1) {
-#pragma unroll
-          for (int u = 0; u < E; ++u) {
-            const double2* t = reinterpret_cast<const double2*>(tab1 + (m1[u] * K + k) * 32u);
-            const double2  lo = t[0], hi = t[1];
-            if (keep_v) {
-              y[u].v[0] = dmul(lo.x, y[u].v[0]);
-              y[u].v[1] = dmul(lo.y, y[u].v[1]);
-              y[u].v[2] = dmul(hi.x, y[u].v[2]);
-              y[u].v[3] = dmul(hi.y, y[u].v[3]);
-            } else {
-              v[u].v[0] = dmul(lo.x, y[u].v[0]);
-              v[u].v[1] = dmul(lo.y, y[u].v[1]);
-              v[u].v[2] = dmul(hi.x, y[u].v[2]);
-              v[u].v[3] = dmul(hi.y, y[u].v[3]);
-            }
-          }
-        } else {
-          const double2* p = reinterpret_cast<const double2*>(tab1 + k * (kPTabDoubles * 8));
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const double2 p01 = p[i * 2], p23 = p[i * 2 + 1];
-#pragma unroll
-            for (int u = 0; u < E; ++u) {
-              double s = dmul(p01.x, c1r[u].v[0]);
-              s = dfma(p01.y, c1r[u].v[1], s);
-              s = dfma(p23.x, c1r[u].v[2], s);
-              s = dfma(p23.y, c1r[u].v[3], s);
-              if (keep_v)
-                y[u].v[i] = dmul(s, y[u].v[i]);
-              else
-                v[u].v[i] = dmul(s, y[u].v[i]);
-            }
-          }
-        }
-      } else if (fl & fLoadV) {
-#pragma unroll
-        for (int u = 0; u < E; ++u) {
-          v[u] = c1r[u];
-          vcnt[u] = cnt1[u];
-        }
-      }
-
-      // ---- the operands of the next instruction of this pass (c1r, m1, cnt1 are dead now) ---
-      if (ii + 1 < n_instr) {
-        wait_full(jg + 1);
-        load_operands(*reinterpret_cast<const Instr*>(slot_of(jg + 1)));
-#if RDK_L2_PREFETCH_DIST > 1
-        if (ii + RDK_L2_PREFETCH_DIST < n_instr && RDK_L2_PREFETCH_DIST < (int)D) {
-          wait_full(jg + RDK_L2_PREFETCH_DIST);
-          const Instr& fx = *reinterpret_cast<const Instr*>(slot_of(jg + RDK_L2_PREFETCH_DIST));
-          if (!(fx.flags & (fTip1 | fNop))) {
-            const char* g = reinterpret_cast<const char*>(fx.c1);
-#pragma unroll
-            for (int u = 0; u < E; ++u) prefetch_l2(g + (size_t)e[u] * 32u);
-          }
-        }
-#endif
-      }
-
-      // ---- rescale, store, evaluate -----------------------------------------------------
-      if (main_op) {
-        if (keep_v) {
-          if (fl & fScale) rescale(y, cnt);
-          evaluate(in, fl, y, cnt);
-        } else {
-          if (fl & fScale) rescale(v, cnt);
-          if ((fl & fWrite) && !RDK_X_NOSTORE) {
-            double* par = in.parent;
-#pragma unroll
-            for (int u = 0; u < E; ++u) st_clv(par, e[u], v[u]);
-          }
-          if ((fl & fWriteS) && k == 0) {
-            unsigned* ps = in.pscale;
-#pragma unroll
-            for (int u = 0; u < E; ++u) __stcg(ps + site[u], cnt[u]);
-          }
-#pragma unroll
-          for (int u = 0; u < E; ++u) vcnt[u] = cnt[u];
-        }
-      }
-#endif
       if (fl & fEvalV) evaluate(in, fl, v, vcnt);
       if (ii + 1 < n_instr) load_v(*reinterpret_cast<const Instr*>(slot_of(jg + 1)));
       release(jg);
