@@ -397,6 +397,44 @@ int rdk_debug_choose_subtree_groups(unsigned int tips, unsigned int n_ops, const
                                     unsigned int sites, unsigned int rate_cats, int sm_count,
                                     unsigned int *longest, unsigned int *n_join);
 
+/* ---- root placement support (new; DESIGN.md section 10) ------------------- */
+/* Reserve a device matrix of `rows` x (local patterns) doubles that
+ * rdk_compute_root_loglikelihood_row fills (rows = 0 frees it). */
+int rdk_partition_set_site_lnl_rows(rdk_partition_t *partition, unsigned int rows);
+/* rdk_compute_root_loglikelihood, same value bit for bit, that also stores every pattern's
+ * UNWEIGHTED log-likelihood (the value before the pattern weight is applied) into row `row`. */
+double rdk_compute_root_loglikelihood_row(rdk_partition_t *partition, unsigned int clv_index,
+                                          int scaler_index, unsigned int row);
+/* copy rows [first, first + count) of that matrix to out ([count][local patterns]) */
+int rdk_partition_get_site_lnl_rows(rdk_partition_t *partition, unsigned int first,
+                                    unsigned int count, double *out);
+
+/* RELL bootstrap proportions and one-sided KH / SH tests over `rows` records whose per-pattern
+ * log-likelihoods L are rows 0..rows-1 of the site matrices of n partitions (all on one device),
+ * or of ONE site shard with a communicator attached (every rank makes the same call and gets the
+ * bits of one GPU); global_index[i] is partition i's global index (it keys the random draws).
+ * Fixed point q = rint(L * 2^exponent), exponent = 52 - frexp exponent of max |L|; replicate b
+ * draws, per partition g, N_g = sum of its weights sites with Philox4x64-10 keyed
+ * {seed, (g << 32) | b}; Z[b][r] = sum c * q and O[r] = sum w * q are exact (int128).
+ * Caller-owned arrays have `rows` entries. */
+typedef struct rdk_rell_out_t {
+  unsigned int        replicate_tile; /* in: replicates per counts tile, 0 = engine default */
+  int                 exponent;       /* out: e */
+  unsigned int        best;           /* out: argmax_r O[r], lowest index on ties */
+  unsigned int        bad_row;        /* out on failure: a record with a non-finite L, or ~0u */
+  double             *lnl_fixed;      /* out: O[r] * 2^-e rounded once */
+  unsigned long long *o_lo;           /* out (optional): O[r] as two's-complement int128, low word */
+  long long          *o_hi;           /* ... high word */
+  unsigned int       *bp_count;       /* out: #b whose argmax_r Z[b][r] is r */
+  unsigned int       *kh_count;       /* out: #b passing the centred KH test against best */
+  unsigned int       *sh_count;       /* out: #b passing the SH test */
+  double              ms[4];          /* out: device time of counts, accumulation, statistics, all */
+  unsigned long long  device_bytes;   /* out: device memory the call allocated (freed on return) */
+} rdk_rell_out_t;
+int rdk_rell_support(rdk_partition_t *const *partitions, unsigned int n,
+                     const unsigned int *global_index, unsigned int rows,
+                     unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out);
+
 #ifdef __cplusplus
 }
 #endif

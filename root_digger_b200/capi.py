@@ -157,6 +157,10 @@ def load_engine() -> C.CDLL:
     L.rdk_partition_set_lazy.argtypes = [_pp, C.c_int]
     L.rdk_partition_set_subtree_groups.argtypes = [_pp, C.c_int]
     L.rdk_set_device.argtypes = [C.c_int]
+    L.rdk_partition_set_site_lnl_rows.argtypes = [_pp, C.c_uint]
+    L.rdk_compute_root_loglikelihood_row.argtypes = [_pp, C.c_uint, C.c_int, C.c_uint]
+    L.rdk_compute_root_loglikelihood_row.restype = C.c_double
+    L.rdk_partition_get_site_lnl_rows.argtypes = [_pp, C.c_uint, C.c_uint, _dp]
     _engine_lib = L
     return L
 
@@ -270,6 +274,24 @@ class Partition:
         if persite:
             return v, ps
         return v
+
+    def set_site_lnl_rows(self, rows: int):
+        """reserve `rows` device rows of unweighted per-pattern log-likelihoods"""
+        if self.L.rdk_partition_set_site_lnl_rows(self.p, rows) != 1:
+            raise EngineError(_err(self.L))
+
+    def root_loglikelihood_row(self, clv_index: int, scaler_index: int, row: int) -> float:
+        """root_loglikelihood (same bits) that also stores the unweighted per-pattern values in `row`"""
+        v = self.L.rdk_compute_root_loglikelihood_row(self.p, clv_index, scaler_index, row)
+        if np.isnan(v):
+            raise EngineError(_err(self.L))
+        return v
+
+    def site_lnl_rows(self, first: int, count: int) -> np.ndarray:
+        out = np.zeros((count, self.sites))
+        if self.L.rdk_partition_get_site_lnl_rows(self.p, first, count, _ptr(out, _dp)) != 1:
+            raise EngineError(_err(self.L))
+        return out
 
     def root_loglikelihood_multi(self, root_op, branch_length_pairs):
         bl = np.ascontiguousarray(branch_length_pairs, dtype=np.float64).reshape(-1)
@@ -775,6 +797,10 @@ def _bind_model(L: C.CDLL):
     L.rdh_model_set_max_outer_iterations.restype = None
     L.rdh_model_last_partition_lh.argtypes = [vp, _dp, C.c_uint]
     L.rdh_model_last_sweep_partition_lh.argtypes = [vp, C.c_uint, _dp, C.c_uint]
+    L.rdh_model_placement_support.argtypes = [vp, C.c_char_p, ull, ull, C.c_uint, C.c_int, C.c_uint, C.POINTER(ull),
+                                              _dp, _dp, _dp, C.POINTER(ull), C.POINTER(C.c_longlong), _up, _up, _up,
+                                              C.POINTER(C.c_int), _up, _dp, _up]
+    L.rdh_model_site_lnl_rows.argtypes = [vp, C.c_uint, _dp, ull, _up, C.c_uint, C.POINTER(ull)]
     L.rdh_model_assign_indicies.argtypes = [vp, C.c_int, C.c_uint, C.c_double, C.c_uint, C.c_uint, C.c_int, _up,
                                             C.c_uint, _up]
     L._rdh_model_bound = True
@@ -1174,6 +1200,59 @@ class Model:
                                                      rank, num_tasks, self.STRATEGY[strategy], _ptr(out, _up),
                                                      len(out), C.byref(got)))
         return out[:got.value].tolist()
+
+    def placement_support(self, checkpoint_prefix: str | None = None, replicates: int = 10000, seed: int = 0,
+                          replicate_tile: int = 0, keep_rows: bool = False) -> dict:
+        """RELL bootstrap proportions and one-sided KH / SH tests of every placement recorded in
+        "<checkpoint_prefix>.ckp" (opened read-only; None: the model's own result log, e.g. of
+        exhaustive_search), from `replicates` (1..2^20) resamplings of the sites, each partition on
+        its own (DESIGN.md section 10).  Per record, in log order: root_id, alpha, llh (as recorded),
+        lnl_fixed, O (the exact fixed-point sum, Python ints), bp, p_kh, p_sh and their integer
+        counts; also exponent, best (record index), replicates and the timings.  The model's
+        parameters and root are unchanged afterwards; the tree's branches carry BP, pKH and pSH in
+        newick(True).  keep_rows keeps the per-pattern rows for site_lnl_rows.  On site shards
+        every rank calls it with the same arguments and gets the same result."""
+        prefix = checkpoint_prefix.encode() if checkpoint_prefix is not None else None
+        cap = 128
+        for attempt in range(2):
+            ids = np.zeros(cap, dtype=np.uint64)
+            alpha, llh, fixed = np.zeros(cap), np.zeros(cap), np.zeros(cap)
+            o_lo, o_hi = np.zeros(cap, dtype=np.uint64), np.zeros(cap, dtype=np.int64)
+            bp, kh, sh = (np.zeros(cap, dtype=np.uint32) for _ in range(3))
+            exponent, best, got = C.c_int(), C.c_uint(), C.c_uint()
+            info = np.zeros(6)
+            rc = self.L.rdh_model_placement_support(
+                self.h, prefix, int(replicates), int(seed) & ((1 << 64) - 1), int(replicate_tile),
+                1 if keep_rows else 0, cap, _ptr(ids, C.POINTER(C.c_ulonglong)), _ptr(alpha, _dp), _ptr(llh, _dp),
+                _ptr(fixed, _dp), _ptr(o_lo, C.POINTER(C.c_ulonglong)), _ptr(o_hi, C.POINTER(C.c_longlong)),
+                _ptr(bp, _up), _ptr(kh, _up), _ptr(sh, _up), C.byref(exponent), C.byref(best), _ptr(info, _dp),
+                C.byref(got))
+            if rc or attempt or got.value <= cap:
+                break
+            cap = got.value  # the log holds more records than the first buffers: nothing was computed
+        self._check(rc)
+        n = got.value
+        self._support_rows = n if keep_rows else 0
+        B = float(replicates)
+        O = [(int(h) << 64) | int(l) for l, h in zip(o_lo[:n], o_hi[:n])]
+        return {"root_id": ids[:n].copy(), "alpha": alpha[:n].copy(), "llh": llh[:n].copy(),
+                "lnl_fixed": fixed[:n].copy(), "O": O, "bp_count": bp[:n].copy(), "kh_count": kh[:n].copy(),
+                "sh_count": sh[:n].copy(), "bp": bp[:n] / B, "p_kh": kh[:n] / B, "p_sh": sh[:n] / B,
+                "exponent": exponent.value, "best": best.value, "replicates": int(replicates),
+                "capture_ms": info[0], "counts_ms": info[1], "accumulate_ms": info[2], "statistics_ms": info[3],
+                "resample_ms": info[4], "device_bytes": int(info[5])}
+
+    def site_lnl_rows(self, part: int = 0):
+        """(rows [record][pattern], pattern weights) of partition `part` from the last
+        placement_support(..., keep_rows=True)"""
+        P = self.sites(part)
+        rows = getattr(self, "_support_rows", 0)
+        buf = np.zeros(max(1, rows * P))
+        w = np.zeros(max(1, P), dtype=np.uint32)
+        n = C.c_ulonglong()
+        self._check(self.L.rdh_model_site_lnl_rows(self.h, part, _ptr(buf, _dp), len(buf), _ptr(w, _up), len(w),
+                                                   C.byref(n)))
+        return buf[:n.value].reshape(rows, P), w[:P].copy()
 
     def lwr(self, llh) -> np.ndarray:
         llh = np.ascontiguousarray(llh, dtype=np.float64)

@@ -9,6 +9,7 @@
 // CUDA call fails the entry point fails (RDK_FAILURE / NaN).
 #include "../../include/rdk.h"
 #include "rdk_kernels.cuh"
+#include "rdk_support.cuh"
 
 #include <dlfcn.h>
 
@@ -184,6 +185,9 @@ struct Engine {
   double *d_nodes = nullptr; // sharded: [slots][global_blocks]
   size_t  nodes_cap = 0;
   double *d_persite = nullptr;
+  double *d_rows = nullptr;    // [rows_cap][S]: unweighted per-pattern values (rdk_partition_set_site_lnl_rows)
+  unsigned rows_cap = 0;
+  double  *want_row = nullptr; // the row the next evaluation stores into, or null
   double *h_results = nullptr;  // pinned, device-visible
   size_t  results_cap = 0;      // doubles
 
@@ -751,7 +755,9 @@ int flush(rdk_partition_t *p) {
     if (!ensure_partials(e, e->pend_slots, a.partial_stride)) return RDK_FAILURE;
     a.partials = e->d_partials;
   }
-  a.persite = e->want_persite ? e->d_persite : nullptr;
+  // a row of unweighted values takes the place of the weighted per-site output (never both)
+  a.persite = e->want_row ? e->want_row : (e->want_persite ? e->d_persite : nullptr);
+  a.persite_unweighted = e->want_row != nullptr;
   // recorded operations -> the instructions the kernel walks (rdk_lower.hpp)
   HostTimer             lower_timer(&e->stats.host_lower_ns);  // lowering, pointer translation, enqueue
   const bool            chunked = e->pend_chunk_off.size() > 2;
@@ -1169,6 +1175,7 @@ extern "C" void rdk_partition_destroy(rdk_partition_t *p) {
     cudaFree(e->d_weights);
     cudaFree(e->d_hist);
     cudaFree(e->d_persite);
+    cudaFree(e->d_rows);
     cudaFree(e->d_pool);
     cudaFree(e->d_partials);
     cudaFree(e->d_nodes);
@@ -1330,10 +1337,9 @@ extern "C" void rdk_update_clvs(rdk_partition_t *p, const rdk_operation_t *ops, 
   }
 }
 
-extern "C" double rdk_compute_root_loglikelihood(rdk_partition_t *p, unsigned int clv_index,
-                                                 int scaler_index, const unsigned int *freqs_indices,
-                                                 double *persite_lnl) {
-  (void)freqs_indices;
+// rdk_compute_root_loglikelihood; `row` (device, [S]) optionally receives the unweighted values
+static double root_loglikelihood(rdk_partition_t *p, unsigned int clv_index, int scaler_index,
+                                 double *persite_lnl, double *row) {
   Engine *e = eng(p);
   const double nan = std::numeric_limits<double>::quiet_NaN();
   std::lock_guard<std::mutex> lk(e->mu);
@@ -1377,8 +1383,9 @@ extern "C" double rdk_compute_root_loglikelihood(rdk_partition_t *p, unsigned in
   e->pend_evals++;
   e->pend_slots = 1;
   e->want_persite = persite_lnl != nullptr;
+  e->want_row = row;
   // a traversal whose only requested result is this log-likelihood may keep its CLVs in registers
-  if (fused && !persite_lnl) {
+  if (fused && !persite_lnl && !row) {
     size_t writes = 0;
     for (const ROp &r : e->pend_prog) writes += (r.flags & rWrite) ? 1 : 0;
     e->pend_lazy_ok = writes >= 16;
@@ -1386,6 +1393,7 @@ extern "C" double rdk_compute_root_loglikelihood(rdk_partition_t *p, unsigned in
   int ok = flush(p);
   e->pend_slots = 0;
   e->want_persite = false;
+  e->want_row = nullptr;
   if (!ok) return nan;
   if (e->S == 0 && e->global_sites == 0) return 0.0;
   if (!finish_evals(p, 1)) return nan;
@@ -1398,6 +1406,97 @@ extern "C" double rdk_compute_root_loglikelihood(rdk_partition_t *p, unsigned in
     e->stats.d2h_bytes += sizeof(double) * e->S;
   }
   return e->h_results[0];
+}
+
+extern "C" double rdk_compute_root_loglikelihood(rdk_partition_t *p, unsigned int clv_index,
+                                                 int scaler_index, const unsigned int *freqs_indices,
+                                                 double *persite_lnl) {
+  (void)freqs_indices;
+  return root_loglikelihood(p, clv_index, scaler_index, persite_lnl, nullptr);
+}
+
+// ---------------------------------------------------------------------------
+// root placement support: per-pattern rows and the RELL statistics (rdk_support.cu)
+// ---------------------------------------------------------------------------
+extern "C" int rdk_partition_set_site_lnl_rows(rdk_partition_t *p, unsigned int rows) {
+  Engine *e = eng(p);
+  std::lock_guard<std::mutex> lk(e->mu);
+  CUDA_TRY(cudaSetDevice(e->device));
+  CUDA_TRY(cudaStreamSynchronize(e->stream));
+  if (e->d_rows) {
+    cudaFree(e->d_rows);
+    e->stats.device_bytes -= sizeof(double) * (size_t)e->rows_cap * std::max(1u, e->S);
+    e->d_rows = nullptr;
+    e->rows_cap = 0;
+  }
+  if (rows == 0) return RDK_SUCCESS;
+  if (!dev_alloc(e, (void **)&e->d_rows, sizeof(double) * (size_t)rows * std::max(1u, e->S))) return RDK_FAILURE;
+  e->rows_cap = rows;
+  return RDK_SUCCESS;
+}
+
+extern "C" double rdk_compute_root_loglikelihood_row(rdk_partition_t *p, unsigned int clv_index,
+                                                     int scaler_index, unsigned int row) {
+  Engine *e = eng(p);
+  if (row >= e->rows_cap) {
+    fail(RDK_ERROR_PARAM, "site row %u out of range (%u rows reserved)", row, e->rows_cap);
+    return std::numeric_limits<double>::quiet_NaN();
+  }
+  return root_loglikelihood(p, clv_index, scaler_index, nullptr, e->d_rows + (size_t)row * e->S);
+}
+
+extern "C" int rdk_partition_get_site_lnl_rows(rdk_partition_t *p, unsigned int first, unsigned int count,
+                                               double *out) {
+  Engine *e = eng(p);
+  if ((unsigned long long)first + count > e->rows_cap) return fail(RDK_ERROR_PARAM, "site rows out of range");
+  std::lock_guard<std::mutex> lk(e->mu);
+  CUDA_TRY(cudaSetDevice(e->device));
+  if (!flush(p)) return RDK_FAILURE;
+  CUDA_TRY(cudaMemcpyAsync(out, e->d_rows + (size_t)first * e->S, sizeof(double) * (size_t)count * e->S,
+                           cudaMemcpyDeviceToHost, e->stream));
+  CUDA_TRY(cudaStreamSynchronize(e->stream));
+  e->stats.d2h_bytes += sizeof(double) * (size_t)count * e->S;
+  return RDK_SUCCESS;
+}
+
+extern "C" int rdk_rell_support(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
+                                unsigned int rows, unsigned long long replicates, unsigned long long seed,
+                                rdk_rell_out_t *out) {
+  if (n == 0 || rows == 0) return fail(RDK_ERROR_PARAM, "rdk_rell_support: no partitions or no rows");
+  if (replicates == 0 || replicates > kRellMaxReplicates)
+    return fail(RDK_ERROR_PARAM, "rdk_rell_support: replicates must be in [1, 2^20]");
+  std::vector<RellPartition> rp(n);
+  RellShard                  shard;
+  const int                  device = eng(parts[0])->device;
+  for (unsigned i = 0; i < n; ++i) {
+    Engine *e = eng(parts[i]);
+    if (e->device != device) return fail(RDK_ERROR_PARAM, "rdk_rell_support: partitions on different devices");
+    if (e->comm) {
+      if (n != 1) return fail(RDK_ERROR_PARAM, "rdk_rell_support: a site shard must be the only partition");
+      shard.comm = e->comm;
+      shard.nranks = e->nranks;
+      shard.rank = e->rank;
+      shard.site_offset = e->site_offset;
+      shard.allreduce = g_nccl.AllReduce;
+    } else if (e->global_sites && (e->site_offset != 0 || e->S != e->global_sites)) {
+      return fail(RDK_ERROR_PARAM, "rdk_rell_support: a site shard needs a communicator (rdk_partition_attach_comm)");
+    }
+    if (e->rows_cap < rows) return fail(RDK_ERROR_PARAM, "rdk_rell_support: partition %u holds %u rows, %u asked",
+                                        i, e->rows_cap, rows);
+    std::lock_guard<std::mutex> lk(e->mu);
+    CUDA_TRY(cudaSetDevice(e->device));
+    if (!flush(parts[i])) return RDK_FAILURE;
+    CUDA_TRY(cudaStreamSynchronize(e->stream));
+    rp[i].rows = e->d_rows;
+    rp[i].weights = parts[i]->pattern_weights;
+    rp[i].patterns = e->S;
+    rp[i].global_index = global_index ? global_index[i] : i;
+  }
+  CUDA_TRY(cudaSetDevice(device));
+  char msg[256];
+  if (!rell_support(rp.data(), n, rows, replicates, seed, shard, out, msg, sizeof(msg)))
+    return fail(RDK_ERROR_CUDA, "%s", msg);
+  return RDK_SUCCESS;
 }
 
 // ---------------------------------------------------------------------------

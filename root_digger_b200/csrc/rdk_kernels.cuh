@@ -471,6 +471,7 @@ struct ProgArgs {
   double*         partials; // [slots][partial_stride], one value per warp iteration
   unsigned        partial_stride;
   double*         persite;  // optional, eval slot 0 only
+  unsigned        persite_unweighted;  // persite receives the values before the pattern weight
   double          pi[4];
   double          w[kMaxCats];
   // n_chunks > 1: the program is n_chunks INDEPENDENT sub-programs (chunk c = instructions
@@ -842,8 +843,9 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
         if (k < (unsigned)E && iw * SPW + sl <= last_site) {
           l = rd_log(x);
           if (fl & fEvalScaler) l = dadd(l, dmul((double)cn, RDK_LOG_SCALE_THRESHOLD));
-          l = dmul(l, (double)wg);
-          if (a.persite && eslot == 0) a.persite[st] = l;
+          const double lw = dmul(l, (double)wg);
+          if (a.persite && eslot == 0) a.persite[st] = a.persite_unweighted ? l : lw;
+          l = lw;
         }
         // canonical tree over the 32/K sites of a warp iteration (the lanes of equal k)
 #pragma unroll
@@ -856,8 +858,9 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
           if (k == 0 && it[u] * SPW + sl <= last_site) {
             l = rd_log(term[u]);
             if (fl & fEvalScaler) l = dadd(l, dmul((double)cnt[u], RDK_LOG_SCALE_THRESHOLD));
-            l = dmul(l, (double)wgt[u]);
-            if (a.persite && eslot == 0) a.persite[site[u]] = l;
+            const double lw = dmul(l, (double)wgt[u]);
+            if (a.persite && eslot == 0) a.persite[site[u]] = a.persite_unweighted ? l : lw;
+            l = lw;
           }
 #pragma unroll
           for (int off2 = 1; off2 < (int)SPW; off2 <<= 1) l = dadd(l, __shfl_xor_sync(0xffffffffu, l, off2 * K));

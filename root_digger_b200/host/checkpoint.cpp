@@ -222,12 +222,13 @@ void append_all(int fd, const std::string &s, const char *what) {
   }
 }
 
-// whole-file write lock, released (with an fsync) at scope exit (src/checkpoint.hpp:205-249)
+// whole-file write lock (a shared read lock on a read-only log), released (with an fsync) at scope
+// exit (src/checkpoint.hpp:205-249)
 class file_lock_t {
 public:
-  explicit file_lock_t(int fd) : _fd{fcntl(fd, F_DUPFD, 0)} {
+  explicit file_lock_t(int fd, short type = F_WRLCK) : _fd{fcntl(fd, F_DUPFD, 0)} {
     memset(&_fl, 0, sizeof(_fl));
-    _fl.l_type = F_WRLCK;
+    _fl.l_type = type;
     _fl.l_whence = SEEK_SET;
     if (_fd == -1 || fcntl(_fd, F_SETLKW, &_fl) == -1) {
       if (_fd != -1) close(_fd);
@@ -294,6 +295,16 @@ checkpoint_t::checkpoint_t(const std::string &prefix) {
   if (_file_descriptor == -1) throw std::runtime_error("Failed to open the checkpoint file");
 }
 
+checkpoint_t checkpoint_t::read_only(const std::string &prefix) {
+  checkpoint_t c;
+  c._checkpoint_filename = prefix + ".ckp";
+  c._file_descriptor = open(c._checkpoint_filename.c_str(), O_RDONLY);
+  if (c._file_descriptor == -1) throw std::runtime_error("no checkpoint " + c._checkpoint_filename);
+  c._existing_results = true;
+  c._read_only = true;
+  return c;
+}
+
 checkpoint_t::~checkpoint_t() {
   if (_file_descriptor != -1) close(_file_descriptor);
 }
@@ -307,6 +318,7 @@ checkpoint_t &checkpoint_t::operator=(checkpoint_t &&o) {
   o._file_descriptor = -1;
   _checkpoint_filename = std::move(o._checkpoint_filename);
   _existing_results = o._existing_results;
+  _read_only = o._read_only;
   _records = std::move(o._records);
   return *this;
 }
@@ -351,7 +363,7 @@ void checkpoint_t::load_options_unlocked(cli_options_t &options) {
 
 // every readable record, in file order; *damaged = the log ends in a record that fails its checksum
 std::vector<checkpoint_t::record_t> checkpoint_t::scan(bool *damaged) {
-  file_lock_t lock(_file_descriptor);
+  file_lock_t lock(_file_descriptor, _read_only ? F_RDLCK : F_WRLCK);
   return scan_unlocked(damaged);
 }
 

@@ -62,6 +62,9 @@ public:
 
   checkpoint_t();                                    // in-memory
   explicit checkpoint_t(const std::string &prefix);  // "<prefix>.ckp", created if absent
+  // an existing "<prefix>.ckp" opened for reading only (read_results under a shared lock); for
+  // callers that only evaluate a log, possibly one they may not write (another user's run)
+  static checkpoint_t read_only(const std::string &prefix);
   ~checkpoint_t();
   checkpoint_t(checkpoint_t &&);
   checkpoint_t &operator=(checkpoint_t &&);
@@ -93,6 +96,7 @@ private:
   std::string           _checkpoint_filename;
   int                   _file_descriptor = -1;
   bool                  _existing_results = false;
+  bool                  _read_only = false;
   std::vector<record_t> _records;  // in-memory backing
   std::mutex            _mu;
 };

@@ -19,7 +19,12 @@
 //     chunks; partitions may be sharded over GPUs (shard_spec_t) and report their terms.
 #include "model.hpp"
 
+#ifdef RD_BACKEND_ORACLE
+#include "rdk_support.h"  // tests/oracle_shim: the placement-support entries over the CPU oracle
+#endif
+
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <exception>
 #include <cstdlib>
@@ -938,6 +943,169 @@ std::pair<root_location_t, double> model_t::exhaustive_search(double atol, doubl
     }
   }
   return best;
+}
+
+// ---------------------------------------------------------------------------
+// root placement support (DESIGN.md section 10)
+// ---------------------------------------------------------------------------
+model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
+                                                        unsigned replicate_tile, bool keep_rows) {
+  if (_exchange)
+    throw std::invalid_argument("placement_support: a model whose partitions are dealt to several processes is "
+                                "not supported");
+  if (replicates == 0 || replicates > (size_t(1) << 20))
+    throw std::invalid_argument("placement_support: replicates must be between 1 and 2^20");
+  const auto records = checkpoint.read_results();
+  if (records.empty()) throw std::invalid_argument("placement_support: the checkpoint holds no records");
+  if (records.size() > std::numeric_limits<unsigned>::max())
+    throw std::invalid_argument("placement_support: too many records");
+  for (size_t r = 0; r < records.size(); ++r) {
+    const auto &rec = records[r];
+    const std::string which = "placement_support: record " + std::to_string(r) + " (root id " +
+                              std::to_string(rec.first.root_id) + ")";
+    if (rec.first.root_id >= _tree.root_count()) throw std::invalid_argument(which + ": root id out of range");
+    if (!(rec.first.alpha >= 0.0 && rec.first.alpha <= 1.0))
+      throw std::invalid_argument(which + ": root position outside [0, 1]");
+    if (rec.second.size() != _partitions.size())
+      throw std::invalid_argument(which + ": " + std::to_string(rec.second.size()) + " parameter sets for " +
+                                  std::to_string(_partitions.size()) + " partitions");
+    for (size_t p = 0; p < _partitions.size(); ++p) {
+      const auto    &pp = rec.second[p];
+      const size_t   states = _partitions[p]->states, cats = _partitions[p]->rate_cats;
+      const bool     free_rates = _rate_category_types[p] == rate_category::FREE;
+      if (pp.subst_rates.size() != states * states - states || pp.freqs.size() != states ||
+          pp.gamma_alpha.size() != (free_rates ? cats : 1) || (free_rates && pp.gamma_weights.size() != cats))
+        throw std::invalid_argument(which + ": the parameters of partition " + std::to_string(p) +
+                                    " do not match the model");
+    }
+  }
+
+  // what is put back afterwards: the installed parameters and the rooting
+  struct installed_t {
+    std::vector<double> subst, freqs, rates, weights, rate_rates;
+  };
+  std::vector<installed_t> installed(_partitions.size());
+  for (size_t p = 0; p < _partitions.size(); ++p) {
+    const rdk_partition_t *part = _partitions[p];
+    const size_t           states = part->states;
+    installed[p].subst.assign(part->subst_params[0], part->subst_params[0] + states * states - states);
+    installed[p].freqs.assign(part->frequencies[0], part->frequencies[0] + states);
+    installed[p].rates.assign(part->rates, part->rates + part->rate_cats);
+    installed[p].weights.assign(part->rate_weights, part->rate_weights + part->rate_cats);
+    installed[p].rate_rates = _rate_rates[p];
+  }
+  const bool            was_rooted = _tree.rooted();
+  const root_location_t was_root = _tree.root_location();
+  auto restore = [&]() {
+    if (!keep_rows) {
+      for (size_t p = 0; p < _partitions.size(); ++p) rdk_partition_set_site_lnl_rows(_partitions[p], 0);
+      _support_rows = 0;
+    }
+    for (size_t p = 0; p < _partitions.size(); ++p) {
+      rdk_set_subst_params(_partitions[p], 0, installed[p].subst.data());
+      rdk_set_frequencies(_partitions[p], 0, installed[p].freqs.data());
+      rdk_set_category_rates(_partitions[p], installed[p].rates.data());
+      rdk_set_category_weights(_partitions[p], installed[p].weights.data());
+      _rate_rates[p] = installed[p].rate_rates;
+    }
+    if (was_rooted) {
+      _tree.root_by(was_root);
+      compute_lh(was_root);  // the CLVs of the previous rooting, for root-only evaluations
+    } else {
+      _tree.unroot();
+    }
+  };
+
+  const unsigned rows = (unsigned)records.size();
+  for (size_t p = 0; p < _partitions.size(); ++p)
+    if (rdk_partition_set_site_lnl_rows(_partitions[p], rows) != RDK_SUCCESS)
+      throw std::runtime_error("placement_support: " + engine_error());
+  _support_rows = rows;
+
+  placement_support_t out;
+  out.replicates = replicates;
+  try {
+    const auto t0 = std::chrono::steady_clock::now();
+    for (unsigned r = 0; r < rows; ++r) {
+      // installed as optimize_params installs them: a record holds the optimiser's variables, whose
+      // frequencies are normalised on the way in (set_model_params would take them as they are)
+      for (size_t p = 0; p < _partitions.size(); ++p) {
+        const auto &pp = records[r].second[p];
+        set_subst_rates(p, pp.subst_rates);
+        set_freqs_all_free(p, pp.freqs);
+        set_gamma_rates(p, pp.gamma_alpha);
+        if (_rate_category_types[p] == rate_category::FREE) set_gamma_weights(p, pp.gamma_weights);
+      }
+      const root_location_t rl = placement_of(records[r].first).first;
+      _tree.root_by(rl);
+      const traversal_t trav = full_traversal(rl);
+      for (size_t p = 0; p < _partitions.size(); ++p) {
+        update_pmatrix_partition(p, trav.pmatrix_indices, trav.branch_lengths);
+        rdk_update_clvs(_partitions[p], trav.ops.data(), (unsigned)trav.ops.size());
+        const double lh = rdk_compute_root_loglikelihood_row(_partitions[p], _tree.root_clv_index(),
+                                                             _tree.root_scaler_index(), r);
+        if (std::isnan(lh))
+          throw std::runtime_error("placement_support: record " + std::to_string(r) + ": " + engine_error());
+      }
+    }
+    out.capture_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+
+    std::vector<unsigned> global_index(_partitions.size());
+    std::iota(global_index.begin(), global_index.end(), 0u);
+    out.lnl_fixed.resize(rows);
+    out.bp_count.resize(rows);
+    out.kh_count.resize(rows);
+    out.sh_count.resize(rows);
+    out.o_lo.resize(rows);
+    out.o_hi.resize(rows);
+    rdk_rell_out_t rell;
+    memset(&rell, 0, sizeof(rell));
+    rell.replicate_tile = replicate_tile;
+    rell.lnl_fixed = out.lnl_fixed.data();
+    rell.bp_count = out.bp_count.data();
+    rell.kh_count = out.kh_count.data();
+    rell.sh_count = out.sh_count.data();
+    rell.o_lo = out.o_lo.data();
+    rell.o_hi = out.o_hi.data();
+    if (rdk_rell_support(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows, replicates, seed,
+                         &rell) != RDK_SUCCESS)
+      throw std::runtime_error("placement_support: " + engine_error());
+    out.best = rell.best;
+    out.exponent = rell.exponent;
+    out.counts_ms = rell.ms[0];
+    out.accumulate_ms = rell.ms[1];
+    out.statistics_ms = rell.ms[2];
+    out.resample_ms = rell.ms[3];
+    out.device_bytes = rell.device_bytes;
+  } catch (...) {
+    restore();
+    throw;
+  }
+  restore();
+
+  for (unsigned r = 0; r < rows; ++r) {
+    const double B = (double)replicates;
+    out.root_id.push_back(records[r].first.root_id);
+    out.alpha.push_back(records[r].first.alpha);
+    out.llh.push_back(records[r].first.llh);
+    out.bp.push_back(out.bp_count[r] / B);
+    out.p_kh.push_back(out.kh_count[r] / B);
+    out.p_sh.push_back(out.sh_count[r] / B);
+    const root_location_t rl = placement_of(records[r].first).first;
+    _tree.annotate_branch(rl, "BP", std::to_string(out.bp[r]));
+    _tree.annotate_branch(rl, "pKH", std::to_string(out.p_kh[r]));
+    _tree.annotate_branch(rl, "pSH", std::to_string(out.p_sh[r]));
+  }
+  return out;
+}
+
+std::vector<double> model_t::site_lnl_rows(size_t partition) {
+  if (partition >= _partitions.size()) throw std::invalid_argument("site_lnl_rows: partition out of range");
+  std::vector<double> out((size_t)_support_rows * _partitions[partition]->sites);
+  if (_support_rows &&
+      rdk_partition_get_site_lnl_rows(_partitions[partition], 0, _support_rows, out.data()) != RDK_SUCCESS)
+    throw std::runtime_error("site_lnl_rows: " + engine_error());
+  return out;
 }
 
 // LWR_i = exp(llh_i - max) / sum_j exp(llh_j - max) (src/model.cpp:1238-1253)

@@ -175,6 +175,31 @@ public:
   };
   const probe_counters_t &probe_counters() const { return _probe_counters; }
 
+  // ---- root placement support (DESIGN.md section 10) ------------------------------------------
+  // RELL bootstrap proportions and one-sided KH / SH tests of every placement in a checkpoint:
+  // each record's parameters are installed, the tree is rooted at (root_id, alpha) and one full
+  // evaluation stores the unweighted per-pattern log-likelihoods; rdk_rell_support resamples them.
+  // The model's parameters and root are put back afterwards; with keep_rows the rows stay on the
+  // device, readable through site_lnl_rows, until the next call (otherwise their memory is freed).
+  // On site shards (a communicator attached) every rank calls it with the same checkpoint,
+  // replicates and seed and gets the bits of one GPU.  Each placement's branch is annotated with
+  // BP, pKH, pSH.
+  struct placement_support_t {
+    std::vector<size_t>   root_id;
+    std::vector<double>   alpha, llh, lnl_fixed, bp, p_kh, p_sh;
+    std::vector<unsigned> bp_count, kh_count, sh_count;
+    std::vector<unsigned long long> o_lo;  // O[r] as a two's-complement int128
+    std::vector<long long>          o_hi;
+    size_t                replicates = 0, best = 0;
+    int                   exponent = 0;
+    double                capture_ms = 0, counts_ms = 0, accumulate_ms = 0, statistics_ms = 0, resample_ms = 0;
+    unsigned long long    device_bytes = 0;
+  };
+  placement_support_t placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
+                                        unsigned replicate_tile = 0, bool keep_rows = false);
+  // the unweighted per-pattern log-likelihoods of the last placement_support: [record][pattern]
+  std::vector<double> site_lnl_rows(size_t partition);
+
   rdk_partition_t *partition(size_t i) { return _partitions[i]; }
   size_t           partition_count() const { return _partitions.size(); }
 
@@ -246,6 +271,7 @@ private:
   probe_counters_t                       _probe_counters;
   partition_exchange_fn                  _exchange = nullptr;     // see set_partition_exchange
   void                                  *_exchange_user = nullptr;
+  unsigned                               _support_rows = 0;       // rows of the last placement_support
   std::vector<size_t>                    _global_index;           // global id of each local partition
   size_t                                 _global_partitions = 0;
   static constexpr unsigned int          _submodels = 1;

@@ -414,6 +414,73 @@ extern "C" int rdh_model_exhaustive_search(void *h, double atol, double pgtol, d
   })
 }
 
+// RELL bootstrap proportions and one-sided KH / SH tests of every placement recorded in
+// "<checkpoint_prefix>.ckp" (opened read-only; NULL: the model's own result log), B = replicates in
+// [1, 2^20] (model_t::placement_support; DESIGN.md section 10).  Per record, in log order (capacity
+// cap): root id, alpha and llh as recorded, the fixed-point log-likelihood, O as a two's-complement
+// int128 (o_lo, o_hi; may be NULL) and the integer counts (bp / p_KH / p_SH = count / replicates).
+// A log of more than cap records fails before any work, with n_out = its record count.  info
+// receives {capture ms, counts ms, accumulation ms, statistics ms, whole resampling ms, device
+// bytes}; replicate_tile 0 = the engine's choice; keep_rows != 0 keeps the per-pattern rows for
+// rdh_model_site_lnl_rows (otherwise their device memory is freed on return).
+extern "C" int rdh_model_placement_support(void *h, const char *checkpoint_prefix, unsigned long long replicates,
+                                           unsigned long long seed, unsigned replicate_tile, int keep_rows,
+                                           unsigned cap, unsigned long long *root_id, double *alpha, double *llh,
+                                           double *lnl_fixed, unsigned long long *o_lo, long long *o_hi,
+                                           unsigned *bp_count, unsigned *kh_count, unsigned *sh_count, int *exponent,
+                                           unsigned *best, double *info, unsigned *n_out) {
+  RDH_TRY({
+    checkpoint_t  external;
+    checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
+    const size_t  records = ckp.read_results().size();
+    if (records > cap) {
+      *n_out = (unsigned)records;
+      throw std::runtime_error("output buffers too small: " + std::to_string(records) + " records");
+    }
+    const auto   res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0);
+    const size_t n = res.root_id.size();
+    if (n > cap) throw std::runtime_error("output buffers too small");
+    for (size_t i = 0; i < n; ++i) {
+      root_id[i] = res.root_id[i];
+      alpha[i] = res.alpha[i];
+      llh[i] = res.llh[i];
+      lnl_fixed[i] = res.lnl_fixed[i];
+      if (o_lo) o_lo[i] = res.o_lo[i];
+      if (o_hi) o_hi[i] = res.o_hi[i];
+      bp_count[i] = res.bp_count[i];
+      kh_count[i] = res.kh_count[i];
+      sh_count[i] = res.sh_count[i];
+    }
+    *exponent = res.exponent;
+    *best = (unsigned)res.best;
+    info[0] = res.capture_ms;
+    info[1] = res.counts_ms;
+    info[2] = res.accumulate_ms;
+    info[3] = res.statistics_ms;
+    info[4] = res.resample_ms;
+    info[5] = (double)res.device_bytes;
+    *n_out = (unsigned)n;
+    return 1;
+  })
+}
+
+// the unweighted per-pattern log-likelihoods of the last placement support, [record][pattern] of
+// partition `part` (capacity cap doubles), and the partition's pattern weights (capacity
+// weights_cap); n_out = records * patterns
+extern "C" int rdh_model_site_lnl_rows(void *h, unsigned part, double *out, unsigned long long cap,
+                                       unsigned *weights, unsigned weights_cap, unsigned long long *n_out) {
+  RDH_TRY({
+    if (part >= H(h).msa.size()) throw std::invalid_argument("partition out of range");
+    const auto rows = H(h).model->site_lnl_rows(part);
+    const auto &msa = H(h).msa[part];
+    if (rows.size() > cap || msa.length() > weights_cap) throw std::runtime_error("output buffers too small");
+    std::memcpy(out, rows.data(), sizeof(double) * rows.size());
+    std::memcpy(weights, msa.weights(), sizeof(unsigned) * msa.length());
+    *n_out = rows.size();
+    return 1;
+  })
+}
+
 extern "C" int rdh_model_lwr(const double *llh, unsigned n, double *out) {
   auto w = model_t::lwr(std::vector<double>(llh, llh + n));
   for (unsigned i = 0; i < n; ++i) out[i] = w[i];

@@ -1,0 +1,88 @@
+#!/usr/bin/env python3
+"""Times root placement support (Model.placement_support, DESIGN.md section 10) at the cfg2 shape:
+a synthetic 500-taxon x 100 000-site alignment, 4 Gamma categories, a checkpoint holding all 2n-3
+placements (written record by record with Checkpoint.write, no search), B = 1 000 and 10 000.
+
+Prints one JSON line: per B the median over --reps calls (after one warm-up call) of the capture
+(host wall time of the 2n-3 full evaluations that store the rows), and of the counts, accumulation
+and statistics kernels (CUDA events inside the engine), the accumulation's term rate
+(B x patterns x records / accumulation time), the device memory the resampling allocated, and the
+card's name and power limit read in the same run.
+
+    python tools/bench_support.py [--taxa 500] [--sites 100000] [--replicates 1000,10000] [--reps 3]
+"""
+from __future__ import annotations
+
+import argparse
+import json
+import statistics
+import subprocess
+import sys
+import tempfile
+from pathlib import Path
+
+ROOT = Path(__file__).resolve().parent.parent
+sys.path.insert(0, str(ROOT))
+
+import numpy as np  # noqa: E402
+
+
+def card():
+    import torch
+    if not torch.cuda.is_available():
+        raise SystemExit("bench_support.py needs a CUDA device")
+    info = {"name": torch.cuda.get_device_name(0)}
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader",
+                              "-i", "0"], capture_output=True, text=True, timeout=30).stdout.strip()
+        info["power_limit"], info["max_sm_clock"] = [s.strip() for s in out.split(",")]
+    except Exception as exc:  # the number is still reported, without its card settings
+        info["power_limit"] = "unavailable: %s" % exc
+    return info
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--taxa", type=int, default=500)
+    ap.add_argument("--sites", type=int, default=100000)
+    ap.add_argument("--cats", type=int, default=4)
+    ap.add_argument("--replicates", default="1000,10000")
+    ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--seed", type=int, default=0x5EED0002)
+    args = ap.parse_args()
+
+    from root_digger_b200 import capi, synth
+    device = card()
+    top = synth.random_tree(args.taxa, args.seed)
+    rates, freqs = synth.random_params(args.seed + 1)
+    aln = synth.simulate_alignment(top, args.sites, args.seed + 2, rates, freqs, capi.gamma_cats(1.0, args.cats))
+    m = capi.Model(capi.RootedTree(synth.to_newick(top)), aln, rate_cats=args.cats, seed=1)
+    m.initialize_partitions(uniform_freqs=False)
+    R, P = m.root_count, m.sites(0)
+    r12, f4, _ = m.get_params()
+    rng = np.random.default_rng(args.seed + 3)
+    with tempfile.TemporaryDirectory() as tmp:
+        prefix = str(Path(tmp) / "support")
+        ckp = capi.Checkpoint(prefix)
+        ckp.save_options(prefix=prefix)
+        for rid in range(R):
+            params = [{"rates": r12, "freqs": f4, "alpha": float(rng.uniform(0.5, 2.0)),
+                       "weights": np.full(args.cats, 1.0 / args.cats)}]
+            ckp.write(rid, 0.0, float(rng.uniform(0.0, 1.0)), params, K=args.cats)
+        ckp.close()
+        results = {}
+        for B in [int(b) for b in args.replicates.split(",")]:
+            m.placement_support(prefix, replicates=B, seed=1)  # warm-up: module load, allocations
+            runs = [m.placement_support(prefix, replicates=B, seed=1 + i) for i in range(args.reps)]
+            med = {k: statistics.median(r[k] for r in runs)
+                   for k in ("capture_ms", "counts_ms", "accumulate_ms", "statistics_ms", "resample_ms")}
+            med["accumulate_terms_per_s"] = B * P * R / (med["accumulate_ms"] / 1e3)
+            med["device_bytes"] = max(r["device_bytes"] for r in runs)
+            med["bp_sum"] = int(runs[0]["bp_count"].sum())
+            results[str(B)] = med
+    print(json.dumps({"tool": "bench_support", "taxa": args.taxa, "patterns": P, "records": R, "cats": args.cats,
+                      "reps": args.reps, "card": device, "results": results}))
+
+
+if __name__ == "__main__":
+    main()
