@@ -435,6 +435,23 @@ int rdk_rell_support(rdk_partition_t *const *partitions, unsigned int n,
                      const unsigned int *global_index, unsigned int rows,
                      unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out);
 
+/* The multiscale RELL bootstrap of the AU test and expected likelihood weights (DESIGN.md section 10,
+ * items 6-8), on top of everything rdk_rell_support computes (it fills *out the same way).  At scale s
+ * (thousandths) replicate b draws max(1, (s N_g + 500) / 1000) sites of partition g with the Philox
+ * counter's second word s - 1000 (mod 2^64), so scale 1000 is the draws of rdk_rell_support and its
+ * column is bp_count.  Scales are strictly ascending, in [100, 10000], 2 to 32 of them. */
+typedef struct rdk_rell_ms_out_t {
+  const unsigned int *scales;      /* in: n_scales scales in thousandths */
+  unsigned int        n_scales;    /* in */
+  unsigned int       *scale_count; /* out: [n_scales][rows], #b whose argmax_r Z_k[b][r] is r */
+  unsigned long long *elw_fixed;   /* out: [rows], sum_b floor(u_b[r] 2^40 / sum_r' u_b[r']) */
+  double              ms[3];       /* out: device time of multiscale counts, accumulation, statistics + ELW */
+} rdk_rell_ms_out_t;
+int rdk_rell_support_ms(rdk_partition_t *const *partitions, unsigned int n,
+                        const unsigned int *global_index, unsigned int rows,
+                        unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
+                        rdk_rell_ms_out_t *ms);
+
 #ifdef __cplusplus
 }
 #endif

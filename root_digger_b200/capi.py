@@ -22,6 +22,22 @@ RDK_GAMMA_RATES_MEDIAN = 1
 RDK_SHARD_ALIGN = 256
 RDK_SWEEP_KEEP_ROOT = 1
 RDK_SWEEP_DISCARD = 2
+# the scales of the AU test's multiscale bootstrap that CONSEL and IQ-TREE use by default
+AU_SCALES = (0.5, 0.6, 0.7, 0.8, 0.9, 1.0, 1.1, 1.2, 1.3, 1.4)
+
+
+def au_thousandths(scales) -> list:
+    """AU scales -> integers in thousandths (what the host and the engine take); ValueError when a
+    scale is not a multiple of 0.001.  Order, range and count are checked by the host."""
+    out = []
+    for s in scales:
+        t = round(float(s) * 1000)
+        if abs(float(s) * 1000 - t) > 1e-6:
+            raise ValueError("AU scale %r is not a multiple of 0.001" % (s,))
+        if t <= 0:
+            raise ValueError("AU scale %r is not positive" % (s,))
+        out.append(t)
+    return out
 
 
 class Operation(C.Structure):
@@ -800,6 +816,11 @@ def _bind_model(L: C.CDLL):
     L.rdh_model_placement_support.argtypes = [vp, C.c_char_p, ull, ull, C.c_uint, C.c_int, C.c_uint, C.POINTER(ull),
                                               _dp, _dp, _dp, C.POINTER(ull), C.POINTER(C.c_longlong), _up, _up, _up,
                                               C.POINTER(C.c_int), _up, _dp, _up]
+    L.rdh_model_placement_support_au.argtypes = [vp, C.c_char_p, ull, ull, C.c_uint, C.c_int, C.c_uint, _up,
+                                                 C.c_uint, C.POINTER(ull), _dp, _dp, _dp, C.POINTER(ull),
+                                                 C.POINTER(C.c_longlong), _up, _up, _up, _up, _dp, _dp, _dp, _dp,
+                                                 _up, _dp, C.POINTER(ull), C.POINTER(C.c_int), _up, _dp, _up]
+    L.rdh_placement_au_fit.argtypes = [_up, C.c_uint, _up, ull, _dp, _up]
     L.rdh_model_site_lnl_rows.argtypes = [vp, C.c_uint, _dp, ull, _up, C.c_uint, C.POINTER(ull)]
     L.rdh_model_assign_indicies.argtypes = [vp, C.c_int, C.c_uint, C.c_double, C.c_uint, C.c_uint, C.c_int, _up,
                                             C.c_uint, _up]
@@ -1202,7 +1223,7 @@ class Model:
         return out[:got.value].tolist()
 
     def placement_support(self, checkpoint_prefix: str | None = None, replicates: int = 10000, seed: int = 0,
-                          replicate_tile: int = 0, keep_rows: bool = False) -> dict:
+                          replicate_tile: int = 0, keep_rows: bool = False, au_scales=None) -> dict:
         """RELL bootstrap proportions and one-sided KH / SH tests of every placement recorded in
         "<checkpoint_prefix>.ckp" (opened read-only; None: the model's own result log, e.g. of
         exhaustive_search), from `replicates` (1..2^20) resamplings of the sites, each partition on
@@ -1211,7 +1232,20 @@ class Model:
         counts; also exponent, best (record index), replicates and the timings.  The model's
         parameters and root are unchanged afterwards; the tree's branches carry BP, pKH and pSH in
         newick(True).  keep_rows keeps the per-pattern rows for site_lnl_rows.  On site shards
-        every rank calls it with the same arguments and gets the same result."""
+        every rank calls it with the same arguments and gets the same result.
+
+        au_scales (e.g. AU_SCALES: multiples of 0.001, 2 to 32 of them, strictly ascending, in
+        [0.1, 10]) adds Shimodaira's approximately unbiased test from a multiscale bootstrap (the
+        replicates drawn at scale s have s times as many sites) and Strimmer & Rambaut's expected
+        likelihood weights (DESIGN.md section 10, items 6-8): scales, scale_counts [scale][record]
+        (the column of scale 1 is bp_count), p_au, the fit's au_d, au_c, au_rss and au_used (scales
+        with 0 < count < replicates), elw and elw_fixed (elw = elw_fixed 2^-40 / replicates), and
+        au_counts_ms, au_accumulate_ms, au_statistics_ms; the branches also carry pAU and ELW.  The
+        fit is the two-parameter model of Shimodaira (2002) without the iterated threshold
+        refinement of CONSEL and IQ-TREE, so p_au may differ from theirs."""
+        if au_scales is not None:
+            return self._placement_support_au(checkpoint_prefix, replicates, seed, replicate_tile, keep_rows,
+                                              au_thousandths(au_scales))
         prefix = checkpoint_prefix.encode() if checkpoint_prefix is not None else None
         cap = 128
         for attempt in range(2):
@@ -1241,6 +1275,47 @@ class Model:
                 "exponent": exponent.value, "best": best.value, "replicates": int(replicates),
                 "capture_ms": info[0], "counts_ms": info[1], "accumulate_ms": info[2], "statistics_ms": info[3],
                 "resample_ms": info[4], "device_bytes": int(info[5])}
+
+    def _placement_support_au(self, checkpoint_prefix, replicates, seed, replicate_tile, keep_rows, scales):
+        prefix = checkpoint_prefix.encode() if checkpoint_prefix is not None else None
+        sc = np.ascontiguousarray(scales, dtype=np.uint32)
+        K, cap = len(sc), 128
+        ull = C.POINTER(C.c_ulonglong)
+        for attempt in range(2):
+            ids = np.zeros(cap, dtype=np.uint64)
+            alpha, llh, fixed = np.zeros(cap), np.zeros(cap), np.zeros(cap)
+            o_lo, o_hi = np.zeros(cap, dtype=np.uint64), np.zeros(cap, dtype=np.int64)
+            bp, kh, sh, used = (np.zeros(cap, dtype=np.uint32) for _ in range(4))
+            counts = np.zeros((max(1, K), cap), dtype=np.uint32)
+            p_au, d, c, rss, elw = (np.zeros(cap) for _ in range(5))
+            elw_fixed = np.zeros(cap, dtype=np.uint64)
+            exponent, best, got = C.c_int(), C.c_uint(), C.c_uint()
+            info = np.zeros(9)
+            rc = self.L.rdh_model_placement_support_au(
+                self.h, prefix, int(replicates), int(seed) & ((1 << 64) - 1), int(replicate_tile),
+                1 if keep_rows else 0, K, _ptr(sc, _up), cap, _ptr(ids, ull), _ptr(alpha, _dp), _ptr(llh, _dp),
+                _ptr(fixed, _dp), _ptr(o_lo, ull), _ptr(o_hi, C.POINTER(C.c_longlong)), _ptr(bp, _up),
+                _ptr(kh, _up), _ptr(sh, _up), _ptr(counts, _up), _ptr(p_au, _dp), _ptr(d, _dp), _ptr(c, _dp),
+                _ptr(rss, _dp), _ptr(used, _up), _ptr(elw, _dp), _ptr(elw_fixed, ull), C.byref(exponent),
+                C.byref(best), _ptr(info, _dp), C.byref(got))
+            if rc or attempt or got.value <= cap:
+                break
+            cap = got.value
+        self._check(rc)
+        n = got.value
+        self._support_rows = n if keep_rows else 0
+        B = float(replicates)
+        O = [(int(h) << 64) | int(l) for l, h in zip(o_lo[:n], o_hi[:n])]
+        return {"root_id": ids[:n].copy(), "alpha": alpha[:n].copy(), "llh": llh[:n].copy(),
+                "lnl_fixed": fixed[:n].copy(), "O": O, "bp_count": bp[:n].copy(), "kh_count": kh[:n].copy(),
+                "sh_count": sh[:n].copy(), "bp": bp[:n] / B, "p_kh": kh[:n] / B, "p_sh": sh[:n] / B,
+                "exponent": exponent.value, "best": best.value, "replicates": int(replicates),
+                "capture_ms": info[0], "counts_ms": info[1], "accumulate_ms": info[2], "statistics_ms": info[3],
+                "resample_ms": info[4], "device_bytes": int(info[5]),
+                "scales": sc / 1000.0, "scale_counts": counts[:, :n].copy(), "p_au": p_au[:n].copy(),
+                "au_d": d[:n].copy(), "au_c": c[:n].copy(), "au_rss": rss[:n].copy(), "au_used": used[:n].copy(),
+                "elw": elw[:n].copy(), "elw_fixed": elw_fixed[:n].copy(), "au_counts_ms": info[6],
+                "au_accumulate_ms": info[7], "au_statistics_ms": info[8]}
 
     def site_lnl_rows(self, part: int = 0):
         """(rows [record][pattern], pattern weights) of partition `part` from the last

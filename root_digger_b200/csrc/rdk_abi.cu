@@ -1459,9 +1459,9 @@ extern "C" int rdk_partition_get_site_lnl_rows(rdk_partition_t *p, unsigned int 
   return RDK_SUCCESS;
 }
 
-extern "C" int rdk_rell_support(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
-                                unsigned int rows, unsigned long long replicates, unsigned long long seed,
-                                rdk_rell_out_t *out) {
+static int rell_entry(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
+                      unsigned int rows, unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
+                      rdk_rell_ms_out_t *ms) {
   if (n == 0 || rows == 0) return fail(RDK_ERROR_PARAM, "rdk_rell_support: no partitions or no rows");
   if (replicates == 0 || replicates > kRellMaxReplicates)
     return fail(RDK_ERROR_PARAM, "rdk_rell_support: replicates must be in [1, 2^20]");
@@ -1494,9 +1494,31 @@ extern "C" int rdk_rell_support(rdk_partition_t *const *parts, unsigned int n, c
   }
   CUDA_TRY(cudaSetDevice(device));
   char msg[256];
-  if (!rell_support(rp.data(), n, rows, replicates, seed, shard, out, msg, sizeof(msg)))
+  if (!rell_support(rp.data(), n, rows, replicates, seed, shard, out, ms, msg, sizeof(msg)))
     return fail(RDK_ERROR_CUDA, "%s", msg);
   return RDK_SUCCESS;
+}
+
+extern "C" int rdk_rell_support(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
+                                unsigned int rows, unsigned long long replicates, unsigned long long seed,
+                                rdk_rell_out_t *out) {
+  return rell_entry(parts, n, global_index, rows, replicates, seed, out, nullptr);
+}
+
+extern "C" int rdk_rell_support_ms(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
+                                   unsigned int rows, unsigned long long replicates, unsigned long long seed,
+                                   rdk_rell_out_t *out, rdk_rell_ms_out_t *ms) {
+  if (!ms || !ms->scales || !ms->scale_count || !ms->elw_fixed)
+    return fail(RDK_ERROR_PARAM, "rdk_rell_support_ms: null scales or output arrays");
+  if (ms->n_scales < 2 || ms->n_scales > 32)
+    return fail(RDK_ERROR_PARAM, "rdk_rell_support_ms: %u scales, 2 to 32 are needed", ms->n_scales);
+  for (unsigned k = 0; k < ms->n_scales; ++k) {
+    if (ms->scales[k] < 100 || ms->scales[k] > 10000)
+      return fail(RDK_ERROR_PARAM, "rdk_rell_support_ms: scale %u is outside [100, 10000] thousandths", ms->scales[k]);
+    if (k && ms->scales[k] <= ms->scales[k - 1])
+      return fail(RDK_ERROR_PARAM, "rdk_rell_support_ms: scales must be strictly ascending");
+  }
+  return rell_entry(parts, n, global_index, rows, replicates, seed, out, ms);
 }
 
 // ---------------------------------------------------------------------------

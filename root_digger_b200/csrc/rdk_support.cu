@@ -6,6 +6,8 @@
 //   accumulation  Z[b][r] += sum_p c[b][p] * q[r][p], q = rint(L * 2^e) converted on load, in
 //                 shared-memory tiles, int128 accumulators (a term is < 2^32 * 2^52)
 //   statistics    column sums over b, row maxima over r, then the KH / SH / BP counts per record
+//   AU / ELW      (rdk_rell_support_ms) the ELW quotients on the unit-scale Z, summed by the column-sum
+//                 kernels; then per further scale the same counts and accumulation, argmax and histogram
 //
 // Every sum is an exact integer, so the result does not depend on launch shape or tiling.
 #include "rdk_support.cuh"
@@ -71,23 +73,26 @@ __global__ void rell_scan_kernel(const double *rows, size_t count, unsigned patt
   }
 }
 
-// c[b][p] for replicates [b0, b0 + tile) of one partition: one thread = one Philox block = 4 draws of
-// the partition's `sites` original sites; the draws that hit this shard's sites [lo, lo + cumw[patterns])
-// are counted (lo = 0 and every site here when the partition is not sharded)
+// c[b][p] for replicates [b0, b0 + tile) of one partition: one thread = one Philox block = 4 of the
+// `draws` draws (counter {j + 1, word, 0, 0}) over the partition's `sites` original sites; the draws
+// that hit this shard's sites [lo, lo + cumw[patterns]) are counted (lo = 0 and every site here when the
+// partition is not sharded).  rdk_rell_support draws `sites` times with word 0; the multiscale
+// bootstrap draws (s sites + 500) / 1000 times with word s - 1000.
 __global__ void rell_counts_kernel(unsigned long long seed, unsigned long long global_index, unsigned long long b0,
-                                   unsigned tile, unsigned long long sites, unsigned long long lo,
-                                   const unsigned long long *cumw, unsigned patterns, unsigned *c) {
-  const unsigned long long blocks = (sites + 3) / 4;
+                                   unsigned tile, unsigned long long draws, unsigned long long word,
+                                   unsigned long long sites, unsigned long long lo, const unsigned long long *cumw,
+                                   unsigned patterns, unsigned *c) {
+  const unsigned long long blocks = (draws + 3) / 4;
   const unsigned long long here = cumw[patterns];
   const unsigned long long total = blocks * tile;
   for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < total;
        i += (unsigned long long)gridDim.x * blockDim.x) {
     const unsigned long long b = i / blocks, j4 = i - b * blocks;
-    unsigned long long       x[4] = {j4 + 1, 0, 0, 0};  // numpy increments the counter before each block
+    unsigned long long       x[4] = {j4 + 1, word, 0, 0};  // numpy increments the counter before each block
     philox4x64_10(x, seed, (global_index << 32) | (b0 + b));
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
-      if (j4 * 4 + u >= sites) break;
+      if (j4 * 4 + u >= draws) break;
       const unsigned long long site = __umul64hi(x[u], sites) - lo;  // wraps below lo
       if (site >= here) continue;
       unsigned p = 0, hi = patterns;  // cumw[p] <= site < cumw[hi]
@@ -222,6 +227,93 @@ __global__ void rell_count_kernel(const i128 *z, unsigned nb, unsigned nr, unsig
   if (nsh) atomicAdd(sh + r, nsh);
 }
 
+// count[argmax[b]] += 1: the multiscale BP counts of one scale
+__global__ void rell_hist_kernel(const unsigned *argmax, unsigned nb, unsigned *count) {
+  const unsigned b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < nb) atomicAdd(count + argmax[b], 1u);
+}
+
+// ---- expected likelihood weights (DESIGN.md section 10, item 8)
+
+// int128 -> double, rounded to nearest even: the top 64 bits with the rest folded into a sticky bit
+// round as the whole value does (11 bits are dropped below the sticky bit's position)
+__device__ double i128_to_double_rn(i128 v) {
+  const bool neg = v < 0;
+  const u128 a = neg ? -(u128)v : (u128)v;
+  const unsigned long long hi = (unsigned long long)(a >> 64);
+  double                   d;
+  if (hi == 0) {
+    d = __ull2double_rn((unsigned long long)a);
+  } else {
+    const int                sh = 64 - __clzll((long long)hi);
+    const unsigned long long top = (unsigned long long)(a >> sh) | (((a << (128 - sh)) != 0) ? 1ull : 0ull);
+    d = scalbn(__ull2double_rn(top), sh);
+  }
+  return neg ? -d : d;
+}
+
+// fdlibm e_exp.c on [-40, 0], every operation rounded on its own; rd_exp(0) == 1
+__device__ double rd_exp(double x) {
+  const double P1 = 1.66666666666666019037e-01, P2 = -2.77777777770155933842e-03, P3 = 6.61375632143793436117e-05,
+               P4 = -1.65339022054652515390e-06, P5 = 4.13813679705723846039e-08;
+  const double ln2hi = 6.93147180369123816490e-01, ln2lo = 1.90821492927058770002e-10,
+               invln2 = 1.44269504088896338700e+00;
+  const unsigned hx = (unsigned)__double2hiint(x) & 0x7fffffffu;
+  double         hi = 0, lo = 0;
+  int            k = 0;
+  if (hx > 0x3fd62e42u) {    // |x| > ln2 / 2
+    if (hx < 0x3ff0a2b2u) {  // |x| < 3 ln2 / 2
+      hi = __dadd_rn(x, ln2hi);
+      lo = -ln2lo;
+      k = -1;
+    } else {
+      k = __double2int_rz(__dadd_rn(__dmul_rn(invln2, x), -0.5));
+      const double t = (double)k;
+      hi = __dadd_rn(x, -__dmul_rn(t, ln2hi));
+      lo = __dmul_rn(t, ln2lo);
+    }
+    x = __dadd_rn(hi, -lo);
+  } else if (hx < 0x3e300000u) {  // |x| < 2^-28
+    return __dadd_rn(1.0, x);
+  }
+  const double t = __dmul_rn(x, x);
+  double       p = __dadd_rn(P4, __dmul_rn(t, P5));
+  p = __dadd_rn(P3, __dmul_rn(t, p));
+  p = __dadd_rn(P2, __dmul_rn(t, p));
+  p = __dadd_rn(P1, __dmul_rn(t, p));
+  const double c = __dadd_rn(x, -__dmul_rn(t, p));
+  if (k == 0) return __dadd_rn(1.0, -__dadd_rn(__ddiv_rn(__dmul_rn(x, c), __dadd_rn(c, -2.0)), -x));
+  const double y = __dadd_rn(1.0, -__dadd_rn(__dadd_rn(lo, -__ddiv_rn(__dmul_rn(x, c), __dadd_rn(2.0, -c))), -hi));
+  return __hiloint2double(__double2hiint(y) + k * (1 << 20), __double2loint(y));  // y 2^k, exact for k >= -1021
+}
+
+// Delta < -40 2^e, exactly (|Delta| < 2^85; e < 0 only when max |L| >= 2^52)
+__device__ __forceinline__ bool elw_below_cut(i128 d, int e) {
+  if (e >= 80) return false;
+  if (e >= 0) return d < -((i128)40 << e);
+  return d != 0 && (-e >= 6 || ((-d) << -e) > 40);
+}
+
+// u = rint(rd_exp(Delta 2^-e) 2^52), 0 below the cut; the record of the maximum gets 2^52
+__device__ __forceinline__ unsigned long long elw_weight(i128 d, int e) {
+  if (elw_below_cut(d, e)) return 0;
+  return __double2ull_rn(scalbn(rd_exp(scalbn(i128_to_double_rn(d), -e)), 52));
+}
+
+// one warp per replicate: D_b = sum_r u_b[r], then Z[b][r] := floor(u_b[r] 2^40 / D_b) in place (the
+// unit-scale statistics are done with Z); the column sums of those quotients are elw_fixed
+__global__ void rell_elw_kernel(i128 *z, unsigned nb, unsigned nr, int e, const unsigned *argmax) {
+  const unsigned b = blockIdx.x * (blockDim.x / 32) + threadIdx.x / 32, lane = threadIdx.x & 31;
+  if (b >= nb) return;
+  i128      *zb = z + (size_t)b * nr;
+  const i128 m = zb[argmax[b]];
+  u128       D = 0;
+  for (unsigned r = lane; r < nr; r += 32) D += elw_weight(zb[r] - m, e);
+  for (int off = 16; off; off >>= 1) D += (u128)shfl_xor_i128((i128)D, off);
+  __syncwarp();  // every lane has read m before any lane writes
+  for (unsigned r = lane; r < nr; r += 32) zb[r] = (i128)(((u128)elw_weight(zb[r] - m, e) << 40) / D);
+}
+
 // int128 <-> three int64 limbs v = l0 + l1 2^42 + l2 2^84 (l0, l1 in [0, 2^42)), so that an NCCL
 // sum of the limbs over up to 2^21 ranks cannot overflow; limbs[k * n + i]
 constexpr int kLimbBits = 42;
@@ -279,7 +371,8 @@ struct Events {
   } while (0)
 
 int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, unsigned long long replicates,
-                 unsigned long long seed, const RellShard &shard, rdk_rell_out_t *out, char *msg, size_t msg_cap) {
+                 unsigned long long seed, const RellShard &shard, rdk_rell_out_t *out, rdk_rell_ms_out_t *ms,
+                 char *msg, size_t msg_cap) {
   cudaStream_t  stream = nullptr;
   DeviceBuffers buf;
   Events        ev;
@@ -400,55 +493,62 @@ int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, 
     RELL_TRY(cudaGetLastError());
   }
 
-  // ---- counts and accumulation, tile by tile
+  // ---- counts and accumulation, tile by tile, of the replicates at one scale (thousandths; the
+  // counter word is s - 1000 mod 2^64, so scale 1000 is word 0 and N_g draws)
   float t_counts = 0, t_acc = 0, t_stats = 0, t_ms = 0;
-  RELL_TRY(cudaEventRecord(ev.ev[6], stream));
-  for (unsigned long long b0 = 0; b0 < nb; b0 += tile) {
-    const unsigned nt = (unsigned)std::min<unsigned long long>(tile, nb - b0);
-    for (unsigned g = 0; g < n; ++g) {
-      const unsigned P = parts[g].patterns;
-      RELL_TRY(cudaEventRecord(ev.ev[0], stream));
-      RELL_TRY(cudaMemsetAsync(d_c, 0, sizeof(unsigned) * (size_t)nt * std::max(1u, P), stream));
-      if (sites[g]) {
-        const unsigned long long work = (sites[g] + 3) / 4 * nt;
-        const unsigned grid = (unsigned)std::min<unsigned long long>((work + 255) / 256, (unsigned long long)sms * 16);
-        rell_counts_kernel<<<grid, 256, 0, stream>>>(seed, parts[g].global_index, b0, nt, sites[g], lo, d_cumw[g],
-                                                     P, d_c);
+  auto  resample = [&](unsigned scale, float &counts_ms, float &acc_ms) -> int {
+    const unsigned long long word = (unsigned long long)scale - 1000ull;
+    for (unsigned long long b0 = 0; b0 < nb; b0 += tile) {
+      const unsigned nt = (unsigned)std::min<unsigned long long>(tile, nb - b0);
+      for (unsigned g = 0; g < n; ++g) {
+        const unsigned           P = parts[g].patterns;
+        const unsigned long long draws = std::max<unsigned long long>(1, (scale * sites[g] + 500) / 1000);
+        RELL_TRY(cudaEventRecord(ev.ev[0], stream));
+        RELL_TRY(cudaMemsetAsync(d_c, 0, sizeof(unsigned) * (size_t)nt * std::max(1u, P), stream));
+        if (sites[g]) {
+          const unsigned long long work = (draws + 3) / 4 * nt;
+          const unsigned grid = (unsigned)std::min<unsigned long long>((work + 255) / 256, (unsigned long long)sms * 16);
+          rell_counts_kernel<<<grid, 256, 0, stream>>>(seed, parts[g].global_index, b0, nt, draws, word, sites[g], lo,
+                                                       d_cumw[g], P, d_c);
+          RELL_TRY(cudaGetLastError());
+        }
+        RELL_TRY(cudaEventRecord(ev.ev[1], stream));
+        const dim3 grid((rows + kTile - 1) / kTile, (nt + kTile - 1) / kTile);
+        rell_accumulate_kernel<<<grid, acc_threads, 0, stream>>>(d_c, parts[g].rows, P, nt, rows, e, g > 0,
+                                                                 d_z + b0 * rows, rows);
         RELL_TRY(cudaGetLastError());
+        RELL_TRY(cudaEventRecord(ev.ev[2], stream));
+        RELL_TRY(cudaEventSynchronize(ev.ev[2]));
+        float t = 0;
+        RELL_TRY(cudaEventElapsedTime(&t, ev.ev[0], ev.ev[1]));
+        counts_ms += t;
+        RELL_TRY(cudaEventElapsedTime(&t, ev.ev[1], ev.ev[2]));
+        acc_ms += t;
       }
-      RELL_TRY(cudaEventRecord(ev.ev[1], stream));
-      const dim3 grid((rows + kTile - 1) / kTile, (nt + kTile - 1) / kTile);
-      rell_accumulate_kernel<<<grid, acc_threads, 0, stream>>>(d_c, parts[g].rows, P, nt, rows, e, g > 0,
-                                                               d_z + b0 * rows, rows);
-      RELL_TRY(cudaGetLastError());
-      RELL_TRY(cudaEventRecord(ev.ev[2], stream));
-      RELL_TRY(cudaEventSynchronize(ev.ev[2]));
-      RELL_TRY(cudaEventElapsedTime(&t_ms, ev.ev[0], ev.ev[1]));
-      t_counts += t_ms;
-      RELL_TRY(cudaEventElapsedTime(&t_ms, ev.ev[1], ev.ev[2]));
-      t_acc += t_ms;
     }
-  }
+    return 1;
+  };
+  RELL_TRY(cudaEventRecord(ev.ev[6], stream));
+  if (!resample(1000, t_counts, t_acc)) return 0;
 
-  // site shards, exchange 3: Z and O summed over the ranks as 42-bit limbs (exact)
-  if (shard.comm) {
-    const size_t n_all = (size_t)nb * rows + rows;
-    long long   *d_limbs = nullptr;
-    RELL_TRY(buf.alloc(&d_limbs, 3 * n_all));
-    const unsigned grid = (unsigned)std::min<size_t>((n_all + 255) / 256, (size_t)sms * 8);
-    for (int pass = 0; pass < 2; ++pass) {  // Z, then O
-      i128        *v = pass ? d_o : d_z;
-      const size_t cnt = pass ? rows : (size_t)nb * rows;
-      rell_to_limbs_kernel<<<grid, 256, 0, stream>>>(v, cnt, d_limbs);
-      RELL_TRY(cudaGetLastError());
-      if (shard.allreduce(d_limbs, d_limbs, 3 * cnt, kNcclInt64, kNcclSum, shard.comm, stream) != 0) {
-        snprintf(msg, msg_cap, "ncclAllReduce (limbs) failed");
-        cudaStreamDestroy(stream);
-        return 0;
-      }
-      rell_from_limbs_kernel<<<grid, 256, 0, stream>>>(d_limbs, cnt, v);
-      RELL_TRY(cudaGetLastError());
+  // site shards, exchange 3: Z and O summed over the ranks as 42-bit limbs (exact); Z_k again per scale
+  long long *d_limbs = nullptr;
+  auto       allreduce = [&](i128 *v, size_t cnt) -> int {
+    const unsigned grid = (unsigned)std::min<size_t>((cnt + 255) / 256, (size_t)sms * 8);
+    rell_to_limbs_kernel<<<grid, 256, 0, stream>>>(v, cnt, d_limbs);
+    RELL_TRY(cudaGetLastError());
+    if (shard.allreduce(d_limbs, d_limbs, 3 * cnt, kNcclInt64, kNcclSum, shard.comm, stream) != 0) {
+      snprintf(msg, msg_cap, "ncclAllReduce (limbs) failed");
+      cudaStreamDestroy(stream);
+      return 0;
     }
+    rell_from_limbs_kernel<<<grid, 256, 0, stream>>>(d_limbs, cnt, v);
+    RELL_TRY(cudaGetLastError());
+    return 1;
+  };
+  if (shard.comm) {
+    RELL_TRY(buf.alloc(&d_limbs, 3 * ((size_t)nb * rows + rows)));
+    if (!allreduce(d_z, (size_t)nb * rows) || !allreduce(d_o, rows)) return 0;
   }
 
   // ---- statistics
@@ -486,6 +586,48 @@ int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, 
   RELL_TRY(cudaStreamSynchronize(stream));
   RELL_TRY(cudaEventElapsedTime(&t_stats, ev.ev[3], ev.ev[4]));
   RELL_TRY(cudaEventElapsedTime(&t_ms, ev.ev[6], ev.ev[7]));
+
+  if (ms) {
+    // ELW on the unit-scale Z (its argmax is still in d_argmax), then overwritten by the quotients
+    float t_ms_counts = 0, t_ms_acc = 0, t_ms_stats = 0, t = 0;
+    RELL_TRY(cudaEventRecord(ev.ev[3], stream));
+    rell_elw_kernel<<<(nb + 7) / 8, 256, 0, stream>>>(d_z, nb, rows, e, d_argmax);
+    rell_colsum_kernel<<<col_grid, 128, 0, stream>>>(d_z, nb, rows, chunk, d_part);
+    rell_colsum_final_kernel<<<(rows + 127) / 128, 128, 0, stream>>>(d_part, chunks, rows, d_colsum);
+    RELL_TRY(cudaGetLastError());
+    RELL_TRY(cudaEventRecord(ev.ev[4], stream));
+    std::vector<i128> elw(rows);
+    RELL_TRY(cudaMemcpyAsync(elw.data(), d_colsum, sizeof(i128) * rows, cudaMemcpyDeviceToHost, stream));
+    RELL_TRY(cudaStreamSynchronize(stream));
+    RELL_TRY(cudaEventElapsedTime(&t, ev.ev[3], ev.ev[4]));
+    t_ms_stats += t;
+    for (unsigned r = 0; r < rows; ++r) ms->elw_fixed[r] = (unsigned long long)elw[r];  // < 2^60
+
+    // the other scales: Z_k in the same buffer, argmax per replicate, histogram
+    for (unsigned k = 0; k < ms->n_scales; ++k) {
+      unsigned *count = ms->scale_count + (size_t)k * rows;
+      if (ms->scales[k] == 1000) {
+        memcpy(count, out->bp_count, sizeof(unsigned) * rows);
+        continue;
+      }
+      if (!resample(ms->scales[k], t_ms_counts, t_ms_acc)) return 0;
+      if (shard.comm && !allreduce(d_z, (size_t)nb * rows)) return 0;
+      RELL_TRY(cudaEventRecord(ev.ev[3], stream));
+      RELL_TRY(cudaMemsetAsync(d_counts, 0, sizeof(unsigned) * rows, stream));
+      rell_rowstat_kernel<<<(nb + 7) / 8, 256, 0, stream>>>(d_z, nb, rows, d_colsum, d_rowmax, d_argmax);
+      rell_hist_kernel<<<(nb + 255) / 256, 256, 0, stream>>>(d_argmax, nb, d_counts);
+      RELL_TRY(cudaGetLastError());
+      RELL_TRY(cudaEventRecord(ev.ev[4], stream));
+      RELL_TRY(cudaMemcpyAsync(count, d_counts, sizeof(unsigned) * rows, cudaMemcpyDeviceToHost, stream));
+      RELL_TRY(cudaStreamSynchronize(stream));
+      RELL_TRY(cudaEventElapsedTime(&t, ev.ev[3], ev.ev[4]));
+      t_ms_stats += t;
+    }
+    ms->ms[0] = t_ms_counts;
+    ms->ms[1] = t_ms_acc;
+    ms->ms[2] = t_ms_stats;
+  }
+
   out->ms[0] = t_counts;
   out->ms[1] = t_acc;
   out->ms[2] = t_stats;

@@ -33,9 +33,11 @@ struct RellShard {
   rell_allreduce_fn  allreduce = nullptr;
 };
 
-// runs on the current device; returns 0 with a message in msg on failure
+// runs on the current device; returns 0 with a message in msg on failure.  ms (validated by the
+// caller; null for rdk_rell_support) adds the multiscale counts and the ELW of rdk_rell_support_ms.
 int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, unsigned long long replicates,
-                 unsigned long long seed, const RellShard &shard, rdk_rell_out_t *out, char *msg, size_t msg_cap);
+                 unsigned long long seed, const RellShard &shard, rdk_rell_out_t *out, rdk_rell_ms_out_t *ms,
+                 char *msg, size_t msg_cap);
 
 }  // namespace rdk
 

@@ -20,8 +20,10 @@
 #include "model.hpp"
 
 #ifdef RD_BACKEND_ORACLE
-#include "rdk_support.h"  // tests/oracle_shim: the placement-support entries over the CPU oracle
+#include "rdk_support.h"     // tests/oracle_shim: the placement-support entries over the CPU oracle
+#include "rdk_support_au.h"  // ... and rdk_rell_support_ms
 #endif
+#include "support_stats.hpp"
 
 #include <algorithm>
 #include <chrono>
@@ -949,12 +951,15 @@ std::pair<root_location_t, double> model_t::exhaustive_search(double atol, doubl
 // root placement support (DESIGN.md section 10)
 // ---------------------------------------------------------------------------
 model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
-                                                        unsigned replicate_tile, bool keep_rows) {
+                                                        unsigned replicate_tile, bool keep_rows,
+                                                        const std::vector<unsigned> &au_scales) {
   if (_exchange)
     throw std::invalid_argument("placement_support: a model whose partitions are dealt to several processes is "
                                 "not supported");
   if (replicates == 0 || replicates > (size_t(1) << 20))
     throw std::invalid_argument("placement_support: replicates must be between 1 and 2^20");
+  const bool au = !au_scales.empty();
+  if (au) rd::check_au_scales(au_scales.data(), au_scales.size());
   const auto records = checkpoint.read_results();
   if (records.empty()) throw std::invalid_argument("placement_support: the checkpoint holds no records");
   if (records.size() > std::numeric_limits<unsigned>::max())
@@ -1067,9 +1072,26 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
     rell.sh_count = out.sh_count.data();
     rell.o_lo = out.o_lo.data();
     rell.o_hi = out.o_hi.data();
-    if (rdk_rell_support(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows, replicates, seed,
-                         &rell) != RDK_SUCCESS)
+    if (au) {
+      out.scales = au_scales;
+      out.scale_count.resize(au_scales.size() * rows);
+      out.elw_fixed.resize(rows);
+      rdk_rell_ms_out_t ms;
+      memset(&ms, 0, sizeof(ms));
+      ms.scales = out.scales.data();
+      ms.n_scales = (unsigned)out.scales.size();
+      ms.scale_count = out.scale_count.data();
+      ms.elw_fixed = out.elw_fixed.data();
+      if (rdk_rell_support_ms(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows,
+                              replicates, seed, &rell, &ms) != RDK_SUCCESS)
+        throw std::runtime_error("placement_support: " + engine_error());
+      out.au_counts_ms = ms.ms[0];
+      out.au_accumulate_ms = ms.ms[1];
+      out.au_statistics_ms = ms.ms[2];
+    } else if (rdk_rell_support(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows,
+                                replicates, seed, &rell) != RDK_SUCCESS) {
       throw std::runtime_error("placement_support: " + engine_error());
+    }
     out.best = rell.best;
     out.exponent = rell.exponent;
     out.counts_ms = rell.ms[0];
@@ -1095,6 +1117,19 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
     _tree.annotate_branch(rl, "BP", std::to_string(out.bp[r]));
     _tree.annotate_branch(rl, "pKH", std::to_string(out.p_kh[r]));
     _tree.annotate_branch(rl, "pSH", std::to_string(out.p_sh[r]));
+    if (au) {
+      std::vector<unsigned> count(au_scales.size());
+      for (size_t k = 0; k < count.size(); ++k) count[k] = out.scale_count[k * rows + r];
+      const rd::au_fit_t fit = rd::au_fit(count.data(), au_scales.data(), count.size(), replicates);
+      out.p_au.push_back(fit.p_au);
+      out.au_d.push_back(fit.d);
+      out.au_c.push_back(fit.c);
+      out.au_rss.push_back(fit.rss);
+      out.au_used.push_back(fit.used);
+      out.elw.push_back(ldexp((double)out.elw_fixed[r], -40) / B);
+      _tree.annotate_branch(rl, "pAU", std::to_string(fit.p_au));
+      _tree.annotate_branch(rl, "ELW", std::to_string(out.elw[r]));
+    }
   }
   return out;
 }

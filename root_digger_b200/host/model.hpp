@@ -184,6 +184,10 @@ public:
   // On site shards (a communicator attached) every rank calls it with the same checkpoint,
   // replicates and seed and gets the bits of one GPU.  Each placement's branch is annotated with
   // BP, pKH, pSH.
+  // With au_scales (thousandths; 2 to 32, strictly ascending, in [100, 10000]) the same call also
+  // runs the multiscale bootstrap at those scales and fits the AU test per record, and computes the
+  // expected likelihood weights (rdk_rell_support_ms; DESIGN.md section 10, items 6-8); the branches
+  // then also carry pAU and ELW.
   struct placement_support_t {
     std::vector<size_t>   root_id;
     std::vector<double>   alpha, llh, lnl_fixed, bp, p_kh, p_sh;
@@ -194,9 +198,15 @@ public:
     int                   exponent = 0;
     double                capture_ms = 0, counts_ms = 0, accumulate_ms = 0, statistics_ms = 0, resample_ms = 0;
     unsigned long long    device_bytes = 0;
+    // AU mode only (empty otherwise): scale_count is [scale][record]
+    std::vector<unsigned>           scales, scale_count, au_used;
+    std::vector<double>             p_au, au_d, au_c, au_rss, elw;
+    std::vector<unsigned long long> elw_fixed;
+    double                          au_counts_ms = 0, au_accumulate_ms = 0, au_statistics_ms = 0;
   };
   placement_support_t placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
-                                        unsigned replicate_tile = 0, bool keep_rows = false);
+                                        unsigned replicate_tile = 0, bool keep_rows = false,
+                                        const std::vector<unsigned> &au_scales = {});
   // the unweighted per-pattern log-likelihoods of the last placement_support: [record][pattern]
   std::vector<double> site_lnl_rows(size_t partition);
 

@@ -2,6 +2,7 @@
 // Python multi-GPU launcher).  Return 1 on success, 0 on failure with the
 // message available from rdh_last_error() (exceptions never cross the boundary).
 #include "model.hpp"
+#include "support_stats.hpp"
 
 #include <cstdio>
 #include <cstdlib>
@@ -414,6 +415,46 @@ extern "C" int rdh_model_exhaustive_search(void *h, double atol, double pgtol, d
   })
 }
 
+// the body of rdh_model_placement_support and rdh_model_placement_support_au
+static model_t::placement_support_t placement_support_into(
+    void *h, const char *checkpoint_prefix, unsigned long long replicates, unsigned long long seed,
+    unsigned replicate_tile, int keep_rows, unsigned cap, unsigned long long *root_id, double *alpha, double *llh,
+    double *lnl_fixed, unsigned long long *o_lo, long long *o_hi, unsigned *bp_count, unsigned *kh_count,
+    unsigned *sh_count, int *exponent, unsigned *best, double *info, unsigned *n_out,
+    const std::vector<unsigned> &au_scales) {
+  checkpoint_t  external;
+  checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
+  const size_t  records = ckp.read_results().size();
+  if (records > cap) {
+    *n_out = (unsigned)records;
+    throw std::runtime_error("output buffers too small: " + std::to_string(records) + " records");
+  }
+  auto res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0, au_scales);
+  const size_t n = res.root_id.size();
+  if (n > cap) throw std::runtime_error("output buffers too small");
+  for (size_t i = 0; i < n; ++i) {
+    root_id[i] = res.root_id[i];
+    alpha[i] = res.alpha[i];
+    llh[i] = res.llh[i];
+    lnl_fixed[i] = res.lnl_fixed[i];
+    if (o_lo) o_lo[i] = res.o_lo[i];
+    if (o_hi) o_hi[i] = res.o_hi[i];
+    bp_count[i] = res.bp_count[i];
+    kh_count[i] = res.kh_count[i];
+    sh_count[i] = res.sh_count[i];
+  }
+  *exponent = res.exponent;
+  *best = (unsigned)res.best;
+  info[0] = res.capture_ms;
+  info[1] = res.counts_ms;
+  info[2] = res.accumulate_ms;
+  info[3] = res.statistics_ms;
+  info[4] = res.resample_ms;
+  info[5] = (double)res.device_bytes;
+  *n_out = (unsigned)n;
+  return res;
+}
+
 // RELL bootstrap proportions and one-sided KH / SH tests of every placement recorded in
 // "<checkpoint_prefix>.ckp" (opened read-only; NULL: the model's own result log), B = replicates in
 // [1, 2^20] (model_t::placement_support; DESIGN.md section 10).  Per record, in log order (capacity
@@ -430,36 +471,71 @@ extern "C" int rdh_model_placement_support(void *h, const char *checkpoint_prefi
                                            unsigned *bp_count, unsigned *kh_count, unsigned *sh_count, int *exponent,
                                            unsigned *best, double *info, unsigned *n_out) {
   RDH_TRY({
-    checkpoint_t  external;
-    checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
-    const size_t  records = ckp.read_results().size();
-    if (records > cap) {
-      *n_out = (unsigned)records;
-      throw std::runtime_error("output buffers too small: " + std::to_string(records) + " records");
-    }
-    const auto   res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0);
+    placement_support_into(h, checkpoint_prefix, replicates, seed, replicate_tile, keep_rows, cap, root_id, alpha,
+                           llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count, exponent, best, info, n_out, {});
+    return 1;
+  })
+}
+
+// rdh_model_placement_support plus the AU test and the expected likelihood weights (DESIGN.md
+// section 10, items 6-8) from a multiscale bootstrap at n_scales scales in thousandths (2 to 32,
+// strictly ascending, in [100, 10000]).  Per record (capacity cap): scale_count[k * cap + r] = #b whose
+// argmax at scale k is r, p_au, the fit's d, c and weighted residual sum of squares, the number of
+// scales it used, elw and its fixed-point sum elw_fixed (elw = elw_fixed 2^-40 / replicates).  info
+// receives the six values of rdh_model_placement_support, then {multiscale counts ms, multiscale
+// accumulation ms, statistics + ELW ms}.  Refuses before any work as rdh_model_placement_support does.
+extern "C" int rdh_model_placement_support_au(void *h, const char *checkpoint_prefix, unsigned long long replicates,
+                                              unsigned long long seed, unsigned replicate_tile, int keep_rows,
+                                              unsigned n_scales, const unsigned *scales, unsigned cap,
+                                              unsigned long long *root_id, double *alpha, double *llh,
+                                              double *lnl_fixed, unsigned long long *o_lo, long long *o_hi,
+                                              unsigned *bp_count, unsigned *kh_count, unsigned *sh_count,
+                                              unsigned *scale_count, double *p_au, double *au_d, double *au_c,
+                                              double *au_rss, unsigned *au_used, double *elw,
+                                              unsigned long long *elw_fixed, int *exponent, unsigned *best,
+                                              double *info, unsigned *n_out) {
+  RDH_TRY({
+    if (!scales) throw std::invalid_argument("AU scales: none given");
+    const std::vector<unsigned> au(scales, scales + n_scales);
+    rd::check_au_scales(au.data(), au.size());
+    const auto res = placement_support_into(h, checkpoint_prefix, replicates, seed, replicate_tile, keep_rows, cap,
+                                            root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count,
+                                            exponent, best, info, n_out, au);
     const size_t n = res.root_id.size();
-    if (n > cap) throw std::runtime_error("output buffers too small");
     for (size_t i = 0; i < n; ++i) {
-      root_id[i] = res.root_id[i];
-      alpha[i] = res.alpha[i];
-      llh[i] = res.llh[i];
-      lnl_fixed[i] = res.lnl_fixed[i];
-      if (o_lo) o_lo[i] = res.o_lo[i];
-      if (o_hi) o_hi[i] = res.o_hi[i];
-      bp_count[i] = res.bp_count[i];
-      kh_count[i] = res.kh_count[i];
-      sh_count[i] = res.sh_count[i];
+      for (size_t k = 0; k < au.size(); ++k) scale_count[k * cap + i] = res.scale_count[k * n + i];
+      p_au[i] = res.p_au[i];
+      au_d[i] = res.au_d[i];
+      au_c[i] = res.au_c[i];
+      au_rss[i] = res.au_rss[i];
+      au_used[i] = res.au_used[i];
+      elw[i] = res.elw[i];
+      elw_fixed[i] = res.elw_fixed[i];
     }
-    *exponent = res.exponent;
-    *best = (unsigned)res.best;
-    info[0] = res.capture_ms;
-    info[1] = res.counts_ms;
-    info[2] = res.accumulate_ms;
-    info[3] = res.statistics_ms;
-    info[4] = res.resample_ms;
-    info[5] = (double)res.device_bytes;
-    *n_out = (unsigned)n;
+    info[6] = res.au_counts_ms;
+    info[7] = res.au_accumulate_ms;
+    info[8] = res.au_statistics_ms;
+    return 1;
+  })
+}
+
+// the AU fit of one record alone (model_t::placement_support in AU mode; DESIGN.md section 10, item 7):
+// counts[k] of B replicates at scales[k] (thousandths) -> out = {p_AU, d, c, rss}, used = the number of
+// scales with 0 < count < B
+extern "C" int rdh_placement_au_fit(const unsigned *counts, unsigned n_scales, const unsigned *scales,
+                                    unsigned long long B, double *out, unsigned *used) {
+  RDH_TRY({
+    if (!counts || !scales) throw std::invalid_argument("AU fit: null counts or scales");
+    rd::check_au_scales(scales, n_scales);
+    if (B == 0) throw std::invalid_argument("AU fit: no replicates");
+    for (unsigned k = 0; k < n_scales; ++k)
+      if (counts[k] > B) throw std::invalid_argument("AU fit: a count exceeds the replicates");
+    const rd::au_fit_t fit = rd::au_fit(counts, scales, n_scales, B);
+    out[0] = fit.p_au;
+    out[1] = fit.d;
+    out[2] = fit.c;
+    out[3] = fit.rss;
+    *used = fit.used;
     return 1;
   })
 }

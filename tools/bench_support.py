@@ -9,7 +9,12 @@ and statistics kernels (CUDA events inside the engine), the accumulation's term 
 (B x patterns x records / accumulation time), the device memory the resampling allocated, and the
 card's name and power limit read in the same run.
 
+With --au-scales (e.g. 0.5,0.6,...,1.4, or "default" for capi.AU_SCALES) every call also runs the
+AU test's multiscale bootstrap and the expected likelihood weights, and the line adds their phases:
+multiscale counts, multiscale accumulation, and statistics + ELW.
+
     python tools/bench_support.py [--taxa 500] [--sites 100000] [--replicates 1000,10000] [--reps 3]
+                                  [--au-scales default]
 """
 from __future__ import annotations
 
@@ -49,9 +54,13 @@ def main():
     ap.add_argument("--replicates", default="1000,10000")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--seed", type=int, default=0x5EED0002)
+    ap.add_argument("--au-scales", default=None, help='comma-separated scales, or "default" (capi.AU_SCALES)')
     args = ap.parse_args()
 
     from root_digger_b200 import capi, synth
+    au = None
+    if args.au_scales:
+        au = capi.AU_SCALES if args.au_scales == "default" else [float(v) for v in args.au_scales.split(",")]
     device = card()
     top = synth.random_tree(args.taxa, args.seed)
     rates, freqs = synth.random_params(args.seed + 1)
@@ -72,16 +81,26 @@ def main():
         ckp.close()
         results = {}
         for B in [int(b) for b in args.replicates.split(",")]:
-            m.placement_support(prefix, replicates=B, seed=1)  # warm-up: module load, allocations
-            runs = [m.placement_support(prefix, replicates=B, seed=1 + i) for i in range(args.reps)]
-            med = {k: statistics.median(r[k] for r in runs)
-                   for k in ("capture_ms", "counts_ms", "accumulate_ms", "statistics_ms", "resample_ms")}
+            m.placement_support(prefix, replicates=B, seed=1, au_scales=au)  # warm-up: module load, allocations
+            runs = [m.placement_support(prefix, replicates=B, seed=1 + i, au_scales=au) for i in range(args.reps)]
+            keys = ["capture_ms", "counts_ms", "accumulate_ms", "statistics_ms", "resample_ms"]
+            if au:
+                keys += ["au_counts_ms", "au_accumulate_ms", "au_statistics_ms"]
+            med = {k: statistics.median(r[k] for r in runs) for k in keys}
             med["accumulate_terms_per_s"] = B * P * R / (med["accumulate_ms"] / 1e3)
             med["device_bytes"] = max(r["device_bytes"] for r in runs)
             med["bp_sum"] = int(runs[0]["bp_count"].sum())
+            if au:
+                extra = len(au) - (1 if 1.0 in au else 0)  # scales resampled beyond the unit scale
+                med["au_terms_per_s"] = B * P * R * extra / (med["au_accumulate_ms"] / 1e3)
+                med["au_extra_scales"] = extra
+                med["elw_sum"] = float(runs[0]["elw"].sum())
             results[str(B)] = med
-    print(json.dumps({"tool": "bench_support", "taxa": args.taxa, "patterns": P, "records": R, "cats": args.cats,
-                      "reps": args.reps, "card": device, "results": results}))
+    line = {"tool": "bench_support", "taxa": args.taxa, "patterns": P, "records": R, "cats": args.cats,
+            "reps": args.reps, "card": device, "results": results}
+    if au:
+        line["au_scales"] = list(au)
+    print(json.dumps(line))
 
 
 if __name__ == "__main__":
