@@ -229,6 +229,13 @@ int rdk_sweep_root_placements(rdk_partition_t *partition,
  * storing it whenever no later operation of the sweep reads it back from memory.  The
  * log-likelihoods are unchanged. */
 #define RDK_SWEEP_DISCARD 2u
+/* RDK_SWEEP_ROWS: the evaluation of placement q also stores every pattern's UNWEIGHTED
+ * log-likelihood (the value rdk_compute_root_loglikelihood_row stores, before the pattern weight)
+ * into row q of the partition's site matrix, which rdk_partition_set_site_lnl_rows must have
+ * reserved with at least `placements` rows (the call fails before any work otherwise).  On a site
+ * shard the rows hold the local patterns.  out_lnl is unchanged, bit for bit.  Combines with the
+ * other flags and with rdk_sweep_root_placements_chunks. */
+#define RDK_SWEEP_ROWS 4u
 int rdk_sweep_root_placements_ex(rdk_partition_t *partition,
                                  unsigned int placements,
                                  const unsigned int *params_indices,
@@ -408,6 +415,12 @@ double rdk_compute_root_loglikelihood_row(rdk_partition_t *partition, unsigned i
 /* copy rows [first, first + count) of that matrix to out ([count][local patterns]) */
 int rdk_partition_get_site_lnl_rows(rdk_partition_t *partition, unsigned int first,
                                     unsigned int count, double *out);
+
+/* reorder the first `count` rows of that matrix on the device: row r afterwards holds what row
+ * order[r] held before (order is a permutation of 0..count-1).  A placement sweep captures rows in
+ * its own placement order; this puts them in the order the statistics below index records by. */
+int rdk_partition_permute_site_lnl_rows(rdk_partition_t *partition, unsigned int count,
+                                        const unsigned int *order);
 
 /* RELL bootstrap proportions and one-sided KH / SH tests over `rows` records whose per-pattern
  * log-likelihoods L are rows 0..rows-1 of the site matrices of n partitions (all on one device),

@@ -22,6 +22,7 @@ RDK_GAMMA_RATES_MEDIAN = 1
 RDK_SHARD_ALIGN = 256
 RDK_SWEEP_KEEP_ROOT = 1
 RDK_SWEEP_DISCARD = 2
+RDK_SWEEP_ROWS = 4
 # the scales of the AU test's multiscale bootstrap that CONSEL and IQ-TREE use by default
 AU_SCALES = (0.5, 0.6, 0.7, 0.8, 0.9, 1.0, 1.1, 1.2, 1.3, 1.4)
 
@@ -177,6 +178,7 @@ def load_engine() -> C.CDLL:
     L.rdk_compute_root_loglikelihood_row.argtypes = [_pp, C.c_uint, C.c_int, C.c_uint]
     L.rdk_compute_root_loglikelihood_row.restype = C.c_double
     L.rdk_partition_get_site_lnl_rows.argtypes = [_pp, C.c_uint, C.c_uint, _dp]
+    L.rdk_partition_permute_site_lnl_rows.argtypes = [_pp, C.c_uint, _up]
     _engine_lib = L
     return L
 
@@ -308,6 +310,12 @@ class Partition:
         if self.L.rdk_partition_get_site_lnl_rows(self.p, first, count, _ptr(out, _dp)) != 1:
             raise EngineError(_err(self.L))
         return out
+
+    def permute_site_lnl_rows(self, order):
+        """row r afterwards holds what row order[r] held (order: a permutation of 0..len(order)-1)"""
+        o = np.ascontiguousarray(order, dtype=np.uint32)
+        if self.L.rdk_partition_permute_site_lnl_rows(self.p, len(o), _ptr(o, _up)) != 1:
+            raise EngineError(_err(self.L))
 
     def root_loglikelihood_multi(self, root_op, branch_length_pairs):
         bl = np.ascontiguousarray(branch_length_pairs, dtype=np.float64).reshape(-1)
@@ -820,6 +828,10 @@ def _bind_model(L: C.CDLL):
                                                  C.c_uint, C.POINTER(ull), _dp, _dp, _dp, C.POINTER(ull),
                                                  C.POINTER(C.c_longlong), _up, _up, _up, _up, _dp, _dp, _dp, _dp,
                                                  _up, _dp, C.POINTER(ull), C.POINTER(C.c_int), _up, _dp, _up]
+    L.rdh_model_branch_support.argtypes = [vp, C.c_char_p, ull, ull, C.c_double, C.c_uint, C.c_int, C.c_uint, _up,
+                                           C.c_uint, C.POINTER(ull), _dp, _dp, _dp, C.POINTER(ull),
+                                           C.POINTER(C.c_longlong), _up, _up, _up, _up, _dp, _dp, _dp, _dp, _up, _dp,
+                                           C.POINTER(ull), C.POINTER(C.c_int), _up, _dp, _up]
     L.rdh_placement_au_fit.argtypes = [_up, C.c_uint, _up, ull, _dp, _up]
     L.rdh_model_site_lnl_rows.argtypes = [vp, C.c_uint, _dp, ull, _up, C.c_uint, C.POINTER(ull)]
     L.rdh_model_assign_indicies.argtypes = [vp, C.c_int, C.c_uint, C.c_double, C.c_uint, C.c_uint, C.c_int, _up,
@@ -1317,9 +1329,59 @@ class Model:
                 "elw": elw[:n].copy(), "elw_fixed": elw_fixed[:n].copy(), "au_counts_ms": info[6],
                 "au_accumulate_ms": info[7], "au_statistics_ms": info[8]}
 
+    def branch_support(self, checkpoint_prefix: str | None = None, replicates: int = 10000, seed: int = 0,
+                       atol: float = 1e-14, replicate_tile: int = 0, keep_rows: bool = False, au_scales=None) -> dict:
+        """The statistics of placement_support for EVERY branch, at one set of parameters (DESIGN.md
+        section 10, items 9-10): the parameters of the best record of "<checkpoint_prefix>.ckp" (None:
+        the model's own result log; highest llh, lowest log index on ties) are installed, root q is
+        put at a_q, its best position on its branch (optimize_alpha from 0.5 with tolerance atol, as
+        optimize_root_location polishes a candidate; atol = 0: 0.5 everywhere, the placements
+        suggest_roots_lh ranks), and record q is the placement (q, a_q), for every root id q in
+        order.  The substitution parameters are NOT re-optimised per branch, as exhaustive mode does.
+        Returns the keys of placement_support (with or without au_scales): root_id = 0..root_count-1,
+        alpha = a_q, llh = the log-likelihood at (q, a_q); plus positions_ms (the alpha searches).
+        capture_ms is the one placement sweep that scores all branches and stores their rows.  Every
+        branch carries BP, pKH, pSH (pAU, ELW) and its LLH and alpha in newick(True)."""
+        prefix = checkpoint_prefix.encode() if checkpoint_prefix is not None else None
+        sc = np.ascontiguousarray(au_thousandths(au_scales) if au_scales is not None else [], dtype=np.uint32)
+        K, n = len(sc), self.root_count
+        ull = C.POINTER(C.c_ulonglong)
+        ids = np.zeros(n, dtype=np.uint64)
+        alpha, llh, fixed = np.zeros(n), np.zeros(n), np.zeros(n)
+        o_lo, o_hi = np.zeros(n, dtype=np.uint64), np.zeros(n, dtype=np.int64)
+        bp, kh, sh, used = (np.zeros(n, dtype=np.uint32) for _ in range(4))
+        counts = np.zeros((max(1, K), n), dtype=np.uint32)
+        p_au, d, c, rss, elw = (np.zeros(n) for _ in range(5))
+        elw_fixed = np.zeros(n, dtype=np.uint64)
+        exponent, best, got = C.c_int(), C.c_uint(), C.c_uint()
+        info = np.zeros(10)
+        self._check(self.L.rdh_model_branch_support(
+            self.h, prefix, int(replicates), int(seed) & ((1 << 64) - 1), float(atol), int(replicate_tile),
+            1 if keep_rows else 0, K, _ptr(sc, _up) if K else None, n, _ptr(ids, ull), _ptr(alpha, _dp),
+            _ptr(llh, _dp), _ptr(fixed, _dp), _ptr(o_lo, ull), _ptr(o_hi, C.POINTER(C.c_longlong)), _ptr(bp, _up),
+            _ptr(kh, _up), _ptr(sh, _up), _ptr(counts, _up), _ptr(p_au, _dp), _ptr(d, _dp), _ptr(c, _dp),
+            _ptr(rss, _dp), _ptr(used, _up), _ptr(elw, _dp), _ptr(elw_fixed, ull), C.byref(exponent), C.byref(best),
+            _ptr(info, _dp), C.byref(got)))
+        n = got.value
+        self._support_rows = n if keep_rows else 0
+        B = float(replicates)
+        O = [(int(h) << 64) | int(l) for l, h in zip(o_lo[:n], o_hi[:n])]
+        out = {"root_id": ids[:n].copy(), "alpha": alpha[:n].copy(), "llh": llh[:n].copy(),
+               "lnl_fixed": fixed[:n].copy(), "O": O, "bp_count": bp[:n].copy(), "kh_count": kh[:n].copy(),
+               "sh_count": sh[:n].copy(), "bp": bp[:n] / B, "p_kh": kh[:n] / B, "p_sh": sh[:n] / B,
+               "exponent": exponent.value, "best": best.value, "replicates": int(replicates),
+               "capture_ms": info[0], "counts_ms": info[1], "accumulate_ms": info[2], "statistics_ms": info[3],
+               "resample_ms": info[4], "device_bytes": int(info[5]), "positions_ms": info[9]}
+        if K:
+            out.update({"scales": sc / 1000.0, "scale_counts": counts[:, :n].copy(), "p_au": p_au[:n].copy(),
+                        "au_d": d[:n].copy(), "au_c": c[:n].copy(), "au_rss": rss[:n].copy(),
+                        "au_used": used[:n].copy(), "elw": elw[:n].copy(), "elw_fixed": elw_fixed[:n].copy(),
+                        "au_counts_ms": info[6], "au_accumulate_ms": info[7], "au_statistics_ms": info[8]})
+        return out
+
     def site_lnl_rows(self, part: int = 0):
         """(rows [record][pattern], pattern weights) of partition `part` from the last
-        placement_support(..., keep_rows=True)"""
+        placement_support(..., keep_rows=True) or branch_support(..., keep_rows=True)"""
         P = self.sites(part)
         rows = getattr(self, "_support_rows", 0)
         buf = np.zeros(max(1, rows * P))

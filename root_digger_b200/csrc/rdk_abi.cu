@@ -188,6 +188,7 @@ struct Engine {
   double *d_rows = nullptr;    // [rows_cap][S]: unweighted per-pattern values (rdk_partition_set_site_lnl_rows)
   unsigned rows_cap = 0;
   double  *want_row = nullptr; // the row the next evaluation stores into, or null
+  double  *want_rows = nullptr; // RDK_SWEEP_ROWS: eval slot s of the next program stores into want_rows + s * S
   double *h_results = nullptr;  // pinned, device-visible
   size_t  results_cap = 0;      // doubles
 
@@ -557,18 +558,19 @@ int launch_lowered(rdk_partition_t *p, ProgArgs &a, const std::vector<LInstr> &l
   if (a.nelem == 0 || a.n_instr == 0) return RDK_SUCCESS;
   LaunchSeg seg[2];
   const int n_seg = plan_segments(e, n_witer, chunked ? a.n_chunks : 1u, a.n_instr, seg);
+  const bool rows = a.row_stride != 0;  // the ROWS variant (flush, RDK_SWEEP_ROWS)
   for (int g = 0; g < n_seg; ++g) {
     const LaunchPlan &pl = seg[g].pl;
     a.it0 = seg[g].it0;
     a.n_witer = seg[g].n_witer;
     cudaError_t lerr;
     switch (e->K) {
-      case 1: lerr = launch_program<1>(a, pl.grid, pl.threads, pl.E, e->stream); break;
-      case 2: lerr = launch_program<2>(a, pl.grid, pl.threads, pl.E, e->stream); break;
-      case 4: lerr = launch_program<4>(a, pl.grid, pl.threads, pl.E, e->stream); break;
-      case 8: lerr = launch_program<8>(a, pl.grid, pl.threads, pl.E, e->stream); break;
-      case 16: lerr = launch_program<16>(a, pl.grid, pl.threads, pl.E, e->stream); break;
-      case 32: lerr = launch_program<32>(a, pl.grid, pl.threads, pl.E, e->stream); break;
+      case 1: lerr = launch_program<1>(a, pl.grid, pl.threads, pl.E, rows, e->stream); break;
+      case 2: lerr = launch_program<2>(a, pl.grid, pl.threads, pl.E, rows, e->stream); break;
+      case 4: lerr = launch_program<4>(a, pl.grid, pl.threads, pl.E, rows, e->stream); break;
+      case 8: lerr = launch_program<8>(a, pl.grid, pl.threads, pl.E, rows, e->stream); break;
+      case 16: lerr = launch_program<16>(a, pl.grid, pl.threads, pl.E, rows, e->stream); break;
+      case 32: lerr = launch_program<32>(a, pl.grid, pl.threads, pl.E, rows, e->stream); break;
       default: return fail(RDK_ERROR_PARAM, "rate_cats must divide 32");
     }
     if (lerr != cudaSuccess) return fail(RDK_ERROR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(lerr));
@@ -758,6 +760,11 @@ int flush(rdk_partition_t *p) {
   // a row of unweighted values takes the place of the weighted per-site output (never both)
   a.persite = e->want_row ? e->want_row : (e->want_persite ? e->d_persite : nullptr);
   a.persite_unweighted = e->want_row != nullptr;
+  if (e->want_rows) {  // a sweep batch capturing rows: the ROWS variant of the kernel, one row per eval slot
+    a.persite = e->want_rows;
+    a.persite_unweighted = 1;
+    a.row_stride = e->S;
+  }
   // recorded operations -> the instructions the kernel walks (rdk_lower.hpp)
   HostTimer             lower_timer(&e->stats.host_lower_ns);  // lowering, pointer translation, enqueue
   const bool            chunked = e->pend_chunk_off.size() > 2;
@@ -1459,6 +1466,39 @@ extern "C" int rdk_partition_get_site_lnl_rows(rdk_partition_t *p, unsigned int 
   return RDK_SUCCESS;
 }
 
+extern "C" int rdk_partition_permute_site_lnl_rows(rdk_partition_t *p, unsigned int count,
+                                                   const unsigned int *order) {
+  Engine *e = eng(p);
+  if (count > e->rows_cap) return fail(RDK_ERROR_PARAM, "site rows out of range");
+  std::vector<char> seen(count, 0);
+  for (unsigned r = 0; r < count; ++r) {
+    if (order[r] >= count || seen[order[r]]) return fail(RDK_ERROR_PARAM, "order is not a permutation of the rows");
+    seen[order[r]] = 1;
+  }
+  std::lock_guard<std::mutex> lk(e->mu);
+  CUDA_TRY(cudaSetDevice(e->device));
+  if (!flush(p)) return RDK_FAILURE;
+  if (e->S == 0) return RDK_SUCCESS;
+  // cycle by cycle, in place, through the per-site scratch row (S doubles)
+  const size_t bytes = sizeof(double) * e->S;
+  auto row = [&](unsigned r) { return e->d_rows + (size_t)r * e->S; };
+  std::fill(seen.begin(), seen.end(), 0);
+  for (unsigned r0 = 0; r0 < count; ++r0) {
+    if (seen[r0] || order[r0] == r0) continue;
+    CUDA_TRY(cudaMemcpyAsync(e->d_persite, row(r0), bytes, cudaMemcpyDeviceToDevice, e->stream));
+    unsigned r = r0;
+    while (order[r] != r0) {
+      seen[r] = 1;
+      CUDA_TRY(cudaMemcpyAsync(row(r), row(order[r]), bytes, cudaMemcpyDeviceToDevice, e->stream));
+      r = order[r];
+    }
+    seen[r] = 1;
+    CUDA_TRY(cudaMemcpyAsync(row(r), e->d_persite, bytes, cudaMemcpyDeviceToDevice, e->stream));
+  }
+  CUDA_TRY(cudaStreamSynchronize(e->stream));
+  return RDK_SUCCESS;
+}
+
 static int rell_entry(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
                       unsigned int rows, unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
                       rdk_rell_ms_out_t *ms) {
@@ -1655,6 +1695,9 @@ extern "C" int rdk_sweep_root_placements_chunks(rdk_partition_t *p, unsigned int
     if (!(branch_lengths[i] >= 0.0) || !std::isfinite(branch_lengths[i]))
       return fail(RDK_ERROR_PARAM, "branch length must be finite and non-negative");
   }
+  if ((flags & RDK_SWEEP_ROWS) && e->rows_cap < placements)
+    return fail(RDK_ERROR_PARAM, "RDK_SWEEP_ROWS: %u placements, %u site rows reserved (rdk_partition_set_site_lnl_rows)",
+                placements, e->rows_cap);
   std::lock_guard<std::mutex> lk(e->mu);
   CUDA_TRY(cudaSetDevice(e->device));
   if (!flush(p)) return RDK_FAILURE;
@@ -1801,7 +1844,10 @@ extern "C" int rdk_sweep_root_placements_chunks(rdk_partition_t *p, unsigned int
       e->pend_scratch_clv = &scratch_clv[batch];
       e->pend_scratch_sc = &scratch_sc[batch];
     }
+    // RDK_SWEEP_ROWS: eval slot s of this batch is placement done + s, and stores into that row
+    if (flags & RDK_SWEEP_ROWS) e->want_rows = e->d_rows + (size_t)done * e->S;
     int ok = flush(p);
+    e->want_rows = nullptr;
     e->pend_scratch_clv = e->pend_scratch_sc = nullptr;
     e->pend_slots = 0;
     if (!ok) return RDK_FAILURE;

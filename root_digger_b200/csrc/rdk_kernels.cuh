@@ -470,7 +470,7 @@ struct ProgArgs {
   const unsigned* weights;  // pattern weights [sites]
   double*         partials; // [slots][partial_stride], one value per warp iteration
   unsigned        partial_stride;
-  double*         persite;  // optional, eval slot 0 only
+  double*         persite;  // optional, eval slot 0 only (the ROWS variant: every eval slot, see row_stride)
   unsigned        persite_unweighted;  // persite receives the values before the pattern weight
   double          pi[4];
   double          w[kMaxCats];
@@ -481,6 +481,10 @@ struct ProgArgs {
   unsigned        n_chunks;
   unsigned        chunk_off[kMaxChunks + 1];
   Instr           inl[kProgInline];
+  // the ROWS variant of the kernel (placement sweeps that capture per-pattern rows): eval slot s
+  // stores its UNWEIGHTED values at persite + s * row_stride.  Last, so that the fields the other
+  // variants read keep their offsets.
+  size_t          row_stride;
 };
 
 // the table ring of one CTA
@@ -574,7 +578,9 @@ constexpr int kScaleThresholdHi = (1023 - 256) << 20;
 // back-off of the producer warp while its ring is full (200 / 1000 / 4000 ns measured the same on B200)
 constexpr unsigned kProducerSleepNs = 200;
 
-template <int K, int E, int MAXT, int MINB>
+// ROWS: every evaluation stores its unweighted per-pattern values into the row of its eval slot
+// (a compile-time variant, so that the instantiations without it compile to the code they had)
+template <int K, int E, int MAXT, int MINB, bool ROWS = false>
 __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_constant__ ProgArgs a) {
   static_assert(32 % K == 0, "K must divide the warp size");
   using R = Ring<K>;
@@ -844,7 +850,8 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
           l = rd_log(x);
           if (fl & fEvalScaler) l = dadd(l, dmul((double)cn, RDK_LOG_SCALE_THRESHOLD));
           const double lw = dmul(l, (double)wg);
-          if (a.persite && eslot == 0) a.persite[st] = a.persite_unweighted ? l : lw;
+          if constexpr (ROWS) a.persite[(size_t)eslot * a.row_stride + st] = l;
+          else if (a.persite && eslot == 0) a.persite[st] = a.persite_unweighted ? l : lw;
           l = lw;
         }
         // canonical tree over the 32/K sites of a warp iteration (the lanes of equal k)
@@ -859,7 +866,8 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
             l = rd_log(term[u]);
             if (fl & fEvalScaler) l = dadd(l, dmul((double)cnt[u], RDK_LOG_SCALE_THRESHOLD));
             const double lw = dmul(l, (double)wgt[u]);
-            if (a.persite && eslot == 0) a.persite[site[u]] = a.persite_unweighted ? l : lw;
+            if constexpr (ROWS) a.persite[(size_t)eslot * a.row_stride + site[u]] = l;
+            else if (a.persite && eslot == 0) a.persite[site[u]] = a.persite_unweighted ? l : lw;
             l = lw;
           }
 #pragma unroll
@@ -999,14 +1007,15 @@ __global__ void __launch_bounds__(MAXT, MINB) clv_program_kernel(const __grid_co
 // each in its own translation unit (rdk_program_inst.cu).  `threads` counts the producer warp.
 // Returns the CUDA status of the launch configuration (the launch itself is checked by the
 // caller with cudaGetLastError).
+// rows != 0 launches the ROWS variant (ProgArgs::row_stride).
 template <int K>
-cudaError_t launch_program(const ProgArgs& a, int grid, int threads, int E, cudaStream_t st);
-template <> cudaError_t launch_program<1>(const ProgArgs&, int, int, int, cudaStream_t);
-template <> cudaError_t launch_program<2>(const ProgArgs&, int, int, int, cudaStream_t);
-template <> cudaError_t launch_program<4>(const ProgArgs&, int, int, int, cudaStream_t);
-template <> cudaError_t launch_program<8>(const ProgArgs&, int, int, int, cudaStream_t);
-template <> cudaError_t launch_program<16>(const ProgArgs&, int, int, int, cudaStream_t);
-template <> cudaError_t launch_program<32>(const ProgArgs&, int, int, int, cudaStream_t);
+cudaError_t launch_program(const ProgArgs& a, int grid, int threads, int E, bool rows, cudaStream_t st);
+template <> cudaError_t launch_program<1>(const ProgArgs&, int, int, int, bool, cudaStream_t);
+template <> cudaError_t launch_program<2>(const ProgArgs&, int, int, int, bool, cudaStream_t);
+template <> cudaError_t launch_program<4>(const ProgArgs&, int, int, int, bool, cudaStream_t);
+template <> cudaError_t launch_program<8>(const ProgArgs&, int, int, int, bool, cudaStream_t);
+template <> cudaError_t launch_program<16>(const ProgArgs&, int, int, int, bool, cudaStream_t);
+template <> cudaError_t launch_program<32>(const ProgArgs&, int, int, int, bool, cudaStream_t);
 // the launch shapes the kernel is compiled for, per elements-per-thread E: threads per CTA
 // (producer warp included) and CTAs per SM
 struct LaunchShape {

@@ -22,6 +22,7 @@
 #ifdef RD_BACKEND_ORACLE
 #include "rdk_support.h"     // tests/oracle_shim: the placement-support entries over the CPU oracle
 #include "rdk_support_au.h"  // ... and rdk_rell_support_ms
+#include "rdk_sweep_rows.h"   // ... and the row capture of the placement sweep
 #endif
 #include "support_stats.hpp"
 
@@ -29,6 +30,7 @@
 #include <chrono>
 #include <cmath>
 #include <exception>
+#include <functional>
 #include <cstdlib>
 #include <cstring>
 #include <limits>
@@ -638,6 +640,34 @@ std::vector<root_location_t> model_t::suggest_roots_random(size_t min, double ra
   return roots;
 }
 
+// The directed sweep of the root ids [begin, end) from the current root, cut into _sweep_chunks
+// ranges of consecutive root ids, each with its own spare buffers (and its own copy of the directed
+// CLVs on the path to its first placement): independent programs the engine may walk side by side.
+// `ratio` as rooted_tree_t::generate_sweep_operations takes it; chunk_off receives the chunk offsets.
+rooted_tree_t::sweep_schedule_t model_t::directed_sweep_schedule(size_t begin, size_t end,
+                                                                 const std::vector<double> &ratio,
+                                                                 std::vector<unsigned int> &chunk_off) const {
+  const size_t                    total = end - begin;
+  const unsigned int              chunks = (unsigned int)std::max<size_t>(1, std::min<size_t>(_sweep_chunks, total / 8));
+  rooted_tree_t::sweep_schedule_t sw;
+  chunk_off.assign(1, 0u);
+  for (unsigned int c = 0; c < chunks; ++c) {
+    const size_t b0 = begin + total * c / chunks, b1 = begin + total * (c + 1) / chunks;
+    auto part = _tree.generate_sweep_operations(b0, b1, _tree.tip_count() + _tree.branch_count() + c * _sweep_extra,
+                                                (int)(_tree.branch_count() + c * _sweep_extra),
+                                                _tree.branch_count(), _sweep_extra, ratio);
+    const unsigned int pm_base = (unsigned int)sw.mi.size(), op_base = (unsigned int)sw.ops.size();
+    sw.mi.insert(sw.mi.end(), part.mi.begin(), part.mi.end());
+    sw.bl.insert(sw.bl.end(), part.bl.begin(), part.bl.end());
+    sw.ops.insert(sw.ops.end(), part.ops.begin(), part.ops.end());
+    for (size_t q = 1; q < part.pm_off.size(); ++q) sw.pm_off.push_back(pm_base + part.pm_off[q]);
+    for (size_t q = 1; q < part.op_off.size(); ++q) sw.op_off.push_back(op_base + part.op_off[q]);
+    sw.root_pos.insert(sw.root_pos.end(), part.root_pos.begin(), part.root_pos.end());
+    chunk_off.push_back((unsigned int)sw.root_pos.size());
+  }
+  return sw;
+}
+
 // log-likelihood of every root placement at its stored ratio, in root-id order:
 // what the loop at src/model.cpp:871-874 computes (move_root + compute_lh_root
 // per root).  With the fused path the whole sweep is ONE engine call.
@@ -665,28 +695,10 @@ std::vector<double> model_t::sweep_root_lh(size_t begin, size_t end) {
   }
   if (_sweep_mode == sweep_mode_t::directed) {
     // one pre-order pass over directed CLVs from the current root; same bits as the loop
-    // above (tree.hpp), ~1 CLV operation + 1 root evaluation per placement
-    // cut into _sweep_chunks ranges of consecutive root ids, each with its own spare buffers
-    // (and its own copy of the directed CLVs on the path to its first placement): independent
-    // programs the engine may walk side by side
-    const size_t                 total = end - begin;
-    const unsigned int           chunks = (unsigned int)std::max<size_t>(1, std::min<size_t>(_sweep_chunks, total / 8));
-    rooted_tree_t::sweep_schedule_t sw;
-    std::vector<unsigned int>    chunk_off{0};
-    for (unsigned int c = 0; c < chunks; ++c) {
-      const size_t b0 = begin + total * c / chunks, b1 = begin + total * (c + 1) / chunks;
-      auto part = _tree.generate_sweep_operations(b0, b1, _tree.tip_count() + _tree.branch_count() + c * _sweep_extra,
-                                                  (int)(_tree.branch_count() + c * _sweep_extra),
-                                                  _tree.branch_count(), _sweep_extra);
-      const unsigned int pm_base = (unsigned int)sw.mi.size(), op_base = (unsigned int)sw.ops.size();
-      sw.mi.insert(sw.mi.end(), part.mi.begin(), part.mi.end());
-      sw.bl.insert(sw.bl.end(), part.bl.begin(), part.bl.end());
-      sw.ops.insert(sw.ops.end(), part.ops.begin(), part.ops.end());
-      for (size_t q = 1; q < part.pm_off.size(); ++q) sw.pm_off.push_back(pm_base + part.pm_off[q]);
-      for (size_t q = 1; q < part.op_off.size(); ++q) sw.op_off.push_back(op_base + part.op_off[q]);
-      sw.root_pos.insert(sw.root_pos.end(), part.root_pos.begin(), part.root_pos.end());
-      chunk_off.push_back((unsigned int)sw.root_pos.size());
-    }
+    // above (tree.hpp), ~1 CLV operation + 1 root evaluation per placement, in chunks
+    std::vector<unsigned int>       chunk_off;
+    const rooted_tree_t::sweep_schedule_t sw = directed_sweep_schedule(begin, end, {}, chunk_off);
+    const unsigned int              chunks = (unsigned int)chunk_off.size() - 1;
     std::vector<double> part(sw.root_pos.size());
     for (size_t i = 0; i < _partitions.size(); ++i) {
       int rc = rdk_sweep_root_placements_chunks(_partitions[i], (unsigned)sw.root_pos.size(),
@@ -950,23 +962,22 @@ std::pair<root_location_t, double> model_t::exhaustive_search(double atol, doubl
 // ---------------------------------------------------------------------------
 // root placement support (DESIGN.md section 10)
 // ---------------------------------------------------------------------------
-model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
-                                                        unsigned replicate_tile, bool keep_rows,
-                                                        const std::vector<unsigned> &au_scales) {
+// what both support calls refuse before any work
+void model_t::check_support_request(const std::string &who, size_t replicates,
+                                    const std::vector<unsigned> &au_scales) const {
   if (_exchange)
-    throw std::invalid_argument("placement_support: a model whose partitions are dealt to several processes is "
-                                "not supported");
+    throw std::invalid_argument(who + ": a model whose partitions are dealt to several processes is not supported");
   if (replicates == 0 || replicates > (size_t(1) << 20))
-    throw std::invalid_argument("placement_support: replicates must be between 1 and 2^20");
-  const bool au = !au_scales.empty();
-  if (au) rd::check_au_scales(au_scales.data(), au_scales.size());
-  const auto records = checkpoint.read_results();
-  if (records.empty()) throw std::invalid_argument("placement_support: the checkpoint holds no records");
-  if (records.size() > std::numeric_limits<unsigned>::max())
-    throw std::invalid_argument("placement_support: too many records");
+    throw std::invalid_argument(who + ": replicates must be between 1 and 2^20");
+  if (!au_scales.empty()) rd::check_au_scales(au_scales.data(), au_scales.size());
+}
+
+void model_t::check_support_records(const std::string &who, const std::vector<checkpoint_t::record_t> &records) const {
+  if (records.empty()) throw std::invalid_argument(who + ": the checkpoint holds no records");
+  if (records.size() > std::numeric_limits<unsigned>::max()) throw std::invalid_argument(who + ": too many records");
   for (size_t r = 0; r < records.size(); ++r) {
     const auto &rec = records[r];
-    const std::string which = "placement_support: record " + std::to_string(r) + " (root id " +
+    const std::string which = who + ": record " + std::to_string(r) + " (root id " +
                               std::to_string(rec.first.root_id) + ")";
     if (rec.first.root_id >= _tree.root_count()) throw std::invalid_argument(which + ": root id out of range");
     if (!(rec.first.alpha >= 0.0 && rec.first.alpha <= 1.0))
@@ -984,8 +995,23 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
                                     " do not match the model");
     }
   }
+}
 
-  // what is put back afterwards: the installed parameters and the rooting
+// installed as optimize_params installs them: a record holds the optimiser's variables, whose
+// frequencies are normalised on the way in (set_model_params would take them as they are)
+void model_t::install_record(const checkpoint_t::record_t &record) {
+  for (size_t p = 0; p < _partitions.size(); ++p) {
+    const auto &pp = record.second[p];
+    set_subst_rates(p, pp.subst_rates);
+    set_freqs_all_free(p, pp.freqs);
+    set_gamma_rates(p, pp.gamma_alpha);
+    if (_rate_category_types[p] == rate_category::FREE) set_gamma_weights(p, pp.gamma_weights);
+  }
+}
+
+// what is put back after a support call: the installed parameters and the rooting (and the row
+// matrix is freed unless keep_rows)
+std::function<void()> model_t::support_restore_point(bool keep_rows) {
   struct installed_t {
     std::vector<double> subst, freqs, rates, weights, rate_rates;
   };
@@ -1001,7 +1027,7 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
   }
   const bool            was_rooted = _tree.rooted();
   const root_location_t was_root = _tree.root_location();
-  auto restore = [&]() {
+  return [this, installed, was_rooted, was_root, keep_rows]() {
     if (!keep_rows) {
       for (size_t p = 0; p < _partitions.size(); ++p) rdk_partition_set_site_lnl_rows(_partitions[p], 0);
       _support_rows = 0;
@@ -1020,27 +1046,113 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
       _tree.unroot();
     }
   };
+}
 
-  const unsigned rows = (unsigned)records.size();
+void model_t::reserve_support_rows(const std::string &who, unsigned rows) {
   for (size_t p = 0; p < _partitions.size(); ++p)
     if (rdk_partition_set_site_lnl_rows(_partitions[p], rows) != RDK_SUCCESS)
-      throw std::runtime_error("placement_support: " + engine_error());
+      throw std::runtime_error(who + ": " + engine_error());
   _support_rows = rows;
+}
+
+// the statistics of DESIGN.md section 10, items 2-8, over rows 0..rows-1 of the partitions' site
+// matrices (rdk_rell_support, or rdk_rell_support_ms in AU mode)
+void model_t::resample_support(const std::string &who, placement_support_t &out, unsigned rows, size_t replicates,
+                               uint64_t seed, unsigned replicate_tile, const std::vector<unsigned> &au_scales) {
+  const bool            au = !au_scales.empty();
+  std::vector<unsigned> global_index(_partitions.size());
+  std::iota(global_index.begin(), global_index.end(), 0u);
+  out.replicates = replicates;
+  out.lnl_fixed.resize(rows);
+  out.bp_count.resize(rows);
+  out.kh_count.resize(rows);
+  out.sh_count.resize(rows);
+  out.o_lo.resize(rows);
+  out.o_hi.resize(rows);
+  rdk_rell_out_t rell;
+  memset(&rell, 0, sizeof(rell));
+  rell.replicate_tile = replicate_tile;
+  rell.lnl_fixed = out.lnl_fixed.data();
+  rell.bp_count = out.bp_count.data();
+  rell.kh_count = out.kh_count.data();
+  rell.sh_count = out.sh_count.data();
+  rell.o_lo = out.o_lo.data();
+  rell.o_hi = out.o_hi.data();
+  if (au) {
+    out.scales = au_scales;
+    out.scale_count.resize(au_scales.size() * rows);
+    out.elw_fixed.resize(rows);
+    rdk_rell_ms_out_t ms;
+    memset(&ms, 0, sizeof(ms));
+    ms.scales = out.scales.data();
+    ms.n_scales = (unsigned)out.scales.size();
+    ms.scale_count = out.scale_count.data();
+    ms.elw_fixed = out.elw_fixed.data();
+    if (rdk_rell_support_ms(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows, replicates,
+                            seed, &rell, &ms) != RDK_SUCCESS)
+      throw std::runtime_error(who + ": " + engine_error());
+    out.au_counts_ms = ms.ms[0];
+    out.au_accumulate_ms = ms.ms[1];
+    out.au_statistics_ms = ms.ms[2];
+  } else if (rdk_rell_support(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows,
+                              replicates, seed, &rell) != RDK_SUCCESS) {
+    throw std::runtime_error(who + ": " + engine_error());
+  }
+  out.best = rell.best;
+  out.exponent = rell.exponent;
+  out.counts_ms = rell.ms[0];
+  out.accumulate_ms = rell.ms[1];
+  out.statistics_ms = rell.ms[2];
+  out.resample_ms = rell.ms[3];
+  out.device_bytes = rell.device_bytes;
+}
+
+// the per-record values the counts stand for, and the branch annotations: record r is the placement
+// on where[r]'s branch
+void model_t::annotate_support(placement_support_t &out, const std::vector<root_location_t> &where) {
+  const bool   au = !out.scales.empty();
+  const size_t rows = where.size();
+  const double B = (double)out.replicates;
+  for (size_t r = 0; r < rows; ++r) {
+    out.bp.push_back(out.bp_count[r] / B);
+    out.p_kh.push_back(out.kh_count[r] / B);
+    out.p_sh.push_back(out.sh_count[r] / B);
+    _tree.annotate_branch(where[r], "BP", std::to_string(out.bp[r]));
+    _tree.annotate_branch(where[r], "pKH", std::to_string(out.p_kh[r]));
+    _tree.annotate_branch(where[r], "pSH", std::to_string(out.p_sh[r]));
+    if (au) {
+      std::vector<unsigned> count(out.scales.size());
+      for (size_t k = 0; k < count.size(); ++k) count[k] = out.scale_count[k * rows + r];
+      const rd::au_fit_t fit = rd::au_fit(count.data(), out.scales.data(), count.size(), out.replicates);
+      out.p_au.push_back(fit.p_au);
+      out.au_d.push_back(fit.d);
+      out.au_c.push_back(fit.c);
+      out.au_rss.push_back(fit.rss);
+      out.au_used.push_back(fit.used);
+      out.elw.push_back(ldexp((double)out.elw_fixed[r], -40) / B);
+      _tree.annotate_branch(where[r], "pAU", std::to_string(fit.p_au));
+      _tree.annotate_branch(where[r], "ELW", std::to_string(out.elw[r]));
+    }
+  }
+}
+
+model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
+                                                        unsigned replicate_tile, bool keep_rows,
+                                                        const std::vector<unsigned> &au_scales) {
+  const std::string who = "placement_support";
+  check_support_request(who, replicates, au_scales);
+  const auto records = checkpoint.read_results();
+  check_support_records(who, records);
+
+  auto           restore = support_restore_point(keep_rows);
+  const unsigned rows = (unsigned)records.size();
+  reserve_support_rows(who, rows);
 
   placement_support_t out;
-  out.replicates = replicates;
   try {
     const auto t0 = std::chrono::steady_clock::now();
     for (unsigned r = 0; r < rows; ++r) {
-      // installed as optimize_params installs them: a record holds the optimiser's variables, whose
-      // frequencies are normalised on the way in (set_model_params would take them as they are)
-      for (size_t p = 0; p < _partitions.size(); ++p) {
-        const auto &pp = records[r].second[p];
-        set_subst_rates(p, pp.subst_rates);
-        set_freqs_all_free(p, pp.freqs);
-        set_gamma_rates(p, pp.gamma_alpha);
-        if (_rate_category_types[p] == rate_category::FREE) set_gamma_weights(p, pp.gamma_weights);
-      }
+      install_record(records[r]);
       const root_location_t rl = placement_of(records[r].first).first;
       _tree.root_by(rl);
       const traversal_t trav = full_traversal(rl);
@@ -1054,82 +1166,104 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
       }
     }
     out.capture_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-
-    std::vector<unsigned> global_index(_partitions.size());
-    std::iota(global_index.begin(), global_index.end(), 0u);
-    out.lnl_fixed.resize(rows);
-    out.bp_count.resize(rows);
-    out.kh_count.resize(rows);
-    out.sh_count.resize(rows);
-    out.o_lo.resize(rows);
-    out.o_hi.resize(rows);
-    rdk_rell_out_t rell;
-    memset(&rell, 0, sizeof(rell));
-    rell.replicate_tile = replicate_tile;
-    rell.lnl_fixed = out.lnl_fixed.data();
-    rell.bp_count = out.bp_count.data();
-    rell.kh_count = out.kh_count.data();
-    rell.sh_count = out.sh_count.data();
-    rell.o_lo = out.o_lo.data();
-    rell.o_hi = out.o_hi.data();
-    if (au) {
-      out.scales = au_scales;
-      out.scale_count.resize(au_scales.size() * rows);
-      out.elw_fixed.resize(rows);
-      rdk_rell_ms_out_t ms;
-      memset(&ms, 0, sizeof(ms));
-      ms.scales = out.scales.data();
-      ms.n_scales = (unsigned)out.scales.size();
-      ms.scale_count = out.scale_count.data();
-      ms.elw_fixed = out.elw_fixed.data();
-      if (rdk_rell_support_ms(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows,
-                              replicates, seed, &rell, &ms) != RDK_SUCCESS)
-        throw std::runtime_error("placement_support: " + engine_error());
-      out.au_counts_ms = ms.ms[0];
-      out.au_accumulate_ms = ms.ms[1];
-      out.au_statistics_ms = ms.ms[2];
-    } else if (rdk_rell_support(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows,
-                                replicates, seed, &rell) != RDK_SUCCESS) {
-      throw std::runtime_error("placement_support: " + engine_error());
-    }
-    out.best = rell.best;
-    out.exponent = rell.exponent;
-    out.counts_ms = rell.ms[0];
-    out.accumulate_ms = rell.ms[1];
-    out.statistics_ms = rell.ms[2];
-    out.resample_ms = rell.ms[3];
-    out.device_bytes = rell.device_bytes;
+    resample_support(who, out, rows, replicates, seed, replicate_tile, au_scales);
   } catch (...) {
     restore();
     throw;
   }
   restore();
 
+  std::vector<root_location_t> where;
   for (unsigned r = 0; r < rows; ++r) {
-    const double B = (double)replicates;
     out.root_id.push_back(records[r].first.root_id);
     out.alpha.push_back(records[r].first.alpha);
     out.llh.push_back(records[r].first.llh);
-    out.bp.push_back(out.bp_count[r] / B);
-    out.p_kh.push_back(out.kh_count[r] / B);
-    out.p_sh.push_back(out.sh_count[r] / B);
-    const root_location_t rl = placement_of(records[r].first).first;
-    _tree.annotate_branch(rl, "BP", std::to_string(out.bp[r]));
-    _tree.annotate_branch(rl, "pKH", std::to_string(out.p_kh[r]));
-    _tree.annotate_branch(rl, "pSH", std::to_string(out.p_sh[r]));
-    if (au) {
-      std::vector<unsigned> count(au_scales.size());
-      for (size_t k = 0; k < count.size(); ++k) count[k] = out.scale_count[k * rows + r];
-      const rd::au_fit_t fit = rd::au_fit(count.data(), au_scales.data(), count.size(), replicates);
-      out.p_au.push_back(fit.p_au);
-      out.au_d.push_back(fit.d);
-      out.au_c.push_back(fit.c);
-      out.au_rss.push_back(fit.rss);
-      out.au_used.push_back(fit.used);
-      out.elw.push_back(ldexp((double)out.elw_fixed[r], -40) / B);
-      _tree.annotate_branch(rl, "pAU", std::to_string(fit.p_au));
-      _tree.annotate_branch(rl, "ELW", std::to_string(out.elw[r]));
+    where.push_back(placement_of(records[r].first).first);
+  }
+  annotate_support(out, where);
+  return out;
+}
+
+model_t::placement_support_t model_t::branch_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
+                                                     double atol, unsigned replicate_tile, bool keep_rows,
+                                                     const std::vector<unsigned> &au_scales) {
+  const std::string who = "branch_support";
+  check_support_request(who, replicates, au_scales);
+  if (!(atol >= 0.0 && atol <= std::numeric_limits<double>::max()))
+    throw std::invalid_argument(who + ": atol must be finite and non-negative");
+  const auto records = checkpoint.read_results();
+  check_support_records(who, records);
+  size_t best = 0;  // highest llh, lowest log index on ties
+  for (size_t r = 1; r < records.size(); ++r)
+    if (records[r].first.llh > records[best].first.llh) best = r;
+
+  auto           restore = support_restore_point(keep_rows);
+  const size_t   n_roots = _tree.root_count();
+  const unsigned rows = (unsigned)n_roots;
+  reserve_support_rows(who, rows);
+
+  placement_support_t out;
+  std::vector<double> alpha(n_roots, 0.5), llh(n_roots, 0.0);
+  try {
+    install_record(records[best]);
+    const root_location_t at = placement_of(records[best].first).first;
+    for (size_t q = 0; !_tree.can_root_by(at) && q < n_roots; ++q)  // an unrooted tree: root it elsewhere first
+      if (_tree.can_root_by(_tree.root_location(q))) _tree.root_by(_tree.root_location(q));
+    compute_lh(at);
+    // a_q: the position optimize_root_location would polish root q to, from ratio 0.5
+    const auto t0 = std::chrono::steady_clock::now();
+    if (atol > 0.0) {
+      for (size_t q = 0; q < n_roots; ++q) {
+        const root_location_t rl = _tree.root_location(q);
+        move_root(rl);
+        alpha[q] = optimize_alpha(rl, atol).brlen_ratio;
+      }
     }
+    const auto t1 = std::chrono::steady_clock::now();
+    out.positions_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
+    compute_lh(at);  // the sweep starts from valid CLVs of one rooting
+
+    // one directed sweep over every placement (q, a_q) that also stores the rows, in sweep order;
+    // then the rows are put in root-id order, the order the statistics index records by
+    const auto t2 = std::chrono::steady_clock::now();
+    std::vector<unsigned int>       chunk_off;
+    const rooted_tree_t::sweep_schedule_t sw = directed_sweep_schedule(0, n_roots, alpha, chunk_off);
+    std::vector<unsigned int> order(n_roots);
+    for (size_t q = 0; q < sw.root_pos.size(); ++q) order[sw.root_pos[q]] = (unsigned)q;
+    std::vector<double> part(sw.root_pos.size());
+    for (size_t i = 0; i < _partitions.size(); ++i) {
+      if (rdk_sweep_root_placements_chunks(_partitions[i], (unsigned)sw.root_pos.size(), _param_indicies[i].data(),
+                                           _param_indicies[i].data(), sw.pm_off.data(), sw.mi.data(), sw.bl.data(),
+                                           sw.op_off.data(), sw.ops.data(), _tree.root_clv_index(),
+                                           _tree.root_scaler_index(),
+                                           RDK_SWEEP_KEEP_ROOT | RDK_SWEEP_DISCARD | RDK_SWEEP_ROWS,
+                                           (unsigned)chunk_off.size() - 1, chunk_off.data(),
+                                           part.data()) == RDK_FAILURE ||
+          rdk_partition_permute_site_lnl_rows(_partitions[i], rows, order.data()) == RDK_FAILURE)
+        throw std::runtime_error(who + ": " + engine_error());
+      for (size_t q = 0; q < part.size(); ++q) llh[sw.root_pos[q]] += part[q];
+    }
+    out.capture_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t2).count();
+    for (double v : llh)
+      if (std::isnan(v)) throw std::runtime_error(who + ": lh at root is not a number");
+    resample_support(who, out, rows, replicates, seed, replicate_tile, au_scales);
+  } catch (...) {
+    restore();
+    throw;
+  }
+  restore();
+
+  std::vector<root_location_t> where;
+  for (size_t q = 0; q < n_roots; ++q) {
+    out.root_id.push_back(q);
+    where.push_back(_tree.root_location(q));
+  }
+  out.alpha = alpha;
+  out.llh = llh;
+  annotate_support(out, where);
+  for (size_t q = 0; q < n_roots; ++q) {
+    _tree.annotate_lh(where[q], llh[q]);
+    _tree.annotate_ratio(where[q], alpha[q]);
   }
   return out;
 }

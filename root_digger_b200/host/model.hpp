@@ -203,11 +203,25 @@ public:
     std::vector<double>             p_au, au_d, au_c, au_rss, elw;
     std::vector<unsigned long long> elw_fixed;
     double                          au_counts_ms = 0, au_accumulate_ms = 0, au_statistics_ms = 0;
+    double                          positions_ms = 0;  // branch_support: the alpha searches
   };
   placement_support_t placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
                                         unsigned replicate_tile = 0, bool keep_rows = false,
                                         const std::vector<unsigned> &au_scales = {});
-  // the unweighted per-pattern log-likelihoods of the last placement_support: [record][pattern]
+  // The same statistics for EVERY branch at one set of parameters (DESIGN.md section 10, items 9-10):
+  // the parameters of the checkpoint's best record (highest llh, lowest log index on ties) are
+  // installed, root q is placed at a_q = optimize_alpha(root q at ratio 0.5, atol) (0.5 everywhere
+  // with atol = 0) and record q of the statistics is the placement (q, a_q), for every root id q in
+  // order.  One directed sweep scores all 2n - 3 placements and stores their rows.  Unlike
+  // exhaustive mode, the substitution parameters are not re-optimised per branch.  alpha and llh
+  // hold a_q and the log-likelihood at (q, a_q); positions_ms times the alpha searches, capture_ms
+  // the sweep.  Every branch is annotated with BP, pKH, pSH (pAU, ELW in AU mode), LLH and alpha.
+  // Refuses what placement_support refuses, and atol < 0.
+  placement_support_t branch_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed, double atol,
+                                     unsigned replicate_tile = 0, bool keep_rows = false,
+                                     const std::vector<unsigned> &au_scales = {});
+  // the unweighted per-pattern log-likelihoods of the last placement_support / branch_support:
+  // [record][pattern]
   std::vector<double> site_lnl_rows(size_t partition);
 
   rdk_partition_t *partition(size_t i) { return _partitions[i]; }
@@ -219,6 +233,18 @@ private:
   // partition when batched probes are on (rdk_root_loglikelihood_multi); compute_dlh and
   // optimize_alpha are rd::unit_segment_search_t (optim.hpp) over this
   std::vector<double> root_lh_on_branch(const root_location_t &root, const std::vector<double> &ratios);
+
+  // ---- placement support, the parts placement_support and branch_support share ------------------
+  void check_support_request(const std::string &who, size_t replicates, const std::vector<unsigned> &au_scales) const;
+  void check_support_records(const std::string &who, const std::vector<checkpoint_t::record_t> &records) const;
+  void install_record(const checkpoint_t::record_t &record);
+  std::function<void()> support_restore_point(bool keep_rows);
+  void reserve_support_rows(const std::string &who, unsigned rows);
+  void resample_support(const std::string &who, placement_support_t &out, unsigned rows, size_t replicates,
+                        uint64_t seed, unsigned replicate_tile, const std::vector<unsigned> &au_scales);
+  void annotate_support(placement_support_t &out, const std::vector<root_location_t> &where);
+  rooted_tree_t::sweep_schedule_t directed_sweep_schedule(size_t begin, size_t end, const std::vector<double> &ratio,
+                                                          std::vector<unsigned int> &chunk_off) const;
 
   // ---- parameter plumbing ----------------------------------------------------------------------
   void set_subst_rates_random(size_t, const msa_t &);

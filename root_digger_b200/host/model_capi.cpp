@@ -415,21 +415,11 @@ extern "C" int rdh_model_exhaustive_search(void *h, double atol, double pgtol, d
   })
 }
 
-// the body of rdh_model_placement_support and rdh_model_placement_support_au
-static model_t::placement_support_t placement_support_into(
-    void *h, const char *checkpoint_prefix, unsigned long long replicates, unsigned long long seed,
-    unsigned replicate_tile, int keep_rows, unsigned cap, unsigned long long *root_id, double *alpha, double *llh,
-    double *lnl_fixed, unsigned long long *o_lo, long long *o_hi, unsigned *bp_count, unsigned *kh_count,
-    unsigned *sh_count, int *exponent, unsigned *best, double *info, unsigned *n_out,
-    const std::vector<unsigned> &au_scales) {
-  checkpoint_t  external;
-  checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
-  const size_t  records = ckp.read_results().size();
-  if (records > cap) {
-    *n_out = (unsigned)records;
-    throw std::runtime_error("output buffers too small: " + std::to_string(records) + " records");
-  }
-  auto res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0, au_scales);
+// the per-record outputs every support entry fills (capacity cap), and info[0..5]
+static void copy_support(const model_t::placement_support_t &res, unsigned cap, unsigned long long *root_id,
+                         double *alpha, double *llh, double *lnl_fixed, unsigned long long *o_lo, long long *o_hi,
+                         unsigned *bp_count, unsigned *kh_count, unsigned *sh_count, int *exponent, unsigned *best,
+                         double *info, unsigned *n_out) {
   const size_t n = res.root_id.size();
   if (n > cap) throw std::runtime_error("output buffers too small");
   for (size_t i = 0; i < n; ++i) {
@@ -452,6 +442,45 @@ static model_t::placement_support_t placement_support_into(
   info[4] = res.resample_ms;
   info[5] = (double)res.device_bytes;
   *n_out = (unsigned)n;
+}
+
+// the AU-mode outputs (scale_count is [scale][cap]) and info[6..8]
+static void copy_support_au(const model_t::placement_support_t &res, unsigned cap, unsigned *scale_count,
+                            double *p_au, double *au_d, double *au_c, double *au_rss, unsigned *au_used, double *elw,
+                            unsigned long long *elw_fixed, double *info) {
+  const size_t n = res.root_id.size();
+  for (size_t i = 0; i < n; ++i) {
+    for (size_t k = 0; k < res.scales.size(); ++k) scale_count[k * cap + i] = res.scale_count[k * n + i];
+    p_au[i] = res.p_au[i];
+    au_d[i] = res.au_d[i];
+    au_c[i] = res.au_c[i];
+    au_rss[i] = res.au_rss[i];
+    au_used[i] = res.au_used[i];
+    elw[i] = res.elw[i];
+    elw_fixed[i] = res.elw_fixed[i];
+  }
+  info[6] = res.au_counts_ms;
+  info[7] = res.au_accumulate_ms;
+  info[8] = res.au_statistics_ms;
+}
+
+// the body of rdh_model_placement_support and rdh_model_placement_support_au
+static model_t::placement_support_t placement_support_into(
+    void *h, const char *checkpoint_prefix, unsigned long long replicates, unsigned long long seed,
+    unsigned replicate_tile, int keep_rows, unsigned cap, unsigned long long *root_id, double *alpha, double *llh,
+    double *lnl_fixed, unsigned long long *o_lo, long long *o_hi, unsigned *bp_count, unsigned *kh_count,
+    unsigned *sh_count, int *exponent, unsigned *best, double *info, unsigned *n_out,
+    const std::vector<unsigned> &au_scales) {
+  checkpoint_t  external;
+  checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
+  const size_t  records = ckp.read_results().size();
+  if (records > cap) {
+    *n_out = (unsigned)records;
+    throw std::runtime_error("output buffers too small: " + std::to_string(records) + " records");
+  }
+  auto res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0, au_scales);
+  copy_support(res, cap, root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count, exponent, best,
+               info, n_out);
   return res;
 }
 
@@ -501,20 +530,48 @@ extern "C" int rdh_model_placement_support_au(void *h, const char *checkpoint_pr
     const auto res = placement_support_into(h, checkpoint_prefix, replicates, seed, replicate_tile, keep_rows, cap,
                                             root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count,
                                             exponent, best, info, n_out, au);
-    const size_t n = res.root_id.size();
-    for (size_t i = 0; i < n; ++i) {
-      for (size_t k = 0; k < au.size(); ++k) scale_count[k * cap + i] = res.scale_count[k * n + i];
-      p_au[i] = res.p_au[i];
-      au_d[i] = res.au_d[i];
-      au_c[i] = res.au_c[i];
-      au_rss[i] = res.au_rss[i];
-      au_used[i] = res.au_used[i];
-      elw[i] = res.elw[i];
-      elw_fixed[i] = res.elw_fixed[i];
+    copy_support_au(res, cap, scale_count, p_au, au_d, au_c, au_rss, au_used, elw, elw_fixed, info);
+    return 1;
+  })
+}
+
+// The support statistics of EVERY branch at the parameters of the best record of
+// "<checkpoint_prefix>.ckp" (opened read-only; NULL: the model's own result log), with root q at
+// a_q = optimize_alpha(q at 0.5, atol) (atol = 0: 0.5) -- model_t::branch_support, DESIGN.md section 10,
+// items 9-10.  One record per root id, in root-id order (capacity cap >= the model's root count):
+// root id, a_q, the log-likelihood at (q, a_q) and the outputs of rdh_model_placement_support.
+// n_scales = 0: the plain statistics, and scales and the AU outputs may be NULL; otherwise as
+// rdh_model_placement_support_au.  info receives the nine values of rdh_model_placement_support_au
+// (zeros for the AU timings in plain mode), then the alpha searches' ms.
+extern "C" int rdh_model_branch_support(void *h, const char *checkpoint_prefix, unsigned long long replicates,
+                                        unsigned long long seed, double atol, unsigned replicate_tile, int keep_rows,
+                                        unsigned n_scales, const unsigned *scales, unsigned cap,
+                                        unsigned long long *root_id, double *alpha, double *llh, double *lnl_fixed,
+                                        unsigned long long *o_lo, long long *o_hi, unsigned *bp_count,
+                                        unsigned *kh_count, unsigned *sh_count, unsigned *scale_count, double *p_au,
+                                        double *au_d, double *au_c, double *au_rss, unsigned *au_used, double *elw,
+                                        unsigned long long *elw_fixed, int *exponent, unsigned *best, double *info,
+                                        unsigned *n_out) {
+  RDH_TRY({
+    std::vector<unsigned> au;
+    if (n_scales) {
+      if (!scales) throw std::invalid_argument("AU scales: none given");
+      au.assign(scales, scales + n_scales);
+      rd::check_au_scales(au.data(), au.size());
     }
-    info[6] = res.au_counts_ms;
-    info[7] = res.au_accumulate_ms;
-    info[8] = res.au_statistics_ms;
+    const size_t roots = H(h).model->tree().root_count();
+    if (roots > cap) {
+      *n_out = (unsigned)roots;
+      throw std::runtime_error("output buffers too small: " + std::to_string(roots) + " branches");
+    }
+    checkpoint_t  external;
+    checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
+    const auto    res = H(h).model->branch_support(ckp, replicates, seed, atol, replicate_tile, keep_rows != 0, au);
+    copy_support(res, cap, root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count, exponent, best,
+                 info, n_out);
+    info[6] = info[7] = info[8] = 0.0;
+    if (n_scales) copy_support_au(res, cap, scale_count, p_au, au_d, au_c, au_rss, au_used, elw, elw_fixed, info);
+    info[9] = res.positions_ms;
     return 1;
   })
 }

@@ -783,11 +783,14 @@ unsigned int rooted_tree_t::sweep_depth_bound() const {
 rooted_tree_t::sweep_schedule_t rooted_tree_t::generate_sweep_operations(size_t begin, size_t end,
                                                                          unsigned int clv0, int scaler0,
                                                                          unsigned int pm0,
-                                                                         unsigned int extra) const {
+                                                                         unsigned int extra,
+                                                                         const std::vector<double> &ratio) const {
   if (!rooted() || _current_rl.edge == nullptr)
     throw std::runtime_error("generate_sweep_operations: the tree has no current root "
                              "(call generate_operations / root_by first)");
   if (begin > end || end > _roots.size()) throw std::invalid_argument("generate_sweep_operations: bad root range");
+  if (!ratio.empty() && ratio.size() != _roots.size())
+    throw std::invalid_argument("generate_sweep_operations: one ratio per root location is needed");
   sweep_schedule_t out;
   if (begin == end) return out;
   {
@@ -849,8 +852,9 @@ rooted_tree_t::sweep_schedule_t rooted_tree_t::generate_sweep_operations(size_t 
   // close a placement: the two root half-branches and the root operation; child1 is the
   // end point root_by would make the left child (src/tree.cpp:273-320)
   auto emit_placement = [&](const unode_t *c, ref_t below, ref_t above) {
-    const size_t           i = pos_of[c->uid];
-    const root_location_t &rl = _roots[i];
+    const size_t    i = pos_of[c->uid];
+    root_location_t rl = _roots[i];
+    if (!ratio.empty()) rl.brlen_ratio = ratio[i];
     out.mi.push_back(ML);
     out.bl.push_back(rl.brlen());
     out.mi.push_back(MR);

@@ -124,6 +124,9 @@ public:
   root_location_t root_location(size_t index) const;
   root_location_t root_location(const std::string &label) const;
   root_location_t root_location() const { return _current_rl; }
+  // whether root_by(rl) roots the tree: on an unrooted tree whose start node is rl's edge it only
+  // rewrites the lengths next to that node (update_root, src/tree.cpp:273-320)
+  bool can_root_by(const root_location_t &rl) const { return rooted() || rl.edge != _tree->vroot; }
 
   root_location_t              midpoint() const;
   std::vector<root_location_t> rank_midpoints() const;
@@ -166,7 +169,11 @@ public:
   // stays rooted where it was and its CLVs, scalers and P-matrices keep their
   // values.  The output has the shape rdk_sweep_root_placements takes; the last
   // operation of each placement is the root operation.  placement q scores the
-  // root at position root_pos[q] of roots().
+  // root at position root_pos[q] of roots(), at the ratio that root location holds
+  // (0.5) or, when `ratio` is not empty, at ratio[root_pos[q]] (one entry per root
+  // of roots()): the two root half-branches are then those generate_derivative_operations
+  // gives for that root location at that ratio, child 1 (the location's edge) taking
+  // ratio * length.
   struct sweep_schedule_t {
     std::vector<unsigned int>    pm_off{0}, op_off{0}, mi;
     std::vector<double>          bl;
@@ -176,7 +183,8 @@ public:
   // spare CLV / scale buffers generate_sweep_operations can need for ANY current root
   unsigned int     sweep_depth_bound() const;
   sweep_schedule_t generate_sweep_operations(size_t begin, size_t end, unsigned int clv0, int scaler0,
-                                             unsigned int pm0, unsigned int extra) const;
+                                             unsigned int pm0, unsigned int extra,
+                                             const std::vector<double> &ratio = {}) const;
 
   void root_by(unsigned int root_id) { root_by(_roots[root_id]); }
   void root_by(const root_location_t &);

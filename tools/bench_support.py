@@ -13,8 +13,15 @@ With --au-scales (e.g. 0.5,0.6,...,1.4, or "default" for capi.AU_SCALES) every c
 AU test's multiscale bootstrap and the expected likelihood weights, and the line adds their phases:
 multiscale counts, multiscale accumulation, and statistics + ELW.
 
+With --branches it times branch support instead (Model.branch_support, DESIGN.md section 10, items
+9-10): the checkpoint holds ONE record, as after a search-mode run, and every call scores all 2n-3
+branches at that record's parameters.  Per B the line gives the median of positions_ms (the 2n-3
+position searches), capture_ms (the one placement sweep that stores the rows) and the resampling
+phases, and, next to them, the capture_ms of placement_support on the equivalent 2n-3-record
+checkpoint (the record-by-record capture this mode replaces), measured once at the first B.
+
     python tools/bench_support.py [--taxa 500] [--sites 100000] [--replicates 1000,10000] [--reps 3]
-                                  [--au-scales default]
+                                  [--au-scales default] [--branches] [--atol 1e-14]
 """
 from __future__ import annotations
 
@@ -55,6 +62,8 @@ def main():
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--seed", type=int, default=0x5EED0002)
     ap.add_argument("--au-scales", default=None, help='comma-separated scales, or "default" (capi.AU_SCALES)')
+    ap.add_argument("--branches", action="store_true", help="time branch_support from a one-record checkpoint")
+    ap.add_argument("--atol", type=float, default=1e-14, help="--branches: tolerance of the position searches")
     args = ap.parse_args()
 
     from root_digger_b200 import capi, synth
@@ -70,6 +79,8 @@ def main():
     R, P = m.root_count, m.sites(0)
     r12, f4, _ = m.get_params()
     rng = np.random.default_rng(args.seed + 3)
+    if args.branches:
+        return branches(args, m, au, device, r12, f4, rng)
     with tempfile.TemporaryDirectory() as tmp:
         prefix = str(Path(tmp) / "support")
         ckp = capi.Checkpoint(prefix)
@@ -98,6 +109,47 @@ def main():
             results[str(B)] = med
     line = {"tool": "bench_support", "taxa": args.taxa, "patterns": P, "records": R, "cats": args.cats,
             "reps": args.reps, "card": device, "results": results}
+    if au:
+        line["au_scales"] = list(au)
+    print(json.dumps(line))
+
+
+def branches(args, m, au, device, r12, f4, rng):
+    from root_digger_b200 import capi
+    R, P = m.root_count, m.sites(0)
+    params = [{"rates": r12, "freqs": f4, "alpha": float(rng.uniform(0.5, 2.0)),
+               "weights": np.full(args.cats, 1.0 / args.cats)}]
+    results = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        one = str(Path(tmp) / "search")
+        ckp = capi.Checkpoint(one)
+        ckp.save_options(prefix=one)
+        ckp.write(R // 2, 0.0, 0.5, params, K=args.cats)
+        ckp.close()
+        Bs = [int(b) for b in args.replicates.split(",")]
+        kw = dict(atol=args.atol, au_scales=au)
+        first = m.branch_support(one, replicates=Bs[0], seed=1, **kw)  # warm-up: module load, allocations
+        # the record-by-record capture of the same 2n-3 placements, for comparison
+        eq = str(Path(tmp) / "equivalent")
+        ckp = capi.Checkpoint(eq)
+        ckp.save_options(prefix=eq)
+        for q in range(R):
+            ckp.write(q, 0.0, float(first["alpha"][q]), params, K=args.cats)
+        ckp.close()
+        checkpoint_capture_ms = m.placement_support(eq, replicates=Bs[0], seed=1, au_scales=au)["capture_ms"]
+        for B in Bs:
+            runs = [m.branch_support(one, replicates=B, seed=1 + i, **kw) for i in range(args.reps)]
+            keys = ["positions_ms", "capture_ms", "counts_ms", "accumulate_ms", "statistics_ms", "resample_ms"]
+            if au:
+                keys += ["au_counts_ms", "au_accumulate_ms", "au_statistics_ms"]
+            med = {k: statistics.median(r[k] for r in runs) for k in keys}
+            med["device_bytes"] = max(r["device_bytes"] for r in runs)
+            med["bp_sum"] = int(runs[0]["bp_count"].sum())
+            med["same_positions"] = all(np.array_equal(r["alpha"], first["alpha"]) for r in runs)
+            results[str(B)] = med
+    line = {"tool": "bench_support", "mode": "branches", "taxa": args.taxa, "patterns": P, "records": R,
+            "cats": args.cats, "reps": args.reps, "atol": args.atol, "card": device,
+            "checkpoint_capture_ms": checkpoint_capture_ms, "row_bytes": 8 * P * R, "results": results}
     if au:
         line["au_scales"] = list(au)
     print(json.dumps(line))
