@@ -236,6 +236,9 @@ int rdk_sweep_root_placements(rdk_partition_t *partition,
  * shard the rows hold the local patterns.  out_lnl is unchanged, bit for bit.  Combines with the
  * other flags and with rdk_sweep_root_placements_chunks. */
 #define RDK_SWEEP_ROWS 4u
+/* If a sweep fails, none of its evaluations stays recorded: no later call runs one.  The engine
+ * may already have run the batches before the failing one, so the buffers the call's operations
+ * write have undefined content afterwards. */
 int rdk_sweep_root_placements_ex(rdk_partition_t *partition,
                                  unsigned int placements,
                                  const unsigned int *params_indices,

@@ -152,9 +152,12 @@ struct Engine {
   std::vector<unsigned> pm_free;     // free physical slots
   std::vector<unsigned> pm_retired;  // freed at the next flush
 
-  // recorded work
+  // recorded work.  What a program must produce is not kept here: the call that records evaluations
+  // hands it to flush (ProgramOutputs), and no rdk_* entry returns with an rEval operation recorded.
   std::vector<PmatEntry> pend_pm;
   std::vector<ROp>       pend_prog;
+  unsigned long long     pend_bytes = 0;  // algorithmic bytes of pend_prog
+  unsigned               pend_ops = 0, pend_evals = 0;
   // Lazily materialised evaluation.  A full evaluation whose only requested result is the root
   // log-likelihood (the closure BFGS calls 13 times per step, reference src/model.cpp:455-476,
   // 1488-1502) stores only the CLVs it reads back itself; the others exist in registers only.  The
@@ -170,14 +173,6 @@ struct Engine {
   } lazy;
   bool     lazy_enabled = true;
   unsigned full_streak = 0;  // consecutive flushed programs that were lazy-eligible full traversals
-  bool pend_lazy_ok = false;  // the pending program may be evaluated lazily
-  // buffers whose content after pend_prog is not required (scratch of a directed sweep), per index
-  const std::vector<char> *pend_scratch_clv = nullptr, *pend_scratch_sc = nullptr;
-  unsigned               pend_slots = 0;  // eval slots used by pend_prog
-  unsigned long long     pend_bytes = 0;  // algorithmic bytes of pend_prog
-  unsigned               pend_ops = 0, pend_evals = 0;
-  std::vector<unsigned>  pend_chunk_off;  // > 2 entries: pend_prog is that many - 1 independent chunks
-  bool                   want_persite = false;
 
   Ring    ring;
   double *d_partials = nullptr;
@@ -187,8 +182,6 @@ struct Engine {
   double *d_persite = nullptr;
   double *d_rows = nullptr;    // [rows_cap][S]: unweighted per-pattern values (rdk_partition_set_site_lnl_rows)
   unsigned rows_cap = 0;
-  double  *want_row = nullptr; // the row the next evaluation stores into, or null
-  double  *want_rows = nullptr; // RDK_SWEEP_ROWS: eval slot s of the next program stores into want_rows + s * S
   double *h_results = nullptr;  // pinned, device-visible
   size_t  results_cap = 0;      // doubles
 
@@ -201,13 +194,14 @@ struct Engine {
   // Lowered programs kept for the next traversal of the same structure (a BFGS closure re-records
   // the same operations with new P-matrices 13 times per step, a search step alternates one full
   // traversal and one sweep): key = the recorded operations without their P slots + everything
-  // else the lowering looks at, compared exactly; value = the instructions, whose P slots are
-  // refreshed from the operations recorded now.
+  // else the lowering looks at (the chunks, scratch sets and lazy decision of the program's
+  // ProgramOutputs), compared exactly; value = the instructions, whose P slots are refreshed from
+  // the operations recorded now.
   struct KeptProgram {
     std::vector<ROp>      ops;
     std::vector<unsigned> chunk_off;
     std::vector<char>     scratch_clv, scratch_sc;
-    bool                  has_scratch_clv = false, has_scratch_sc = false, lazy = false;
+    bool                  lazy = false;
     // the lowering
     bool                  grouped = false;
     std::vector<LInstr>   lowered, lowered_join;
@@ -637,6 +631,20 @@ bool pending_needs_materialization(const Engine *e) {
   return false;
 }
 
+// What a flushed program must produce besides the buffers its operations write.  It belongs to the
+// one call that records evaluations and runs them (run_evals); every other flush passes none, and
+// no operation recorded then carries rEval.
+struct ProgramOutputs {
+  unsigned slots = 0;           // eval slots: one partial sum per slot and warp iteration
+  double  *persite = nullptr;   // per-pattern values of eval slot 0, or of every slot (row_stride)
+  bool     unweighted = false;  // persite receives the values before the pattern weight
+  size_t   row_stride = 0;      // != 0: eval slot s stores at persite + s * row_stride (the ROWS kernel)
+  std::vector<unsigned> chunk_off;  // empty, or the n + 1 offsets of n >= 2 independent chunks
+  // per index: the buffer's content after the program is not required (a sweep's scratch); empty: none
+  std::vector<char> scratch_clv, scratch_sc;
+  bool              lazy_ok = false;  // the program may be evaluated lazily (Engine::Lazy)
+};
+
 constexpr size_t kKeptPrograms = 8;    // entries (least recently used replaced)
 constexpr size_t kKeptMinOps = 32;     // shorter programs are lowered every time
 
@@ -646,13 +654,11 @@ bool same_structure(const ROp &a, const ROp &b) {
          a.c2scale == b.c2scale && a.flags == b.flags && a.slot == b.slot;
 }
 
-Engine::KeptProgram *find_kept_program(Engine *e, bool lazy, bool chunked) {
+Engine::KeptProgram *find_kept_program(Engine *e, const ProgramOutputs &out, bool lazy) {
   for (Engine::KeptProgram &k : e->kept_programs) {
-    if (k.lazy != lazy || k.ops.size() != e->pend_prog.size()) continue;
-    if (chunked ? k.chunk_off != e->pend_chunk_off : !k.chunk_off.empty()) continue;
-    if (k.has_scratch_clv != (e->pend_scratch_clv != nullptr) || k.has_scratch_sc != (e->pend_scratch_sc != nullptr)) continue;
-    if (k.has_scratch_clv && k.scratch_clv != *e->pend_scratch_clv) continue;
-    if (k.has_scratch_sc && k.scratch_sc != *e->pend_scratch_sc) continue;
+    if (k.lazy != lazy || k.ops.size() != e->pend_prog.size() || k.chunk_off != out.chunk_off ||
+        k.scratch_clv != out.scratch_clv || k.scratch_sc != out.scratch_sc)
+      continue;
     bool same = true;
     for (size_t i = 0; same && i < k.ops.size(); ++i) same = same_structure(k.ops[i], e->pend_prog[i]);
     if (same) return &k;
@@ -726,8 +732,14 @@ bool choose_subtree_groups(const Engine *e, unsigned n_witer, std::vector<ROp> &
   return true;
 }
 
-// launch recorded P-matrix work and the recorded program (no host sync)
-int flush(rdk_partition_t *p) {
+void clear_pending_ops(Engine *e) {
+  e->pend_prog.clear();
+  e->pend_ops = e->pend_evals = 0;
+  e->pend_bytes = 0;
+}
+
+// launch recorded P-matrix work and the recorded program, which produces `out` (no host sync)
+int flush(rdk_partition_t *p, const ProgramOutputs &out = {}) {
   Engine *e = eng(p);
   if (!launch_pmatrices(p)) return RDK_FAILURE;
   if (e->pend_prog.empty()) {
@@ -753,60 +765,52 @@ int flush(rdk_partition_t *p) {
   a.partial_stride = n_witer ? n_witer : 1;
   for (int i = 0; i < 4; ++i) a.pi[i] = p->frequencies[0][i];
   for (unsigned k = 0; k < e->K; ++k) a.w[k] = k < e->Kreal ? p->rate_weights[k] : 0.0;
-  if (e->pend_slots) {
-    if (!ensure_partials(e, e->pend_slots, a.partial_stride)) return RDK_FAILURE;
+  if (out.slots) {
+    if (!ensure_partials(e, out.slots, a.partial_stride)) return RDK_FAILURE;
     a.partials = e->d_partials;
   }
-  // a row of unweighted values takes the place of the weighted per-site output (never both)
-  a.persite = e->want_row ? e->want_row : (e->want_persite ? e->d_persite : nullptr);
-  a.persite_unweighted = e->want_row != nullptr;
-  if (e->want_rows) {  // a sweep batch capturing rows: the ROWS variant of the kernel, one row per eval slot
-    a.persite = e->want_rows;
-    a.persite_unweighted = 1;
-    a.row_stride = e->S;
-  }
+  a.persite = out.persite;
+  a.persite_unweighted = out.unweighted;
+  a.row_stride = out.row_stride;
   // recorded operations -> the instructions the kernel walks (rdk_lower.hpp)
   HostTimer             lower_timer(&e->stats.host_lower_ns);  // lowering, pointer translation, enqueue
-  const bool            chunked = e->pend_chunk_off.size() > 2;
+  const bool            chunked = !out.chunk_off.empty();
+  const bool            scratch = !out.scratch_clv.empty() || !out.scratch_sc.empty();
   // Lazy only in a STREAK of such traversals (the second consecutive one onwards): that is the
   // signature of a BFGS closure -- 13 evaluations per step, reference src/model.cpp:1488-1502 --
   // whereas the single compute_lh before a sweep or a root move would only have to be replayed
   // (measured on B200, cfg2 search step: 9.06 ms with an always-lazy compute_lh against 8.03 ms).
-  e->full_streak = e->pend_lazy_ok ? e->full_streak + 1 : 0;
-  const bool lazy = e->pend_lazy_ok && e->full_streak >= 2 && e->lazy_enabled && !chunked && !e->pend_scratch_clv;
+  e->full_streak = out.lazy_ok ? e->full_streak + 1 : 0;
+  const bool lazy = out.lazy_ok && e->full_streak >= 2 && e->lazy_enabled && !chunked && !scratch;
   for (size_t i = 0; i < e->pend_prog.size(); ++i) e->pend_prog[i].id = (unsigned)i;
   Engine::KeptProgram  scratch_entry;  // programs that are not kept are lowered into this one
   Engine::KeptProgram *kp = nullptr;
   const bool           keepable = e->pend_prog.size() >= kKeptMinOps;
-  if (keepable) kp = find_kept_program(e, lazy, chunked);
+  if (keepable) kp = find_kept_program(e, out, lazy);
   if (kp) {
     e->stats.programs_reused++;
   } else {
     kp = keepable ? new_kept_program(e) : &scratch_entry;
     LowerOptions lopt;
     lopt.tips = e->tips;
-    lopt.scratch_clv = e->pend_scratch_clv;
-    lopt.scratch_scaler = e->pend_scratch_sc;
+    lopt.scratch_clv = &out.scratch_clv;
+    lopt.scratch_scaler = &out.scratch_sc;
     lopt.discard_writes = lazy;  // keep only the stores the program reads back itself
     // a long traversal on a small shard: disjoint subtrees side by side, then what joins them
     std::vector<ROp>      group_ops, join_ops;
     std::vector<unsigned> group_off;
     kp->lowered_join.clear();
-    kp->grouped = !chunked && !e->pend_scratch_clv && !e->pend_scratch_sc && nelem != 0 &&
-                  choose_subtree_groups(e, n_witer, group_ops, group_off, join_ops);
+    kp->grouped = !chunked && !scratch && nelem != 0 && choose_subtree_groups(e, n_witer, group_ops, group_off, join_ops);
     if (kp->grouped)
       lower_grouped(group_ops, group_off, join_ops, lopt, kp->lowered, kp->lchunk, kp->lowered_join, &kp->lst);
     else
-      lower_program(e->pend_prog, chunked ? e->pend_chunk_off : std::vector<unsigned>(), lopt, kp->lowered, kp->lchunk,
-                    &kp->lst);
+      lower_program(e->pend_prog, out.chunk_off, lopt, kp->lowered, kp->lchunk, &kp->lst);
     if (keepable) {
       kp->ops = e->pend_prog;
-      kp->chunk_off = chunked ? e->pend_chunk_off : std::vector<unsigned>();
+      kp->chunk_off = out.chunk_off;
+      kp->scratch_clv = out.scratch_clv;
+      kp->scratch_sc = out.scratch_sc;
       kp->lazy = lazy;
-      kp->has_scratch_clv = e->pend_scratch_clv != nullptr;
-      kp->has_scratch_sc = e->pend_scratch_sc != nullptr;
-      if (kp->has_scratch_clv) kp->scratch_clv = *e->pend_scratch_clv; else kp->scratch_clv.clear();
-      if (kp->has_scratch_sc) kp->scratch_sc = *e->pend_scratch_sc; else kp->scratch_sc.clear();
     }
   }
   kp->last_use = ++e->kept_clock;
@@ -868,11 +872,7 @@ int flush(rdk_partition_t *p) {
   e->stats.clv_ops += e->pend_ops;
   e->stats.root_evals += e->pend_evals;
   e->stats.algorithmic_bytes += e->pend_bytes;
-  e->pend_prog.clear();
-  e->pend_chunk_off.clear();
-  e->pend_lazy_ok = false;
-  e->pend_ops = e->pend_evals = 0;
-  e->pend_bytes = 0;
+  clear_pending_ops(e);
   for (unsigned s : e->pm_retired) e->pm_free.push_back(s);
   e->pm_retired.clear();
   return RDK_SUCCESS;
@@ -943,6 +943,20 @@ int finish_evals(rdk_partition_t *p, unsigned slots) {
   return RDK_SUCCESS;
 }
 
+// Run the recorded program with the evaluations `out` asks for and copy their values to
+// results[0..out.slots).  If that fails, the recorded operations are dropped: a later flush would
+// run their evaluations without outputs.  The recorded P-matrix updates stay, because the indices
+// already name their new slots (as after eager execution).
+int run_evals(rdk_partition_t *p, const ProgramOutputs &out, double *results) {
+  Engine *e = eng(p);
+  if (!flush(p, out) || !finish_evals(p, out.slots)) {
+    clear_pending_ops(e);
+    return RDK_FAILURE;
+  }
+  for (unsigned i = 0; i < out.slots; ++i) results[i] = e->h_results[i];
+  return RDK_SUCCESS;
+}
+
 // translate a corax-shaped operation into a recorded operation (buffers allocated, P-matrix
 // indices resolved to the physical pool slots they name NOW)
 int make_rop(rdk_partition_t *p, const rdk_operation_t &op, unsigned flags, ROp *out) {
@@ -994,6 +1008,51 @@ unsigned long long op_bytes(const Engine *e, const ROp &r) {
   if ((r.flags & rWrite) && r.pscale >= 0) b += 4 * S;
   if (r.flags & rEval) b += 4 * S;  // pattern weights
   return b;
+}
+
+// record CLV operations in order; when one is refused, those before it stay recorded
+int record_ops(rdk_partition_t *p, const rdk_operation_t *ops, unsigned count) {
+  Engine *e = eng(p);
+  for (unsigned i = 0; i < count; ++i) {
+    ROp r;
+    if (!make_rop(p, ops[i], rWrite, &r)) return RDK_FAILURE;
+    e->pend_bytes += op_bytes(e, r);
+    e->pend_prog.push_back(r);
+    e->pend_ops++;
+  }
+  return RDK_SUCCESS;
+}
+
+// Record the evaluation of root CLV `clv` (scale buffer rs, -1: none) into eval slot `slot`: fused
+// into the last recorded operation if that one writes this CLV (keep_root: it is then only
+// evaluated in registers and stores nothing), else as an operation that loads the CLV.  Returns
+// whether the evaluation was fused.
+bool record_root_eval(Engine *e, unsigned clv, int rs, unsigned slot, bool keep_root) {
+  e->pend_evals++;
+  if (!e->pend_prog.empty()) {
+    ROp &last = e->pend_prog.back();
+    if ((last.flags & rWrite) && !(last.flags & rEval) && last.parent == clv && last.pscale == rs) {
+      e->pend_bytes -= op_bytes(e, last);
+      last.flags |= rEval;
+      if (keep_root) last.flags &= ~rWrite;
+      last.slot = slot;
+      e->pend_bytes += op_bytes(e, last);
+      return true;
+    }
+  }
+  ROp r;
+  memset(&r, 0, sizeof(r));
+  r.flags = rLoadOnly | rEval;
+  r.parent = kNoClv;
+  r.pscale = -1;
+  r.c1 = clv;
+  r.c1scale = rs;
+  r.c2 = kNoClv;
+  r.c2scale = -1;
+  r.slot = slot;
+  e->pend_bytes += 32ull * e->Kreal * e->S + (rs >= 0 ? 4ull * e->S : 0) + 4ull * e->S;
+  e->pend_prog.push_back(r);
+  return false;
 }
 
 // record a P-matrix update with slot renaming; caller holds the mutex
@@ -1335,13 +1394,7 @@ extern "C" void rdk_update_clvs(rdk_partition_t *p, const rdk_operation_t *ops, 
   std::lock_guard<std::mutex> lk(e->mu);
   cudaSetDevice(e->device);
   HostTimer record_timer(&e->stats.host_record_ns);
-  for (unsigned i = 0; i < count; ++i) {
-    ROp r;
-    if (!make_rop(p, ops[i], rWrite, &r)) return;  // error left in rdk_errno
-    e->pend_bytes += op_bytes(e, r);
-    e->pend_prog.push_back(r);
-    e->pend_ops++;
-  }
+  record_ops(p, ops, count);  // error left in rdk_errno
 }
 
 // rdk_compute_root_loglikelihood; `row` (device, [S]) optionally receives the unweighted values
@@ -1362,48 +1415,25 @@ static double root_loglikelihood(rdk_partition_t *p, unsigned int clv_index, int
   if (!ensure_clv(e, clv_index - e->tips)) return nan;
   const int rs = scaler_index == RDK_SCALE_BUFFER_NONE ? -1 : scaler_index;
   if (!ensure_scaler(e, rs)) return nan;
-  // fuse with the recorded operation that produces this CLV, if it is the last one
-  bool fused = false;
-  if (!e->pend_prog.empty()) {
-    ROp &last = e->pend_prog.back();
-    if ((last.flags & rWrite) && !(last.flags & rEval) && last.parent == clv_index && last.pscale == rs) {
-      last.flags |= rEval;
-      last.slot = 0;
-      e->pend_bytes += 4ull * e->S;
-      fused = true;
-    }
-  }
-  if (!fused) {
-    ROp r;
-    memset(&r, 0, sizeof(r));
-    r.flags = rLoadOnly | rEval;
-    r.parent = kNoClv;
-    r.pscale = -1;
-    r.c1 = clv_index;
-    r.c1scale = rs;
-    r.c2 = kNoClv;
-    r.c2scale = -1;
-    r.slot = 0;
-    e->pend_bytes += 32ull * e->Kreal * e->S + (rs >= 0 ? 4ull * e->S : 0) + 4ull * e->S;
-    e->pend_prog.push_back(r);
-  }
-  e->pend_evals++;
-  e->pend_slots = 1;
-  e->want_persite = persite_lnl != nullptr;
-  e->want_row = row;
+  const bool fused = record_root_eval(e, clv_index, rs, 0, false);
+  ProgramOutputs out;
+  out.slots = 1;
+  // a row of unweighted values takes the place of the weighted per-site output (never both)
+  out.persite = row ? row : (persite_lnl ? e->d_persite : nullptr);
+  out.unweighted = row != nullptr;
   // a traversal whose only requested result is this log-likelihood may keep its CLVs in registers
-  if (fused && !persite_lnl && !row) {
+  if (fused && !out.persite) {
     size_t writes = 0;
     for (const ROp &r : e->pend_prog) writes += (r.flags & rWrite) ? 1 : 0;
-    e->pend_lazy_ok = writes >= 16;
+    out.lazy_ok = writes >= 16;
   }
-  int ok = flush(p);
-  e->pend_slots = 0;
-  e->want_persite = false;
-  e->want_row = nullptr;
-  if (!ok) return nan;
-  if (e->S == 0 && e->global_sites == 0) return 0.0;
-  if (!finish_evals(p, 1)) return nan;
+  if (e->S == 0 && e->global_sites == 0) {  // no sites at all: nothing to reduce
+    if (flush(p, out)) return 0.0;
+    clear_pending_ops(e);
+    return nan;
+  }
+  double lnl;
+  if (!run_evals(p, out, &lnl)) return nan;
   if (persite_lnl) {
     if (cudaMemcpy(persite_lnl, e->d_persite, sizeof(double) * e->S, cudaMemcpyDeviceToHost) !=
         cudaSuccess) {
@@ -1412,7 +1442,7 @@ static double root_loglikelihood(rdk_partition_t *p, unsigned int clv_index, int
     }
     e->stats.d2h_bytes += sizeof(double) * e->S;
   }
-  return e->h_results[0];
+  return lnl;
 }
 
 extern "C" double rdk_compute_root_loglikelihood(rdk_partition_t *p, unsigned int clv_index,
@@ -1603,14 +1633,11 @@ extern "C" int rdk_root_loglikelihood_multi(rdk_partition_t *p, const rdk_operat
     e->pend_prog.push_back(r);
     e->pend_evals++;
   }
-  e->pend_slots = count;
-  int ok = flush(p);
-  e->pend_slots = 0;
+  ProgramOutputs out;
+  out.slots = count;
+  const int ok = run_evals(p, out, out_lnl);
   for (unsigned s : used) e->pm_free.push_back(s);
-  if (!ok) return RDK_FAILURE;
-  if (!finish_evals(p, count)) return RDK_FAILURE;
-  for (unsigned b = 0; b < count; ++b) out_lnl[b] = e->h_results[b];
-  return RDK_SUCCESS;
+  return ok;
 }
 
 extern "C" int rdk_sweep_root_placements(rdk_partition_t *p, unsigned int placements,
@@ -1715,11 +1742,6 @@ extern "C" int rdk_sweep_root_placements_chunks(rdk_partition_t *p, unsigned int
     const int v = atoi(env);
     if (v >= 1) max_slots = std::min(max_slots, (unsigned)v);
   }
-  // whatever way this call ends, the chunk table does not outlive it
-  struct chunk_table_guard {
-    Engine *e;
-    ~chunk_table_guard() { e->pend_chunk_off.clear(); }
-  } chunk_guard{e};
   // the chunks run side by side only when nothing they share is written (the root CLV is:
   // RDK_SWEEP_KEEP_ROOT must be set) and the whole sweep is one launch; otherwise they run
   // in order, which the contract always allows
@@ -1782,78 +1804,44 @@ extern "C" int rdk_sweep_root_placements_chunks(rdk_partition_t *p, unsigned int
       }
     }
   }
-  struct scratch_guard {
-    Engine *e;
-    ~scratch_guard() { e->pend_scratch_clv = e->pend_scratch_sc = nullptr; }
-  } sguard{e};
-  unsigned       done = 0;
-  for (size_t batch = 0; batch < n_batches; ++batch) {
-    unsigned b = 0;
-    size_t   pm_budget = e->pm_free.size();
-    unsigned next_chunk = 0;
-    if (concurrent) e->pend_chunk_off.clear();
-    auto record_t0 = std::chrono::steady_clock::now();
-    while (done + b < cuts[batch + 1]) {
-      unsigned q = done + b;
-      size_t   need = pm_offsets[q + 1] - pm_offsets[q];
+  // ---- batch k: one program whose eval slot s is placement cuts[k] + s ------------------------
+  auto record_batch = [&](size_t k, ProgramOutputs &out) -> int {
+    HostTimer record_timer(&e->stats.host_record_ns);
+    size_t    pm_budget = e->pm_free.size();
+    unsigned  next_chunk = 0;
+    for (unsigned q = cuts[k]; q < cuts[k + 1]; ++q) {
+      const size_t need = pm_offsets[q + 1] - pm_offsets[q];
       if (need > pm_budget) return fail(RDK_ERROR_MEM, "P-matrix pool smaller than planned");
+      pm_budget -= need;
       if (concurrent && next_chunk < n_chunks && q == chunk_offsets[next_chunk]) {
-        e->pend_chunk_off.push_back((unsigned)e->pend_prog.size());
+        out.chunk_off.push_back((unsigned)e->pend_prog.size());
         ++next_chunk;
       }
-      pm_budget -= need;
       for (unsigned i = pm_offsets[q]; i < pm_offsets[q + 1]; ++i)
         if (!record_pmatrix(p, matrix_indices[i], branch_lengths[i])) return RDK_FAILURE;
-      bool fused = false;
-      for (unsigned i = op_offsets[q]; i < op_offsets[q + 1]; ++i) {
-        ROp r;
-        if (!make_rop(p, operations[i], rWrite, &r)) return RDK_FAILURE;
-        if (i + 1 == op_offsets[q + 1] && r.parent == root_clv_index && r.pscale == rs) {
-          r.flags |= rEval;
-          r.slot = b;
-          fused = true;
-          if (flags & RDK_SWEEP_KEEP_ROOT) r.flags &= ~rWrite;  // evaluate in registers, store nothing
-        }
-        e->pend_bytes += op_bytes(e, r);
-        e->pend_prog.push_back(r);
-        e->pend_ops++;
-      }
-      if (!fused) {
-        ROp r;
-        memset(&r, 0, sizeof(r));
-        r.flags = rLoadOnly | rEval;
-        r.parent = kNoClv;
-        r.pscale = -1;
-        r.c1 = root_clv_index;
-        r.c1scale = rs;
-        r.c2 = kNoClv;
-        r.c2scale = -1;
-        r.slot = b;
-        e->pend_bytes += 32ull * e->Kreal * e->S + (rs >= 0 ? 4ull * e->S : 0) + 4ull * e->S;
-        e->pend_prog.push_back(r);
-      }
-      e->pend_evals++;
-      ++b;
+      if (!record_ops(p, operations + op_offsets[q], op_offsets[q + 1] - op_offsets[q])) return RDK_FAILURE;
+      record_root_eval(e, root_clv_index, rs, q - cuts[k], flags & RDK_SWEEP_KEEP_ROOT);
     }
-    if (b == 0) return fail(RDK_ERROR_PARAM, "a placement needs more P-matrices than the pool holds");
-    e->stats.host_record_ns += (unsigned long long)std::chrono::duration_cast<std::chrono::nanoseconds>(
-                                   std::chrono::steady_clock::now() - record_t0).count();
-    if (concurrent) e->pend_chunk_off.push_back((unsigned)e->pend_prog.size());
-    e->pend_slots = b;
+    if (concurrent) out.chunk_off.push_back((unsigned)e->pend_prog.size());
+    out.slots = cuts[k + 1] - cuts[k];
     if (flags & RDK_SWEEP_DISCARD) {
-      e->pend_scratch_clv = &scratch_clv[batch];
-      e->pend_scratch_sc = &scratch_sc[batch];
+      out.scratch_clv = std::move(scratch_clv[k]);
+      out.scratch_sc = std::move(scratch_sc[k]);
     }
-    // RDK_SWEEP_ROWS: eval slot s of this batch is placement done + s, and stores into that row
-    if (flags & RDK_SWEEP_ROWS) e->want_rows = e->d_rows + (size_t)done * e->S;
-    int ok = flush(p);
-    e->want_rows = nullptr;
-    e->pend_scratch_clv = e->pend_scratch_sc = nullptr;
-    e->pend_slots = 0;
-    if (!ok) return RDK_FAILURE;
-    if (!finish_evals(p, b)) return RDK_FAILURE;
-    for (unsigned i = 0; i < b; ++i) out_lnl[done + i] = e->h_results[i];
-    done += b;
+    if (flags & RDK_SWEEP_ROWS) {  // eval slot s stores into the row of its placement
+      out.persite = e->d_rows + (size_t)cuts[k] * e->S;
+      out.unweighted = true;
+      out.row_stride = e->S;
+    }
+    return RDK_SUCCESS;
+  };
+  for (size_t k = 0; k < n_batches; ++k) {
+    ProgramOutputs out;
+    if (!record_batch(k, out)) {
+      clear_pending_ops(e);  // no evaluation outlives the call
+      return RDK_FAILURE;
+    }
+    if (!run_evals(p, out, out_lnl + cuts[k])) return RDK_FAILURE;
   }
   return RDK_SUCCESS;
 }
