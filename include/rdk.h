@@ -468,6 +468,28 @@ int rdk_rell_support_ms(rdk_partition_t *const *partitions, unsigned int n,
                         unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
                         rdk_rell_ms_out_t *ms);
 
+/* Gene and gene-then-site resampling of n >= 2 whole partitions (DESIGN.md section 10, items
+ * 11-14), with everything rdk_rell_support computes (it fills *out the same way).  Replicate b draws
+ * n partitions with replacement, draw j = word j of Philox4x64-10 keyed {seed, b} from the counter
+ * {0, 0, 1, 0} picking partition (x_j n) >> 64; m[b][i] = how often it drew partition i.
+ * RDK_RELL_GENE: Z[b][r] = sum_i m[b][i] O_i[r].  RDK_RELL_GENE_SITE: replicate b takes the first
+ * m[b][i] N_i draws of rdk_rell_support's stream of partition i (m = 1: exactly its draws).  O_i is
+ * O over partition i alone (O = sum_i O_i).  Refuses site shards, n * max_i N_i >= 2^32 and
+ * replicates outside [1, 2^20]. */
+#define RDK_RELL_GENE      1u
+#define RDK_RELL_GENE_SITE 2u
+typedef struct rdk_rell_gene_out_t {
+  unsigned int        sampling;            /* in: RDK_RELL_GENE or RDK_RELL_GENE_SITE */
+  double             *partition_lnl_fixed; /* out: [n][rows], O_i[r] * 2^-e rounded once */
+  unsigned long long *o_lo;                /* out (optional): [n][rows] O_i[r] as int128, low word */
+  long long          *o_hi;                /* ... high word */
+  double              draws_ms;            /* out: device time of the gene draws (out->ms has the rest) */
+} rdk_rell_gene_out_t;
+int rdk_rell_support_genes(rdk_partition_t *const *partitions, unsigned int n,
+                           const unsigned int *global_index, unsigned int rows,
+                           unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
+                           rdk_rell_gene_out_t *genes);
+
 #ifdef __cplusplus
 }
 #endif

@@ -832,6 +832,13 @@ def _bind_model(L: C.CDLL):
                                            C.c_uint, C.POINTER(ull), _dp, _dp, _dp, C.POINTER(ull),
                                            C.POINTER(C.c_longlong), _up, _up, _up, _up, _dp, _dp, _dp, _dp, _up, _dp,
                                            C.POINTER(ull), C.POINTER(C.c_int), _up, _dp, _up]
+    gene_outputs = [_dp, C.POINTER(ull), C.POINTER(C.c_longlong), _up, C.POINTER(C.c_int), _up, _dp, _up]
+    L.rdh_model_placement_support_genes.argtypes = [vp, C.c_char_p, ull, ull, C.c_uint, C.c_int, C.c_uint, C.c_uint,
+                                                    C.POINTER(ull), _dp, _dp, _dp, C.POINTER(ull),
+                                                    C.POINTER(C.c_longlong), _up, _up, _up] + gene_outputs
+    L.rdh_model_branch_support_genes.argtypes = [vp, C.c_char_p, ull, ull, C.c_double, C.c_uint, C.c_int, C.c_uint,
+                                                 C.c_uint, C.POINTER(ull), _dp, _dp, _dp, C.POINTER(ull),
+                                                 C.POINTER(C.c_longlong), _up, _up, _up] + gene_outputs
     L.rdh_placement_au_fit.argtypes = [_up, C.c_uint, _up, ull, _dp, _up]
     L.rdh_model_site_lnl_rows.argtypes = [vp, C.c_uint, _dp, ull, _up, C.c_uint, C.POINTER(ull)]
     L.rdh_model_assign_indicies.argtypes = [vp, C.c_int, C.c_uint, C.c_double, C.c_uint, C.c_uint, C.c_int, _up,
@@ -1234,8 +1241,56 @@ class Model:
                                                      len(out), C.byref(got)))
         return out[:got.value].tolist()
 
+    SAMPLING = {"gene": 1, "gene_site": 2}
+
+    def _gene_sampling(self, who, sampling, au_scales):
+        """the C code of a gene mode, or None for site resampling"""
+        if sampling == "site":
+            return None
+        if sampling not in self.SAMPLING:
+            raise ValueError("%s: unknown sampling %r (site, gene or gene_site)" % (who, sampling))
+        if au_scales is not None:
+            raise ValueError("%s: the AU test and ELW (au_scales) are not available with gene sampling" % who)
+        return self.SAMPLING[sampling]
+
+    def _support_genes(self, call, cap, args, retry):
+        """one gene-mode support entry (placement or branch) and its result dict"""
+        G = self.partition_count
+        ull = C.POINTER(C.c_ulonglong)
+        for attempt in range(2):
+            ids = np.zeros(cap, dtype=np.uint64)
+            alpha, llh, fixed = np.zeros(cap), np.zeros(cap), np.zeros(cap)
+            o_lo, o_hi = np.zeros(cap, dtype=np.uint64), np.zeros(cap, dtype=np.int64)
+            bp, kh, sh = (np.zeros(cap, dtype=np.uint32) for _ in range(3))
+            p_fixed = np.zeros((G, cap))
+            p_lo, p_hi = np.zeros((G, cap), dtype=np.uint64), np.zeros((G, cap), dtype=np.int64)
+            p_best = np.zeros(G, dtype=np.uint32)
+            exponent, best, got = C.c_int(), C.c_uint(), C.c_uint()
+            info = np.zeros(8)
+            rc = call(*args, cap, _ptr(ids, ull), _ptr(alpha, _dp), _ptr(llh, _dp), _ptr(fixed, _dp), _ptr(o_lo, ull),
+                      _ptr(o_hi, C.POINTER(C.c_longlong)), _ptr(bp, _up), _ptr(kh, _up), _ptr(sh, _up),
+                      _ptr(p_fixed, _dp), _ptr(p_lo, ull), _ptr(p_hi, C.POINTER(C.c_longlong)), _ptr(p_best, _up),
+                      C.byref(exponent), C.byref(best), _ptr(info, _dp), C.byref(got))
+            if rc or attempt or not retry or got.value <= cap:
+                break
+            cap = got.value  # the log holds more records than the first buffers: nothing was computed
+        self._check(rc)
+        n = got.value
+        B = float(args[2])
+        O = [(int(h) << 64) | int(l) for l, h in zip(o_lo[:n], o_hi[:n])]
+        return {"root_id": ids[:n].copy(), "alpha": alpha[:n].copy(), "llh": llh[:n].copy(),
+                "lnl_fixed": fixed[:n].copy(), "O": O, "bp_count": bp[:n].copy(), "kh_count": kh[:n].copy(),
+                "sh_count": sh[:n].copy(), "bp": bp[:n] / B, "p_kh": kh[:n] / B, "p_sh": sh[:n] / B,
+                "exponent": exponent.value, "best": best.value, "replicates": int(args[2]),
+                "capture_ms": info[0], "counts_ms": info[1], "accumulate_ms": info[2], "statistics_ms": info[3],
+                "resample_ms": info[4], "device_bytes": int(info[5]), "gene_draws_ms": info[6],
+                "positions_ms": info[7], "partition_llh": p_fixed[:, :n].copy(),
+                "partition_O": [[(int(h) << 64) | int(l) for l, h in zip(p_lo[i, :n], p_hi[i, :n])] for i in range(G)],
+                "partition_best": p_best.copy()}
+
     def placement_support(self, checkpoint_prefix: str | None = None, replicates: int = 10000, seed: int = 0,
-                          replicate_tile: int = 0, keep_rows: bool = False, au_scales=None) -> dict:
+                          replicate_tile: int = 0, keep_rows: bool = False, au_scales=None,
+                          sampling: str = "site") -> dict:
         """RELL bootstrap proportions and one-sided KH / SH tests of every placement recorded in
         "<checkpoint_prefix>.ckp" (opened read-only; None: the model's own result log, e.g. of
         exhaustive_search), from `replicates` (1..2^20) resamplings of the sites, each partition on
@@ -1254,7 +1309,25 @@ class Model:
         with 0 < count < replicates), elw and elw_fixed (elw = elw_fixed 2^-40 / replicates), and
         au_counts_ms, au_accumulate_ms, au_statistics_ms; the branches also carry pAU and ELW.  The
         fit is the two-parameter model of Shimodaira (2002) without the iterated threshold
-        refinement of CONSEL and IQ-TREE, so p_au may differ from theirs."""
+        refinement of CONSEL and IQ-TREE, so p_au may differ from theirs.
+
+        sampling chooses what a replicate resamples (DESIGN.md section 10, items 11-14): "site" (the
+        above), "gene" (the model's partitions, with replacement) or "gene_site" (partitions, then
+        the sites of each drawn partition, as Gadagkar, Rosenberg & Kumar 2005).  The gene modes need
+        at least 2 partitions and refuse au_scales; the counts come from the chosen resampling, and
+        the result adds sampling, partition_llh [partition][record] (O_i 2^-exponent, the gene-wise
+        log-likelihoods), partition_O (Python ints), partition_best (each partition's record of the
+        highest log-likelihood) and gene_draws_ms."""
+        mode = self._gene_sampling("placement_support", sampling, au_scales)
+        if mode is not None:
+            prefix = checkpoint_prefix.encode() if checkpoint_prefix is not None else None
+            args = (self.h, prefix, int(replicates), int(seed) & ((1 << 64) - 1), int(replicate_tile),
+                    1 if keep_rows else 0, mode)
+            out = self._support_genes(self.L.rdh_model_placement_support_genes, 128, args, retry=True)
+            del out["positions_ms"]
+            self._support_rows = len(out["root_id"]) if keep_rows else 0
+            out["sampling"] = sampling
+            return out
         if au_scales is not None:
             return self._placement_support_au(checkpoint_prefix, replicates, seed, replicate_tile, keep_rows,
                                               au_thousandths(au_scales))
@@ -1330,7 +1403,8 @@ class Model:
                 "au_accumulate_ms": info[7], "au_statistics_ms": info[8]}
 
     def branch_support(self, checkpoint_prefix: str | None = None, replicates: int = 10000, seed: int = 0,
-                       atol: float = 1e-14, replicate_tile: int = 0, keep_rows: bool = False, au_scales=None) -> dict:
+                       atol: float = 1e-14, replicate_tile: int = 0, keep_rows: bool = False, au_scales=None,
+                       sampling: str = "site") -> dict:
         """The statistics of placement_support for EVERY branch, at one set of parameters (DESIGN.md
         section 10, items 9-10): the parameters of the best record of "<checkpoint_prefix>.ckp" (None:
         the model's own result log; highest llh, lowest log index on ties) are installed, root q is
@@ -1341,8 +1415,17 @@ class Model:
         Returns the keys of placement_support (with or without au_scales): root_id = 0..root_count-1,
         alpha = a_q, llh = the log-likelihood at (q, a_q); plus positions_ms (the alpha searches).
         capture_ms is the one placement sweep that scores all branches and stores their rows.  Every
-        branch carries BP, pKH, pSH (pAU, ELW) and its LLH and alpha in newick(True)."""
+        branch carries BP, pKH, pSH (pAU, ELW) and its LLH and alpha in newick(True).  sampling is
+        placement_support's: "gene" and "gene_site" add the same per-partition keys."""
         prefix = checkpoint_prefix.encode() if checkpoint_prefix is not None else None
+        mode = self._gene_sampling("branch_support", sampling, au_scales)
+        if mode is not None:
+            args = (self.h, prefix, int(replicates), int(seed) & ((1 << 64) - 1), float(atol), int(replicate_tile),
+                    1 if keep_rows else 0, mode)
+            out = self._support_genes(self.L.rdh_model_branch_support_genes, self.root_count, args, retry=False)
+            self._support_rows = len(out["root_id"]) if keep_rows else 0
+            out["sampling"] = sampling
+            return out
         sc = np.ascontiguousarray(au_thousandths(au_scales) if au_scales is not None else [], dtype=np.uint32)
         K, n = len(sc), self.root_count
         ull = C.POINTER(C.c_ulonglong)

@@ -1531,7 +1531,7 @@ extern "C" int rdk_partition_permute_site_lnl_rows(rdk_partition_t *p, unsigned 
 
 static int rell_entry(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
                       unsigned int rows, unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
-                      rdk_rell_ms_out_t *ms) {
+                      rdk_rell_ms_out_t *ms, rdk_rell_gene_out_t *genes) {
   if (n == 0 || rows == 0) return fail(RDK_ERROR_PARAM, "rdk_rell_support: no partitions or no rows");
   if (replicates == 0 || replicates > kRellMaxReplicates)
     return fail(RDK_ERROR_PARAM, "rdk_rell_support: replicates must be in [1, 2^20]");
@@ -1542,6 +1542,7 @@ static int rell_entry(rdk_partition_t *const *parts, unsigned int n, const unsig
     Engine *e = eng(parts[i]);
     if (e->device != device) return fail(RDK_ERROR_PARAM, "rdk_rell_support: partitions on different devices");
     if (e->comm) {
+      if (genes) return fail(RDK_ERROR_PARAM, "rdk_rell_support_genes: gene resampling needs whole partitions, not a site shard");
       if (n != 1) return fail(RDK_ERROR_PARAM, "rdk_rell_support: a site shard must be the only partition");
       shard.comm = e->comm;
       shard.nranks = e->nranks;
@@ -1562,9 +1563,20 @@ static int rell_entry(rdk_partition_t *const *parts, unsigned int n, const unsig
     rp[i].patterns = e->S;
     rp[i].global_index = global_index ? global_index[i] : i;
   }
+  if (genes) {  // item 14: n N_max < 2^32 keeps |Z| < 2^84
+    unsigned long long n_max = 0;
+    for (unsigned i = 0; i < n; ++i) {
+      unsigned long long N = 0;
+      for (unsigned p = 0; p < rp[i].patterns; ++p) N += rp[i].weights[p];
+      n_max = std::max(n_max, N);
+    }
+    if ((unsigned long long)n * n_max >= (1ull << 32))
+      return fail(RDK_ERROR_PARAM, "rdk_rell_support_genes: %u partitions x %llu sites (the largest) reach 2^32", n,
+                  n_max);
+  }
   CUDA_TRY(cudaSetDevice(device));
   char msg[256];
-  if (!rell_support(rp.data(), n, rows, replicates, seed, shard, out, ms, msg, sizeof(msg)))
+  if (!rell_support(rp.data(), n, rows, replicates, seed, shard, out, ms, genes, msg, sizeof(msg)))
     return fail(RDK_ERROR_CUDA, "%s", msg);
   return RDK_SUCCESS;
 }
@@ -1572,7 +1584,7 @@ static int rell_entry(rdk_partition_t *const *parts, unsigned int n, const unsig
 extern "C" int rdk_rell_support(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
                                 unsigned int rows, unsigned long long replicates, unsigned long long seed,
                                 rdk_rell_out_t *out) {
-  return rell_entry(parts, n, global_index, rows, replicates, seed, out, nullptr);
+  return rell_entry(parts, n, global_index, rows, replicates, seed, out, nullptr, nullptr);
 }
 
 extern "C" int rdk_rell_support_ms(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
@@ -1588,7 +1600,18 @@ extern "C" int rdk_rell_support_ms(rdk_partition_t *const *parts, unsigned int n
     if (k && ms->scales[k] <= ms->scales[k - 1])
       return fail(RDK_ERROR_PARAM, "rdk_rell_support_ms: scales must be strictly ascending");
   }
-  return rell_entry(parts, n, global_index, rows, replicates, seed, out, ms);
+  return rell_entry(parts, n, global_index, rows, replicates, seed, out, ms, nullptr);
+}
+
+extern "C" int rdk_rell_support_genes(rdk_partition_t *const *parts, unsigned int n, const unsigned int *global_index,
+                                      unsigned int rows, unsigned long long replicates, unsigned long long seed,
+                                      rdk_rell_out_t *out, rdk_rell_gene_out_t *genes) {
+  if (!genes || !genes->partition_lnl_fixed)
+    return fail(RDK_ERROR_PARAM, "rdk_rell_support_genes: null output arrays");
+  if (genes->sampling != RDK_RELL_GENE && genes->sampling != RDK_RELL_GENE_SITE)
+    return fail(RDK_ERROR_PARAM, "rdk_rell_support_genes: unknown sampling mode %u", genes->sampling);
+  if (n < 2) return fail(RDK_ERROR_PARAM, "rdk_rell_support_genes: %u partitions, at least 2 are needed", n);
+  return rell_entry(parts, n, global_index, rows, replicates, seed, out, nullptr, genes);
 }
 
 // ---------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-// rdk_support.cu -- the three kernels of rdk_rell_support (DESIGN.md section 10).
+// rdk_support.cu -- the kernels of rdk_rell_support and its variants (DESIGN.md section 10).
 //
 //   counts        c[b][p]: Philox4x64-10 draws of the original sites of a partition, mapped to
 //                 their pattern by a binary search in the cumulative weights (integer atomics);
@@ -8,6 +8,9 @@
 //   statistics    column sums over b, row maxima over r, then the KH / SH / BP counts per record
 //   AU / ELW      (rdk_rell_support_ms) the ELW quotients on the unit-scale Z, summed by the column-sum
 //                 kernels; then per further scale the same counts and accumulation, argmax and histogram
+//   genes         (rdk_rell_support_genes) per replicate tile the gene draws m[b][i] (integer histogram);
+//                 then Z = m O_i (gene), or counts of m[b][i] N_i site draws per partition found through
+//                 a prefix sum of the replicates' Philox blocks, accumulated as above (gene_site)
 //
 // Every sum is an exact integer, so the result does not depend on launch shape or tiling.
 #include "rdk_support.cuh"
@@ -233,6 +236,121 @@ __global__ void rell_hist_kernel(const unsigned *argmax, unsigned nb, unsigned *
   if (b < nb) atomicAdd(count + argmax[b], 1u);
 }
 
+// ---- gene and gene-then-site resampling (DESIGN.md section 10, items 11-13)
+
+// m[b][i] for replicates [b0, b0 + tile): one thread = one Philox block (counter {j + 1, 0, 1, 0},
+// key {seed, b}) = 4 of the G draws, each picking partition (x G) >> 64
+__global__ void rell_gene_draws_kernel(unsigned long long seed, unsigned long long b0, unsigned tile, unsigned G,
+                                       unsigned *m) {
+  const unsigned long long blocks = (G + 3) / 4, total = blocks * tile;
+  for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < total;
+       i += (unsigned long long)gridDim.x * blockDim.x) {
+    const unsigned long long b = i / blocks, j4 = i - b * blocks;
+    unsigned long long       x[4] = {j4 + 1, 0, 1, 0};
+    philox4x64_10(x, seed, b0 + b);
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      if (j4 * 4 + u >= G) break;
+      atomicAdd(m + b * G + __umul64hi(x[u], G), 1u);
+    }
+  }
+}
+
+// off[b] = sum over b' < b of the Philox blocks replicate b' draws from partition g (m[b'][g] N
+// draws, 4 per block), off[tile] = the total: one block of 1024 threads, each summing a run of
+// replicates, then a scan of the 1024 run sums
+__global__ void __launch_bounds__(1024) rell_gene_offsets_kernel(const unsigned *m, unsigned G, unsigned g,
+                                                                 unsigned tile, unsigned long long N,
+                                                                 unsigned long long *off) {
+  __shared__ unsigned long long run[1024];
+  const unsigned per = (tile + 1023) / 1024, first = threadIdx.x * per, last = min(tile, first + per);
+  unsigned long long s = 0;
+  for (unsigned b = first; b < last; ++b) s += (m[(size_t)b * G + g] * N + 3) / 4;
+  run[threadIdx.x] = s;
+  __syncthreads();
+  for (unsigned d = 1; d < 1024; d <<= 1) {
+    const unsigned long long v = threadIdx.x >= d ? run[threadIdx.x - d] : 0;
+    __syncthreads();
+    run[threadIdx.x] += v;
+    __syncthreads();
+  }
+  s = run[threadIdx.x] - s;  // exclusive
+  for (unsigned b = first; b < last; ++b) {
+    off[b] = s;
+    s += (m[(size_t)b * G + g] * N + 3) / 4;
+  }
+  if (threadIdx.x == 1023) off[tile] = run[1023];
+}
+
+// c[b][p] of gene-then-site resampling for partition g: as rell_counts_kernel with word 0 and an
+// unsharded partition, but replicate b draws m[b][g] N of its sites; thread i takes block i - off[b]
+// of the replicate b with off[b] <= i < off[b + 1]
+__global__ void rell_gene_counts_kernel(unsigned long long seed, unsigned long long global_index,
+                                        unsigned long long b0, unsigned tile, const unsigned *m, unsigned G,
+                                        unsigned g, unsigned long long N, const unsigned long long *off,
+                                        const unsigned long long *cumw, unsigned patterns, unsigned *c) {
+  const unsigned long long total = off[tile];
+  for (unsigned long long i = blockIdx.x * (unsigned long long)blockDim.x + threadIdx.x; i < total;
+       i += (unsigned long long)gridDim.x * blockDim.x) {
+    unsigned b = 0, hi = tile;  // the last b with off[b] <= i: a replicate without draws is skipped
+    while (hi - b > 1) {
+      const unsigned mid = (b + hi) / 2;
+      if (off[mid] <= i)
+        b = mid;
+      else
+        hi = mid;
+    }
+    const unsigned long long j4 = i - off[b], draws = m[(size_t)b * G + g] * N;
+    unsigned long long       x[4] = {j4 + 1, 0, 0, 0};
+    philox4x64_10(x, seed, (global_index << 32) | (b0 + b));
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      if (j4 * 4 + u >= draws) break;
+      const unsigned long long site = __umul64hi(x[u], N);
+      unsigned                 p = 0, top = patterns;  // cumw[p] <= site < cumw[top]
+      while (top - p > 1) {
+        const unsigned mid = (p + top) / 2;
+        if (cumw[mid] <= site)
+          p = mid;
+        else
+          top = mid;
+      }
+      atomicAdd(c + (size_t)b * patterns + p, 1u);
+    }
+  }
+}
+
+// Z[b][r] = sum_i m[b][i] O_i[r] for b < nb, r < nr, with 32 x 32 tiles of m and O_i in shared memory
+__global__ void __launch_bounds__(256) rell_gene_accumulate_kernel(const unsigned *m, unsigned G, const i128 *oi,
+                                                                   unsigned nb, unsigned nr, i128 *z,
+                                                                   size_t z_stride) {
+  __shared__ unsigned ms[kTile][kTile + 1];
+  __shared__ i128     os[kTile][kTile];
+  const unsigned tx = threadIdx.x & 31, ty = threadIdx.x >> 5;  // 32 x 8
+  const unsigned b_base = blockIdx.y * kTile, r_base = blockIdx.x * kTile;
+  i128           acc[4] = {0, 0, 0, 0};
+  for (unsigned i0 = 0; i0 < G; i0 += kTile) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const unsigned row = ty + 8 * k, i = i0 + tx;
+      ms[row][tx] = (b_base + row < nb && i < G) ? m[(size_t)(b_base + row) * G + i] : 0u;
+      os[row][tx] = (i0 + row < G && r_base + tx < nr) ? oi[(size_t)(i0 + row) * nr + r_base + tx] : (i128)0;
+    }
+    __syncthreads();
+    for (int ii = 0; ii < kTile; ++ii) {
+      const i128 o = os[ii][tx];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) acc[k] += (i128)ms[ty + 8 * k][ii] * o;
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const unsigned b = b_base + ty + 8 * k, r = r_base + tx;
+    if (b < nb && r < nr) z[(size_t)b * z_stride + r] = acc[k];
+  }
+}
+
 // ---- expected likelihood weights (DESIGN.md section 10, item 8)
 
 // int128 -> double, rounded to nearest even: the top 64 bits with the rest folded into a sticky bit
@@ -351,7 +469,7 @@ struct DeviceBuffers {
 };
 
 struct Events {
-  cudaEvent_t ev[8] = {};
+  cudaEvent_t ev[10] = {};
   ~Events() {
     for (cudaEvent_t e : ev)
       if (e) cudaEventDestroy(e);
@@ -372,7 +490,7 @@ struct Events {
 
 int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, unsigned long long replicates,
                  unsigned long long seed, const RellShard &shard, rdk_rell_out_t *out, rdk_rell_ms_out_t *ms,
-                 char *msg, size_t msg_cap) {
+                 rdk_rell_gene_out_t *genes, char *msg, size_t msg_cap) {
   cudaStream_t  stream = nullptr;
   DeviceBuffers buf;
   Events        ev;
@@ -459,8 +577,9 @@ int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, 
   // ---- per-partition inputs: cumulative weights, weights as a 1-row count matrix
   size_t max_patterns = 1;
   for (unsigned g = 0; g < n; ++g) max_patterns = std::max<size_t>(max_patterns, parts[g].patterns);
+  const size_t   per_replicate = genes ? std::max<size_t>(max_patterns, n) : max_patterns;  // c and m per tile
   const unsigned tile = (unsigned)std::max<unsigned long long>(
-      1, std::min<unsigned long long>(out->replicate_tile ? out->replicate_tile : kCountsBytes / (4 * max_patterns),
+      1, std::min<unsigned long long>(out->replicate_tile ? out->replicate_tile : kCountsBytes / (4 * per_replicate),
                                       nb));
   std::vector<unsigned long long *> d_cumw(n);
   std::vector<unsigned *>           d_w(n);
@@ -479,33 +598,72 @@ int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, 
   }
 
   unsigned *d_c = nullptr;
-  i128     *d_z = nullptr, *d_o = nullptr;
+  i128     *d_z = nullptr, *d_o = nullptr, *d_oi = nullptr;
   RELL_TRY(buf.alloc(&d_c, (size_t)tile * max_patterns));
   RELL_TRY(buf.alloc(&d_z, (size_t)nb * rows));
   RELL_TRY(buf.alloc(&d_o, rows));
+  RELL_TRY(buf.alloc(&d_oi, (size_t)n * rows));
+  unsigned           *d_m = nullptr;  // gene modes: m[b][i] of a tile, and gene_site's block offsets
+  unsigned long long *d_off = nullptr;
+  if (genes) {
+    RELL_TRY(buf.alloc(&d_m, (size_t)tile * n));
+    if (genes->sampling == RDK_RELL_GENE_SITE) RELL_TRY(buf.alloc(&d_off, (size_t)tile + 1));
+  }
 
-  // ---- O[r] = sum_g sum_p w q (the weights are a count matrix of one replicate)
+  // ---- O_g[r] = sum_p w q (the weights are a count matrix of one replicate), O[r] = sum_g O_g[r]
   const dim3 acc_threads(256);
   for (unsigned g = 0; g < n; ++g) {
     const dim3 grid((rows + kTile - 1) / kTile, 1);
     rell_accumulate_kernel<<<grid, acc_threads, 0, stream>>>(d_w[g], parts[g].rows, parts[g].patterns, 1, rows, e,
-                                                             g > 0, d_o, rows);
+                                                             0, d_oi + (size_t)g * rows, rows);
     RELL_TRY(cudaGetLastError());
   }
+  rell_colsum_kernel<<<(rows + 127) / 128, 128, 0, stream>>>(d_oi, n, rows, n, d_o);
+  RELL_TRY(cudaGetLastError());
 
   // ---- counts and accumulation, tile by tile, of the replicates at one scale (thousandths; the
   // counter word is s - 1000 mod 2^64, so scale 1000 is word 0 and N_g draws)
-  float t_counts = 0, t_acc = 0, t_stats = 0, t_ms = 0;
+  // (gene modes: first the gene draws of the tile; then Z = m O_g, or the counts of m[b][g] N_g draws)
+  float t_counts = 0, t_acc = 0, t_stats = 0, t_ms = 0, t_draws = 0;
   auto  resample = [&](unsigned scale, float &counts_ms, float &acc_ms) -> int {
     const unsigned long long word = (unsigned long long)scale - 1000ull;
     for (unsigned long long b0 = 0; b0 < nb; b0 += tile) {
       const unsigned nt = (unsigned)std::min<unsigned long long>(tile, nb - b0);
+      if (genes) {
+        RELL_TRY(cudaEventRecord(ev.ev[8], stream));
+        RELL_TRY(cudaMemsetAsync(d_m, 0, sizeof(unsigned) * (size_t)nt * n, stream));
+        const unsigned long long work = (n + 3) / 4 * (unsigned long long)nt;
+        rell_gene_draws_kernel<<<(unsigned)std::min<unsigned long long>((work + 255) / 256, (unsigned long long)sms * 16),
+                                 256, 0, stream>>>(seed, b0, nt, n, d_m);
+        RELL_TRY(cudaGetLastError());
+        RELL_TRY(cudaEventRecord(ev.ev[9], stream));
+        if (genes->sampling == RDK_RELL_GENE) {
+          const dim3 grid((rows + kTile - 1) / kTile, (nt + kTile - 1) / kTile);
+          rell_gene_accumulate_kernel<<<grid, acc_threads, 0, stream>>>(d_m, n, d_oi, nt, rows, d_z + b0 * rows, rows);
+          RELL_TRY(cudaGetLastError());
+        }
+        RELL_TRY(cudaEventRecord(ev.ev[2], stream));
+        RELL_TRY(cudaEventSynchronize(ev.ev[2]));
+        float t = 0;
+        RELL_TRY(cudaEventElapsedTime(&t, ev.ev[8], ev.ev[9]));
+        t_draws += t;
+        RELL_TRY(cudaEventElapsedTime(&t, ev.ev[9], ev.ev[2]));
+        acc_ms += t;
+        if (genes->sampling == RDK_RELL_GENE) continue;
+      }
       for (unsigned g = 0; g < n; ++g) {
         const unsigned           P = parts[g].patterns;
         const unsigned long long draws = std::max<unsigned long long>(1, (scale * sites[g] + 500) / 1000);
         RELL_TRY(cudaEventRecord(ev.ev[0], stream));
         RELL_TRY(cudaMemsetAsync(d_c, 0, sizeof(unsigned) * (size_t)nt * std::max(1u, P), stream));
-        if (sites[g]) {
+        if (sites[g] && genes) {
+          rell_gene_offsets_kernel<<<1, 1024, 0, stream>>>(d_m, n, g, nt, sites[g], d_off);
+          const unsigned long long work = (sites[g] + 3) / 4 * nt;  // the expected blocks: E[m] = 1
+          const unsigned grid = (unsigned)std::min<unsigned long long>((work + 255) / 256, (unsigned long long)sms * 16);
+          rell_gene_counts_kernel<<<grid, 256, 0, stream>>>(seed, parts[g].global_index, b0, nt, d_m, n, g, sites[g],
+                                                            d_off, d_cumw[g], P, d_c);
+          RELL_TRY(cudaGetLastError());
+        } else if (sites[g]) {
           const unsigned long long work = (draws + 3) / 4 * nt;
           const unsigned grid = (unsigned)std::min<unsigned long long>((work + 255) / 256, (unsigned long long)sms * 16);
           rell_counts_kernel<<<grid, 256, 0, stream>>>(seed, parts[g].global_index, b0, nt, draws, word, sites[g], lo,
@@ -626,6 +784,17 @@ int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, 
     ms->ms[0] = t_ms_counts;
     ms->ms[1] = t_ms_acc;
     ms->ms[2] = t_ms_stats;
+  }
+  if (genes) {
+    std::vector<i128> oi((size_t)n * rows);
+    RELL_TRY(cudaMemcpyAsync(oi.data(), d_oi, sizeof(i128) * oi.size(), cudaMemcpyDeviceToHost, stream));
+    RELL_TRY(cudaStreamSynchronize(stream));
+    for (size_t i = 0; i < oi.size(); ++i) {
+      genes->partition_lnl_fixed[i] = ldexp((double)oi[i], -e);
+      if (genes->o_lo) genes->o_lo[i] = (unsigned long long)(u128)oi[i];
+      if (genes->o_hi) genes->o_hi[i] = (long long)(oi[i] >> 64);
+    }
+    genes->draws_ms = t_draws;
   }
 
   out->ms[0] = t_counts;

@@ -34,10 +34,12 @@ struct RellShard {
 };
 
 // runs on the current device; returns 0 with a message in msg on failure.  ms (validated by the
-// caller; null for rdk_rell_support) adds the multiscale counts and the ELW of rdk_rell_support_ms.
+// caller; null for rdk_rell_support) adds the multiscale counts and the ELW of rdk_rell_support_ms;
+// genes (validated by the caller; null for site resampling) resamples genes as
+// rdk_rell_support_genes does.
 int rell_support(const RellPartition *parts, unsigned int n, unsigned int rows, unsigned long long replicates,
                  unsigned long long seed, const RellShard &shard, rdk_rell_out_t *out, rdk_rell_ms_out_t *ms,
-                 char *msg, size_t msg_cap);
+                 rdk_rell_gene_out_t *genes, char *msg, size_t msg_cap);
 
 }  // namespace rdk
 

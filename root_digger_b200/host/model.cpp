@@ -22,6 +22,7 @@
 #ifdef RD_BACKEND_ORACLE
 #include "rdk_support.h"     // tests/oracle_shim: the placement-support entries over the CPU oracle
 #include "rdk_support_au.h"  // ... and rdk_rell_support_ms
+#include "rdk_support_genes.h"  // ... and rdk_rell_support_genes
 #include "rdk_sweep_rows.h"   // ... and the row capture of the placement sweep
 #endif
 #include "support_stats.hpp"
@@ -964,12 +965,19 @@ std::pair<root_location_t, double> model_t::exhaustive_search(double atol, doubl
 // ---------------------------------------------------------------------------
 // what both support calls refuse before any work
 void model_t::check_support_request(const std::string &who, size_t replicates,
-                                    const std::vector<unsigned> &au_scales) const {
+                                    const std::vector<unsigned> &au_scales, support_sampling_t sampling) const {
   if (_exchange)
     throw std::invalid_argument(who + ": a model whose partitions are dealt to several processes is not supported");
   if (replicates == 0 || replicates > (size_t(1) << 20))
     throw std::invalid_argument(who + ": replicates must be between 1 and 2^20");
   if (!au_scales.empty()) rd::check_au_scales(au_scales.data(), au_scales.size());
+  if (sampling != support_sampling_t::site) {
+    if (!au_scales.empty())
+      throw std::invalid_argument(who + ": the AU test and ELW (au_scales) are not available with gene sampling");
+    if (_partitions.size() < 2)
+      throw std::invalid_argument(who + ": gene sampling needs at least 2 partitions, the model has " +
+                                  std::to_string(_partitions.size()));
+  }
 }
 
 void model_t::check_support_records(const std::string &who, const std::vector<checkpoint_t::record_t> &records) const {
@@ -1055,10 +1063,12 @@ void model_t::reserve_support_rows(const std::string &who, unsigned rows) {
   _support_rows = rows;
 }
 
-// the statistics of DESIGN.md section 10, items 2-8, over rows 0..rows-1 of the partitions' site
-// matrices (rdk_rell_support, or rdk_rell_support_ms in AU mode)
+// the statistics of DESIGN.md section 10, items 2-8 and 11-14, over rows 0..rows-1 of the partitions'
+// site matrices (rdk_rell_support, rdk_rell_support_ms in AU mode, rdk_rell_support_genes in the gene
+// modes)
 void model_t::resample_support(const std::string &who, placement_support_t &out, unsigned rows, size_t replicates,
-                               uint64_t seed, unsigned replicate_tile, const std::vector<unsigned> &au_scales) {
+                               uint64_t seed, unsigned replicate_tile, const std::vector<unsigned> &au_scales,
+                               support_sampling_t sampling) {
   const bool            au = !au_scales.empty();
   std::vector<unsigned> global_index(_partitions.size());
   std::iota(global_index.begin(), global_index.end(), 0u);
@@ -1094,6 +1104,31 @@ void model_t::resample_support(const std::string &who, placement_support_t &out,
     out.au_counts_ms = ms.ms[0];
     out.au_accumulate_ms = ms.ms[1];
     out.au_statistics_ms = ms.ms[2];
+  } else if (sampling != support_sampling_t::site) {
+    const size_t n = _partitions.size();
+    out.sampling = sampling;
+    out.partition_lnl_fixed.resize(n * rows);
+    out.partition_o_lo.resize(n * rows);
+    out.partition_o_hi.resize(n * rows);
+    rdk_rell_gene_out_t genes;
+    memset(&genes, 0, sizeof(genes));
+    genes.sampling = sampling == support_sampling_t::gene ? RDK_RELL_GENE : RDK_RELL_GENE_SITE;
+    genes.partition_lnl_fixed = out.partition_lnl_fixed.data();
+    genes.o_lo = out.partition_o_lo.data();
+    genes.o_hi = out.partition_o_hi.data();
+    if (rdk_rell_support_genes(_partitions.data(), (unsigned)n, global_index.data(), rows, replicates, seed, &rell,
+                               &genes) != RDK_SUCCESS)
+      throw std::runtime_error(who + ": " + engine_error());
+    out.gene_draws_ms = genes.draws_ms;
+    auto o_i = [&](size_t i) {
+      return (__int128)(((unsigned __int128)(unsigned long long)out.partition_o_hi[i] << 64) | out.partition_o_lo[i]);
+    };
+    for (size_t p = 0; p < n; ++p) {
+      unsigned top = 0;
+      for (unsigned r = 1; r < rows; ++r)
+        if (o_i(p * rows + r) > o_i(p * rows + top)) top = r;
+      out.partition_best.push_back(top);
+    }
   } else if (rdk_rell_support(_partitions.data(), (unsigned)_partitions.size(), global_index.data(), rows,
                               replicates, seed, &rell) != RDK_SUCCESS) {
     throw std::runtime_error(who + ": " + engine_error());
@@ -1138,9 +1173,10 @@ void model_t::annotate_support(placement_support_t &out, const std::vector<root_
 
 model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
                                                         unsigned replicate_tile, bool keep_rows,
-                                                        const std::vector<unsigned> &au_scales) {
+                                                        const std::vector<unsigned> &au_scales,
+                                                        support_sampling_t sampling) {
   const std::string who = "placement_support";
-  check_support_request(who, replicates, au_scales);
+  check_support_request(who, replicates, au_scales, sampling);
   const auto records = checkpoint.read_results();
   check_support_records(who, records);
 
@@ -1166,7 +1202,7 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
       }
     }
     out.capture_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    resample_support(who, out, rows, replicates, seed, replicate_tile, au_scales);
+    resample_support(who, out, rows, replicates, seed, replicate_tile, au_scales, sampling);
   } catch (...) {
     restore();
     throw;
@@ -1186,9 +1222,10 @@ model_t::placement_support_t model_t::placement_support(checkpoint_t &checkpoint
 
 model_t::placement_support_t model_t::branch_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
                                                      double atol, unsigned replicate_tile, bool keep_rows,
-                                                     const std::vector<unsigned> &au_scales) {
+                                                     const std::vector<unsigned> &au_scales,
+                                                     support_sampling_t sampling) {
   const std::string who = "branch_support";
-  check_support_request(who, replicates, au_scales);
+  check_support_request(who, replicates, au_scales, sampling);
   if (!(atol >= 0.0 && atol <= std::numeric_limits<double>::max()))
     throw std::invalid_argument(who + ": atol must be finite and non-negative");
   const auto records = checkpoint.read_results();
@@ -1246,7 +1283,7 @@ model_t::placement_support_t model_t::branch_support(checkpoint_t &checkpoint, s
     out.capture_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t2).count();
     for (double v : llh)
       if (std::isnan(v)) throw std::runtime_error(who + ": lh at root is not a number");
-    resample_support(who, out, rows, replicates, seed, replicate_tile, au_scales);
+    resample_support(who, out, rows, replicates, seed, replicate_tile, au_scales, sampling);
   } catch (...) {
     restore();
     throw;

@@ -188,6 +188,11 @@ public:
   // runs the multiscale bootstrap at those scales and fits the AU test per record, and computes the
   // expected likelihood weights (rdk_rell_support_ms; DESIGN.md section 10, items 6-8); the branches
   // then also carry pAU and ELW.
+  // sampling chooses the resampling unit (DESIGN.md section 10, items 11-14): site (the above; each
+  // partition resampled on its own), gene (the partitions themselves, with replacement) or gene_site
+  // (partitions, then the sites of each drawn partition).  The gene modes need at least 2 partitions
+  // and refuse au_scales; they also return each partition's fixed-point log-likelihood per record.
+  enum class support_sampling_t { site, gene, gene_site };
   struct placement_support_t {
     std::vector<size_t>   root_id;
     std::vector<double>   alpha, llh, lnl_fixed, bp, p_kh, p_sh;
@@ -204,10 +209,19 @@ public:
     std::vector<unsigned long long> elw_fixed;
     double                          au_counts_ms = 0, au_accumulate_ms = 0, au_statistics_ms = 0;
     double                          positions_ms = 0;  // branch_support: the alpha searches
+    // gene modes only (empty otherwise): [partition][record] O_i 2^-e and O_i as int128, and the
+    // record of each partition's highest O_i (lowest index on ties)
+    support_sampling_t              sampling = support_sampling_t::site;
+    std::vector<double>             partition_lnl_fixed;
+    std::vector<unsigned long long> partition_o_lo;
+    std::vector<long long>          partition_o_hi;
+    std::vector<unsigned>           partition_best;
+    double                          gene_draws_ms = 0;
   };
   placement_support_t placement_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed,
                                         unsigned replicate_tile = 0, bool keep_rows = false,
-                                        const std::vector<unsigned> &au_scales = {});
+                                        const std::vector<unsigned> &au_scales = {},
+                                        support_sampling_t sampling = support_sampling_t::site);
   // The same statistics for EVERY branch at one set of parameters (DESIGN.md section 10, items 9-10):
   // the parameters of the checkpoint's best record (highest llh, lowest log index on ties) are
   // installed, root q is placed at a_q = optimize_alpha(root q at ratio 0.5, atol) (0.5 everywhere
@@ -219,7 +233,8 @@ public:
   // Refuses what placement_support refuses, and atol < 0.
   placement_support_t branch_support(checkpoint_t &checkpoint, size_t replicates, uint64_t seed, double atol,
                                      unsigned replicate_tile = 0, bool keep_rows = false,
-                                     const std::vector<unsigned> &au_scales = {});
+                                     const std::vector<unsigned> &au_scales = {},
+                                     support_sampling_t sampling = support_sampling_t::site);
   // the unweighted per-pattern log-likelihoods of the last placement_support / branch_support:
   // [record][pattern]
   std::vector<double> site_lnl_rows(size_t partition);
@@ -235,13 +250,15 @@ private:
   std::vector<double> root_lh_on_branch(const root_location_t &root, const std::vector<double> &ratios);
 
   // ---- placement support, the parts placement_support and branch_support share ------------------
-  void check_support_request(const std::string &who, size_t replicates, const std::vector<unsigned> &au_scales) const;
+  void check_support_request(const std::string &who, size_t replicates, const std::vector<unsigned> &au_scales,
+                             support_sampling_t sampling) const;
   void check_support_records(const std::string &who, const std::vector<checkpoint_t::record_t> &records) const;
   void install_record(const checkpoint_t::record_t &record);
   std::function<void()> support_restore_point(bool keep_rows);
   void reserve_support_rows(const std::string &who, unsigned rows);
   void resample_support(const std::string &who, placement_support_t &out, unsigned rows, size_t replicates,
-                        uint64_t seed, unsigned replicate_tile, const std::vector<unsigned> &au_scales);
+                        uint64_t seed, unsigned replicate_tile, const std::vector<unsigned> &au_scales,
+                        support_sampling_t sampling);
   void annotate_support(placement_support_t &out, const std::vector<root_location_t> &where);
   rooted_tree_t::sweep_schedule_t directed_sweep_schedule(size_t begin, size_t end, const std::vector<double> &ratio,
                                                           std::vector<unsigned int> &chunk_off) const;

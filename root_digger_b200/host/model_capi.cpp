@@ -464,13 +464,37 @@ static void copy_support_au(const model_t::placement_support_t &res, unsigned ca
   info[8] = res.au_statistics_ms;
 }
 
-// the body of rdh_model_placement_support and rdh_model_placement_support_au
+// the gene-mode sampling code of the C entries (1: gene, 2: gene_site)
+static model_t::support_sampling_t gene_sampling(unsigned sampling) {
+  if (sampling == 1) return model_t::support_sampling_t::gene;
+  if (sampling == 2) return model_t::support_sampling_t::gene_site;
+  throw std::invalid_argument("unknown sampling mode " + std::to_string(sampling) + " (1: gene, 2: gene_site)");
+}
+
+// the gene-mode outputs ([partition][cap] for the per-record values) and info[k_draws]
+static void copy_support_genes(const model_t::placement_support_t &res, unsigned cap, double *partition_lnl_fixed,
+                               unsigned long long *partition_o_lo, long long *partition_o_hi,
+                               unsigned *partition_best, double *info, unsigned k_draws) {
+  const size_t n = res.root_id.size(), parts = res.partition_best.size();
+  for (size_t p = 0; p < parts; ++p) {
+    for (size_t i = 0; i < n; ++i) {
+      partition_lnl_fixed[p * cap + i] = res.partition_lnl_fixed[p * n + i];
+      if (partition_o_lo) partition_o_lo[p * cap + i] = res.partition_o_lo[p * n + i];
+      if (partition_o_hi) partition_o_hi[p * cap + i] = res.partition_o_hi[p * n + i];
+    }
+    partition_best[p] = res.partition_best[p];
+  }
+  info[k_draws] = res.gene_draws_ms;
+}
+
+// the body of rdh_model_placement_support, rdh_model_placement_support_au and _genes
 static model_t::placement_support_t placement_support_into(
     void *h, const char *checkpoint_prefix, unsigned long long replicates, unsigned long long seed,
     unsigned replicate_tile, int keep_rows, unsigned cap, unsigned long long *root_id, double *alpha, double *llh,
     double *lnl_fixed, unsigned long long *o_lo, long long *o_hi, unsigned *bp_count, unsigned *kh_count,
     unsigned *sh_count, int *exponent, unsigned *best, double *info, unsigned *n_out,
-    const std::vector<unsigned> &au_scales) {
+    const std::vector<unsigned> &au_scales,
+    model_t::support_sampling_t sampling = model_t::support_sampling_t::site) {
   checkpoint_t  external;
   checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
   const size_t  records = ckp.read_results().size();
@@ -478,7 +502,7 @@ static model_t::placement_support_t placement_support_into(
     *n_out = (unsigned)records;
     throw std::runtime_error("output buffers too small: " + std::to_string(records) + " records");
   }
-  auto res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0, au_scales);
+  auto res = H(h).model->placement_support(ckp, replicates, seed, replicate_tile, keep_rows != 0, au_scales, sampling);
   copy_support(res, cap, root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count, exponent, best,
                info, n_out);
   return res;
@@ -535,6 +559,32 @@ extern "C" int rdh_model_placement_support_au(void *h, const char *checkpoint_pr
   })
 }
 
+// rdh_model_placement_support with gene (sampling = 1) or gene-then-site (sampling = 2) resampling of
+// the model's partitions instead of site resampling (model_t::placement_support; DESIGN.md section
+// 10, items 11-14); at least 2 partitions.  Per partition p and record r: partition_lnl_fixed[p * cap
+// + r] = O_p[r] 2^-e, O_p as a two's-complement int128 (partition_o_lo, partition_o_hi; may be NULL),
+// and partition_best[p] = the record of the highest O_p (lowest index on ties); the counts come from
+// the chosen resampling.  info receives the six values of rdh_model_placement_support, then the gene
+// draws' ms.
+extern "C" int rdh_model_placement_support_genes(void *h, const char *checkpoint_prefix, unsigned long long replicates,
+                                                 unsigned long long seed, unsigned replicate_tile, int keep_rows,
+                                                 unsigned sampling, unsigned cap, unsigned long long *root_id,
+                                                 double *alpha, double *llh, double *lnl_fixed,
+                                                 unsigned long long *o_lo, long long *o_hi, unsigned *bp_count,
+                                                 unsigned *kh_count, unsigned *sh_count, double *partition_lnl_fixed,
+                                                 unsigned long long *partition_o_lo, long long *partition_o_hi,
+                                                 unsigned *partition_best, int *exponent, unsigned *best,
+                                                 double *info, unsigned *n_out) {
+  RDH_TRY({
+    const auto mode = gene_sampling(sampling);
+    const auto res = placement_support_into(h, checkpoint_prefix, replicates, seed, replicate_tile, keep_rows, cap,
+                                            root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count,
+                                            exponent, best, info, n_out, {}, mode);
+    copy_support_genes(res, cap, partition_lnl_fixed, partition_o_lo, partition_o_hi, partition_best, info, 6);
+    return 1;
+  })
+}
+
 // The support statistics of EVERY branch at the parameters of the best record of
 // "<checkpoint_prefix>.ckp" (opened read-only; NULL: the model's own result log), with root q at
 // a_q = optimize_alpha(q at 0.5, atol) (atol = 0: 0.5) -- model_t::branch_support, DESIGN.md section 10,
@@ -572,6 +622,37 @@ extern "C" int rdh_model_branch_support(void *h, const char *checkpoint_prefix, 
     info[6] = info[7] = info[8] = 0.0;
     if (n_scales) copy_support_au(res, cap, scale_count, p_au, au_d, au_c, au_rss, au_used, elw, elw_fixed, info);
     info[9] = res.positions_ms;
+    return 1;
+  })
+}
+
+// rdh_model_branch_support with gene (sampling = 1) or gene-then-site (sampling = 2) resampling and the
+// per-partition outputs of rdh_model_placement_support_genes (capacity cap >= the model's root
+// count).  info receives the six values of rdh_model_placement_support, then the gene draws' ms and
+// the alpha searches' ms.
+extern "C" int rdh_model_branch_support_genes(void *h, const char *checkpoint_prefix, unsigned long long replicates,
+                                              unsigned long long seed, double atol, unsigned replicate_tile,
+                                              int keep_rows, unsigned sampling, unsigned cap,
+                                              unsigned long long *root_id, double *alpha, double *llh,
+                                              double *lnl_fixed, unsigned long long *o_lo, long long *o_hi,
+                                              unsigned *bp_count, unsigned *kh_count, unsigned *sh_count,
+                                              double *partition_lnl_fixed, unsigned long long *partition_o_lo,
+                                              long long *partition_o_hi, unsigned *partition_best, int *exponent,
+                                              unsigned *best, double *info, unsigned *n_out) {
+  RDH_TRY({
+    const auto   mode = gene_sampling(sampling);
+    const size_t roots = H(h).model->tree().root_count();
+    if (roots > cap) {
+      *n_out = (unsigned)roots;
+      throw std::runtime_error("output buffers too small: " + std::to_string(roots) + " branches");
+    }
+    checkpoint_t  external;
+    checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
+    const auto    res = H(h).model->branch_support(ckp, replicates, seed, atol, replicate_tile, keep_rows != 0, {}, mode);
+    copy_support(res, cap, root_id, alpha, llh, lnl_fixed, o_lo, o_hi, bp_count, kh_count, sh_count, exponent, best,
+                 info, n_out);
+    copy_support_genes(res, cap, partition_lnl_fixed, partition_o_lo, partition_o_hi, partition_best, info, 6);
+    info[7] = res.positions_ms;
     return 1;
   })
 }

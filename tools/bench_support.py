@@ -20,8 +20,14 @@ position searches), capture_ms (the one placement sweep that stores the rows) an
 phases, and, next to them, the capture_ms of placement_support on the equivalent 2n-3-record
 checkpoint (the record-by-record capture this mode replaces), measured once at the first B.
 
+With --partitions G the sites are split into G equal partitions (each with its own parameters), and
+--sampling gene or gene_site resamples those partitions (DESIGN.md section 10, items 11-14) instead of
+their sites; the line then adds the gene draws' time.  The defaults (one partition, site resampling)
+measure what the script measured before these options existed.
+
     python tools/bench_support.py [--taxa 500] [--sites 100000] [--replicates 1000,10000] [--reps 3]
                                   [--au-scales default] [--branches] [--atol 1e-14]
+                                  [--partitions 1] [--sampling site|gene|gene_site]
 """
 from __future__ import annotations
 
@@ -64,6 +70,8 @@ def main():
     ap.add_argument("--au-scales", default=None, help='comma-separated scales, or "default" (capi.AU_SCALES)')
     ap.add_argument("--branches", action="store_true", help="time branch_support from a one-record checkpoint")
     ap.add_argument("--atol", type=float, default=1e-14, help="--branches: tolerance of the position searches")
+    ap.add_argument("--partitions", type=int, default=1, help="split the sites into this many equal partitions")
+    ap.add_argument("--sampling", default="site", choices=("site", "gene", "gene_site"))
     args = ap.parse_args()
 
     from root_digger_b200 import capi, synth
@@ -74,10 +82,15 @@ def main():
     top = synth.random_tree(args.taxa, args.seed)
     rates, freqs = synth.random_params(args.seed + 1)
     aln = synth.simulate_alignment(top, args.sites, args.seed + 2, rates, freqs, capi.gamma_cats(1.0, args.cats))
-    m = capi.Model(capi.RootedTree(synth.to_newick(top)), aln, rate_cats=args.cats, seed=1)
+    G = args.partitions
+    split = [(i * args.sites // G, (i + 1) * args.sites // G) for i in range(G)] if G > 1 else None
+    m = capi.Model(capi.RootedTree(synth.to_newick(top)), aln, rate_cats=args.cats, seed=1, partitions=split)
     m.initialize_partitions(uniform_freqs=False)
-    R, P = m.root_count, m.sites(0)
+    R, P = m.root_count, sum(m.sites(p) for p in range(G))
     r12, f4, _ = m.get_params()
+    kw = {"au_scales": au}
+    if args.sampling != "site":
+        kw["sampling"] = args.sampling
     rng = np.random.default_rng(args.seed + 3)
     if args.branches:
         return branches(args, m, au, device, r12, f4, rng)
@@ -87,14 +100,16 @@ def main():
         ckp.save_options(prefix=prefix)
         for rid in range(R):
             params = [{"rates": r12, "freqs": f4, "alpha": float(rng.uniform(0.5, 2.0)),
-                       "weights": np.full(args.cats, 1.0 / args.cats)}]
+                       "weights": np.full(args.cats, 1.0 / args.cats)} for _ in range(G)]
             ckp.write(rid, 0.0, float(rng.uniform(0.0, 1.0)), params, K=args.cats)
         ckp.close()
         results = {}
         for B in [int(b) for b in args.replicates.split(",")]:
-            m.placement_support(prefix, replicates=B, seed=1, au_scales=au)  # warm-up: module load, allocations
-            runs = [m.placement_support(prefix, replicates=B, seed=1 + i, au_scales=au) for i in range(args.reps)]
+            m.placement_support(prefix, replicates=B, seed=1, **kw)  # warm-up: module load, allocations
+            runs = [m.placement_support(prefix, replicates=B, seed=1 + i, **kw) for i in range(args.reps)]
             keys = ["capture_ms", "counts_ms", "accumulate_ms", "statistics_ms", "resample_ms"]
+            if args.sampling != "site":
+                keys += ["gene_draws_ms"]
             if au:
                 keys += ["au_counts_ms", "au_accumulate_ms", "au_statistics_ms"]
             med = {k: statistics.median(r[k] for r in runs) for k in keys}
@@ -109,6 +124,8 @@ def main():
             results[str(B)] = med
     line = {"tool": "bench_support", "taxa": args.taxa, "patterns": P, "records": R, "cats": args.cats,
             "reps": args.reps, "card": device, "results": results}
+    if G > 1 or args.sampling != "site":
+        line.update({"partitions": G, "sampling": args.sampling})
     if au:
         line["au_scales"] = list(au)
     print(json.dumps(line))
@@ -116,9 +133,9 @@ def main():
 
 def branches(args, m, au, device, r12, f4, rng):
     from root_digger_b200 import capi
-    R, P = m.root_count, m.sites(0)
+    R, P = m.root_count, sum(m.sites(p) for p in range(args.partitions))
     params = [{"rates": r12, "freqs": f4, "alpha": float(rng.uniform(0.5, 2.0)),
-               "weights": np.full(args.cats, 1.0 / args.cats)}]
+               "weights": np.full(args.cats, 1.0 / args.cats)} for _ in range(args.partitions)]
     results = {}
     with tempfile.TemporaryDirectory() as tmp:
         one = str(Path(tmp) / "search")
@@ -128,6 +145,8 @@ def branches(args, m, au, device, r12, f4, rng):
         ckp.close()
         Bs = [int(b) for b in args.replicates.split(",")]
         kw = dict(atol=args.atol, au_scales=au)
+        if args.sampling != "site":
+            kw["sampling"] = args.sampling
         first = m.branch_support(one, replicates=Bs[0], seed=1, **kw)  # warm-up: module load, allocations
         # the record-by-record capture of the same 2n-3 placements, for comparison
         eq = str(Path(tmp) / "equivalent")
@@ -140,6 +159,8 @@ def branches(args, m, au, device, r12, f4, rng):
         for B in Bs:
             runs = [m.branch_support(one, replicates=B, seed=1 + i, **kw) for i in range(args.reps)]
             keys = ["positions_ms", "capture_ms", "counts_ms", "accumulate_ms", "statistics_ms", "resample_ms"]
+            if args.sampling != "site":
+                keys += ["gene_draws_ms"]
             if au:
                 keys += ["au_counts_ms", "au_accumulate_ms", "au_statistics_ms"]
             med = {k: statistics.median(r[k] for r in runs) for k in keys}
