@@ -490,6 +490,32 @@ int rdk_rell_support_genes(rdk_partition_t *const *partitions, unsigned int n,
                            unsigned long long replicates, unsigned long long seed, rdk_rell_out_t *out,
                            rdk_rell_gene_out_t *genes);
 
+/* ---- marginal ancestral states (new; DESIGN.md section 11) ----------------- */
+/* The posterior of every internal node of the rooted tree whose post-order operations are
+ * ops[0..count) -- those of the last full traversal: node i is ops[i].parent_clv_index, the root is
+ * the parent of ops[count - 1], whose state has the prior pi.  One pre-order pass over outside vectors
+ * (smaller subtree first: at most ceil(log2 count) + 2 CLV-sized scratch buffers) from the stored child
+ * CLVs, their scalers and the P-matrices of the operations; recorded P-matrix updates are run and a
+ * kept lazy program is materialised first.  The patterns are walked in tiles, so the device holds the
+ * outputs and scratch of one tile at a time.  full_ops must not repeat an operation.  On a site shard the outputs hold the local patterns.
+ * Arrays are caller-owned; patterns = the partition's `sites`. */
+typedef struct rdk_ancestral_out_t {
+  const unsigned int *full_ops;     /* in: positions i of the nodes whose full posterior is wanted */
+  unsigned int        n_full;       /* in */
+  unsigned int        threads;      /* in: threads per block, a multiple of 32 up to 256 (0: 256) */
+  unsigned int        tile_sites;   /* in: patterns per pass (0: as many as keep the outputs and scratch of a
+                                       pass within 512 MiB); out: the tile used */
+  unsigned char      *map_state;    /* out: [count][patterns], argmax of the posterior, lowest state on ties */
+  double             *map_prob;     /* out: [count][patterns], its posterior */
+  double             *posterior;    /* out: [n_full][patterns][4] */
+  double             *log_norm;     /* out (optional): [count][patterns], log of the normaliser + scalers */
+  double              ms;           /* out: device time of the pass */
+  unsigned long long  device_bytes; /* out: device memory the call allocated (freed on return) */
+  unsigned int        scratch;      /* out: outside-vector buffers the pass used */
+} rdk_ancestral_out_t;
+int rdk_marginal_ancestral_states(rdk_partition_t *partition, const rdk_operation_t *ops, unsigned int count,
+                                  const unsigned int *freqs_indices, rdk_ancestral_out_t *out);
+
 #ifdef __cplusplus
 }
 #endif

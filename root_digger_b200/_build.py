@@ -67,8 +67,9 @@ def build_engine(force: bool = False, verbose: bool = False) -> Path:
     LIBDIR.mkdir(exist_ok=True)
     out = LIBDIR / "librdk_b200.so"
     srcs = [CSRC / "rdk_abi.cu", CSRC / "rdk_host_math.cpp", CSRC / "rdk_lower_debug.cpp", CSRC / "rdk_program_inst.cu",
-            CSRC / "rdk_support.cu"]
-    deps = srcs + [CSRC / "rdk_kernels.cuh", CSRC / "rdk_lower.hpp", CSRC / "rdk_support.cuh", INCLUDE / "rdk.h"]
+            CSRC / "rdk_support.cu", CSRC / "rdk_ancestral.cu"]
+    deps = srcs + [CSRC / "rdk_kernels.cuh", CSRC / "rdk_lower.hpp", CSRC / "rdk_support.cuh", CSRC / "rdk_ancestral.cuh",
+                   INCLUDE / "rdk.h"]
     if not force and _newer(out, deps):
         return out
     objdir = LIBDIR / "obj_librdk_b200"
@@ -80,7 +81,8 @@ def build_engine(force: bool = False, verbose: bool = False) -> Path:
     jobs = [(base + ["-c", CSRC / "rdk_abi.cu", "-o", objdir / "rdk_abi.o"]),
             (base + ["-c", CSRC / "rdk_host_math.cpp", "-o", objdir / "rdk_host_math.o"]),
             (base + ["-c", CSRC / "rdk_lower_debug.cpp", "-o", objdir / "rdk_lower_debug.o"]),
-            (base + ["-c", CSRC / "rdk_support.cu", "-o", objdir / "rdk_support.o"])]
+            (base + ["-c", CSRC / "rdk_support.cu", "-o", objdir / "rdk_support.o"]),
+            (base + ["-c", CSRC / "rdk_ancestral.cu", "-o", objdir / "rdk_ancestral.o"])]
     for k in PROGRAM_KS:
         jobs.append(base + ["-DRDK_INST_K=%d" % k, "-c", CSRC / "rdk_program_inst.cu", "-o", objdir / ("rdk_program_k%d.o" % k)])
     with ThreadPoolExecutor(max_workers=max(1, min(len(jobs), os.cpu_count() or 1))) as pool:

@@ -85,6 +85,13 @@ class Stats(C.Structure):
         return {n: int(getattr(self, n)) for n, _ in self._fields_}
 
 
+class AncestralOut(C.Structure):  # rdk_ancestral_out_t
+    _fields_ = [("full_ops", C.POINTER(C.c_uint)), ("n_full", C.c_uint), ("threads", C.c_uint),
+                ("tile_sites", C.c_uint), ("map_state", C.POINTER(C.c_ubyte)), ("map_prob", C.POINTER(C.c_double)),
+                ("posterior", C.POINTER(C.c_double)), ("log_norm", C.POINTER(C.c_double)), ("ms", C.c_double),
+                ("device_bytes", C.c_ulonglong), ("scratch", C.c_uint)]
+
+
 _dp = C.POINTER(C.c_double)
 _up = C.POINTER(C.c_uint)
 _pp = C.POINTER(PartitionStruct)
@@ -179,6 +186,7 @@ def load_engine() -> C.CDLL:
     L.rdk_compute_root_loglikelihood_row.restype = C.c_double
     L.rdk_partition_get_site_lnl_rows.argtypes = [_pp, C.c_uint, C.c_uint, _dp]
     L.rdk_partition_permute_site_lnl_rows.argtypes = [_pp, C.c_uint, _up]
+    L.rdk_marginal_ancestral_states.argtypes = [_pp, C.POINTER(Operation), C.c_uint, _up, C.POINTER(AncestralOut)]
     _engine_lib = L
     return L
 
@@ -316,6 +324,22 @@ class Partition:
         o = np.ascontiguousarray(order, dtype=np.uint32)
         if self.L.rdk_partition_permute_site_lnl_rows(self.p, len(o), _ptr(o, _up)) != 1:
             raise EngineError(_err(self.L))
+
+    def marginal_ancestral_states(self, ops, full_ops=(), threads: int = 0, tile_sites: int = 0) -> dict:
+        """rdk_marginal_ancestral_states over the post-order operations `ops` of the last full traversal:
+        map_state (0..3) and map_prob, log_norm [op][pattern], posterior [len(full_ops)][pattern][4], and
+        ms, device_bytes, scratch, tile_sites"""
+        arr = ops if isinstance(ops, C.Array) else ops_array(ops)
+        n, S = len(ops), self.sites
+        full = np.ascontiguousarray(list(full_ops), dtype=np.uint32)
+        ms_, mp, ln = np.zeros((n, S), dtype=np.uint8), np.zeros((n, S)), np.zeros((n, S))
+        post = np.zeros((max(1, len(full)), S, 4))
+        out = AncestralOut(_ptr(full, _up) if len(full) else None, len(full), threads, tile_sites,
+                           _ptr(ms_, C.POINTER(C.c_ubyte)), _ptr(mp, _dp), _ptr(post, _dp), _ptr(ln, _dp))
+        if not self.L.rdk_marginal_ancestral_states(self.p, arr, n, self._zeros, C.byref(out)):
+            raise EngineError(_err(self.L))
+        return {"map_state": ms_, "map_prob": mp, "log_norm": ln, "posterior": post[:len(full)], "ms": out.ms,
+                "device_bytes": int(out.device_bytes), "scratch": int(out.scratch), "tile_sites": int(out.tile_sites)}
 
     def root_loglikelihood_multi(self, root_op, branch_length_pairs):
         bl = np.ascontiguousarray(branch_length_pairs, dtype=np.float64).reshape(-1)
@@ -843,6 +867,14 @@ def _bind_model(L: C.CDLL):
     L.rdh_model_site_lnl_rows.argtypes = [vp, C.c_uint, _dp, ull, _up, C.c_uint, C.POINTER(ull)]
     L.rdh_model_assign_indicies.argtypes = [vp, C.c_int, C.c_uint, C.c_double, C.c_uint, C.c_uint, C.c_int, _up,
                                             C.c_uint, _up]
+    L.rdh_model_ancestral_states.argtypes = [vp, C.c_uint, C.c_double, C.c_char_p, C.c_int, C.c_uint, _up, C.c_uint,
+                                             C.c_uint, _up, _up]
+    L.rdh_model_ancestral_nodes.argtypes = [vp, C.c_uint, C.c_uint, _up, C.POINTER(C.c_int), _up, C.POINTER(ull), _dp,
+                                            C.POINTER(C.c_int)]
+    L.rdh_model_ancestral_clade.argtypes = [vp, C.c_uint]
+    L.rdh_model_ancestral_clade.restype = vp
+    L.rdh_model_ancestral_partition.argtypes = [vp, C.c_uint, ull, ull, C.POINTER(C.c_ubyte), _dp, _dp, _dp, _dp]
+    L.rdh_model_pattern_of_column.argtypes = [vp, C.c_uint, _up, C.c_uint, _up]
     L._rdh_model_bound = True
 
 
@@ -1018,6 +1050,37 @@ def msa_partition_lengths(msa_path: str, partition_text: str, compress_first: bo
     if not rc:
         raise ValueError(L.rdh_last_error().decode())
     return [int(out[i]) for i in range(rc - 1)]
+
+
+def write_state_file(result: dict, path, fasta_path=None) -> None:
+    """Write the result of Model.ancestral_states as IQ-TREE's .state table, one line per node with a
+    full posterior (in the order of result["full"]) and alignment column: the node ("Node<CLV index>"),
+    the site, the MAP state and the posterior of A, C, G, T (5 decimals).  With one partition the header
+    is "Node Site State p_A p_C p_G p_T" and Site is the alignment column, from 1.  With several
+    partitions a "Part" column (the partition, from 1) follows Node, as in IQ-TREE's partitioned output,
+    and Site counts from 1 within the partition, over its columns in the order of its ranges (a
+    partition "1-100, 301-400" has sites 1-200; site 101 is alignment column 301).  Fields are
+    tab-separated.  Also writes the root's MAP sequence as FASTA (">root", 60 columns per line, the
+    partitions' columns in the same order) to fasta_path (default: path with the suffix .fasta)."""
+    path = Path(path)
+    nodes, full = result["nodes"], result["full"]
+    parts = result["pattern_of_column"]
+    several = len(parts) > 1
+    lines = ["Node\tPart\tSite\tState\tp_A\tp_C\tp_G\tp_T" if several else "Node\tSite\tState\tp_A\tp_C\tp_G\tp_T"]
+    for f, node in enumerate(full.tolist()):
+        name = "Node%d" % nodes[node]
+        for part, cols in enumerate(parts):
+            post = result["posterior"][part][f]
+            state = result["map_state"][part][node]
+            lead = "%s\t%d\t" % (name, part + 1) if several else name + "\t"
+            for site, p in enumerate(cols.tolist(), start=1):
+                q = post[p]
+                lines.append("%s%d\t%s\t%.5f\t%.5f\t%.5f\t%.5f" % (lead, site, chr(state[p]), q[0], q[1], q[2], q[3]))
+    root = len(nodes) - 1
+    seq = "".join(bytes(result["map_state"][part][root][cols]).decode() for part, cols in enumerate(parts))
+    path.write_text("\n".join(lines) + "\n")
+    fasta = Path(fasta_path) if fasta_path is not None else path.with_suffix(".fasta")
+    fasta.write_text(">root\n" + "".join(seq[i:i + 60] + "\n" for i in range(0, len(seq), 60)))
 
 
 class Model:
@@ -1478,6 +1541,90 @@ class Model:
         llh = np.ascontiguousarray(llh, dtype=np.float64)
         out = np.zeros(len(llh))
         self.L.rdh_model_lwr(_ptr(llh, _dp), len(llh), _ptr(out, _dp))
+        return out
+
+    def pattern_of_column(self, part: int = 0) -> np.ndarray:
+        """the pattern every column of partition `part` was compressed into (a partition's columns in
+        the order of its ranges)"""
+        n = C.c_uint()
+        self.L.rdh_model_pattern_of_column(self.h, part, None, 0, C.byref(n))
+        out = np.zeros(max(1, n.value), dtype=np.uint32)
+        self._check(self.L.rdh_model_pattern_of_column(self.h, part, _ptr(out, _up), n.value, C.byref(n)))
+        return out[:n.value].copy()
+
+    def ancestral_states(self, root_id: int | None = None, ratio: float | None = None,
+                         checkpoint_prefix: str | None = None, full_nodes="root", threads: int = 0,
+                         tile_sites: int = 0) -> dict:
+        """Marginal ancestral states of the rooted tree (DESIGN.md section 11): the posterior of every
+        internal node's state, with the root's prior pi, at the model's parameters and root position.
+
+        root_id / ratio: the placement (ratio 0.5 if not given).  checkpoint_prefix: instead, the
+        parameters and placement of the best record of "<checkpoint_prefix>.ckp" (highest llh, lowest
+        log index on ties).  Parameters and rooting are left as they were.  full_nodes: "root", "all" or
+        distinct CLV indices of the nodes whose full posterior is returned.  threads / tile_sites: the
+        engine's launch shape (threads per block, patterns per pass; 0 = its default), which does not
+        change any result.  Keys: nodes (CLV indices in post-order, the root last), parent (position of
+        the parent node, -1 at the root), clade (sorted tip labels below each node), full (positions of
+        the nodes in `posterior`), ops (each node's post-order operation, the 8 fields of
+        rdk_operation_t), root_id, ratio, and per partition (lists): map_state (bytes of ACGT,
+        [node][pattern]), map_prob, posterior ([full node][pattern][4]), log_norm, pattern_of_column,
+        ms (device time of the pass), device_bytes, tile_sites."""
+        if checkpoint_prefix is not None and (root_id is not None or ratio is not None):
+            raise ValueError("ancestral_states: give a placement or a checkpoint, not both")
+        if checkpoint_prefix is None and root_id is None:
+            raise ValueError("ancestral_states: give root_id (and ratio) or checkpoint_prefix")
+        full = np.zeros(1, dtype=np.uint32)
+        if isinstance(full_nodes, str):
+            if full_nodes not in ("root", "all"):
+                raise ValueError("ancestral_states: full_nodes is 'root', 'all' or a list of CLV indices")
+            nf = 0 if full_nodes == "root" else 0xFFFFFFFF
+        else:
+            full = np.ascontiguousarray(list(full_nodes), dtype=np.uint32)
+            nf = len(full)
+        n_nodes, n_full = C.c_uint(), C.c_uint()
+        self._check(self.L.rdh_model_ancestral_states(
+            self.h, int(root_id or 0), float(0.5 if ratio is None else ratio),
+            checkpoint_prefix.encode() if checkpoint_prefix is not None else None,
+            1 if checkpoint_prefix is not None else 0, nf, _ptr(full, _up) if len(full) else None, int(threads),
+            int(tile_sites), C.byref(n_nodes), C.byref(n_full)))
+        n, nf = n_nodes.value, n_full.value
+        nodes = np.zeros(n, dtype=np.uint32)
+        parent = np.zeros(n, dtype=np.int32)
+        pos = np.zeros(max(1, nf), dtype=np.uint32)
+        ops = np.zeros((n, 8), dtype=np.int32)
+        rid, rr = C.c_ulonglong(), C.c_double()
+        self._check(self.L.rdh_model_ancestral_nodes(self.h, n, nf, _ptr(nodes, _up), _ptr(parent, C.POINTER(C.c_int)),
+                                                     _ptr(pos, _up), C.byref(rid), C.byref(rr),
+                                                     _ptr(ops, C.POINTER(C.c_int))))
+        clade = []
+        for i in range(n):
+            p = self.L.rdh_model_ancestral_clade(self.h, i)
+            if not p:
+                raise RuntimeError(self.L.rdh_last_error().decode())
+            text = C.string_at(p).decode()
+            self.L.rdh_free(p)
+            clade.append(text.split("\n") if text else [])
+        out = {"nodes": nodes, "parent": parent, "clade": clade, "full": pos[:nf].copy(), "ops": ops,
+               "root_id": int(rid.value), "ratio": float(rr.value), "map_state": [], "map_prob": [], "posterior": [],
+               "log_norm": [], "pattern_of_column": [], "ms": [], "device_bytes": [], "tile_sites": []}
+        acgt = np.frombuffer(b"ACGT", dtype=np.uint8)
+        for part in range(self.partition_count):
+            P = self.sites(part)
+            ms_ = np.zeros((n, P), dtype=np.uint8)
+            mp, ln = np.zeros((n, P)), np.zeros((n, P))
+            post = np.zeros((nf, P, 4))
+            info = np.zeros(4)
+            self._check(self.L.rdh_model_ancestral_partition(
+                self.h, part, n * P, nf * P * 4, _ptr(ms_, C.POINTER(C.c_ubyte)), _ptr(mp, _dp),
+                _ptr(post, _dp) if post.size else None, _ptr(ln, _dp), _ptr(info, _dp)))
+            out["map_state"].append(acgt[ms_])
+            out["map_prob"].append(mp)
+            out["posterior"].append(post)
+            out["log_norm"].append(ln)
+            out["pattern_of_column"].append(self.pattern_of_column(part))
+            out["ms"].append(float(info[0]))
+            out["device_bytes"].append(int(info[1]))
+            out["tile_sites"].append(int(info[3]))
         return out
 
     def newick(self, annotations: bool = True) -> str:

@@ -10,6 +10,7 @@
 #include "../../include/rdk.h"
 #include "rdk_kernels.cuh"
 #include "rdk_support.cuh"
+#include "rdk_ancestral.cuh"
 
 #include <dlfcn.h>
 
@@ -1617,6 +1618,97 @@ extern "C" int rdk_rell_support_genes(rdk_partition_t *const *parts, unsigned in
 // ---------------------------------------------------------------------------
 // fused extensions
 // ---------------------------------------------------------------------------
+// ---------------------------------------------------------------------------
+// marginal ancestral states (rdk_ancestral.cu; DESIGN.md section 11)
+// ---------------------------------------------------------------------------
+extern "C" int rdk_marginal_ancestral_states(rdk_partition_t *p, const rdk_operation_t *ops, unsigned int count,
+                                             const unsigned int *freqs_indices, rdk_ancestral_out_t *out) {
+  (void)freqs_indices;
+  if (!p || !ops || !out) return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: null argument");
+  if (!out->map_state || !out->map_prob || (out->n_full && (!out->full_ops || !out->posterior)))
+    return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: missing output arrays");
+  Engine *e = eng(p);
+  char    msg[256];
+  std::vector<AncNode> nodes;
+  unsigned             scratch = 0;
+  if (!ancestral_schedule(ops, count, e->tips, e->tips + e->clv_buffers, nodes, scratch, msg, sizeof(msg)))
+    return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: %s", msg);
+  std::vector<int> full_row(count, -1);
+  for (unsigned f = 0; f < out->n_full; ++f) {
+    if (out->full_ops[f] >= count)
+      return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: full posterior for operation %u of %u",
+                  out->full_ops[f], count);
+    if (full_row[out->full_ops[f]] >= 0)
+      return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: operation %u is listed twice in full_ops",
+                  out->full_ops[f]);
+    full_row[out->full_ops[f]] = (int)f;
+  }
+  for (unsigned i = 0; i < count; ++i) {
+    const rdk_operation_t &op = ops[i];
+    if (op.child1_matrix_index >= e->prob_matrices || op.child2_matrix_index >= e->prob_matrices)
+      return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: operation %u: matrix index out of range", i);
+    const int sc[3] = {op.parent_scaler_index, op.child1_scaler_index, op.child2_scaler_index};
+    for (int s : sc)
+      if (s != RDK_SCALE_BUFFER_NONE && (s < 0 || (unsigned)s >= e->scale_buffers))
+        return fail(RDK_ERROR_PARAM, "rdk_marginal_ancestral_states: operation %u: scaler index out of range", i);
+  }
+  std::lock_guard<std::mutex> lk(e->mu);
+  CUDA_TRY(cudaSetDevice(e->device));
+  if (!flush(p)) return RDK_FAILURE;
+  if (e->lazy.active) {  // the pass reads the children's CLVs and scalers from memory
+    bool stale = false;
+    for (unsigned i = 0; i < count && !stale; ++i) {
+      const rdk_operation_t &op = ops[i];
+      for (unsigned c : {op.child1_clv_index, op.child2_clv_index})
+        stale |= c < e->lazy.stale_clv.size() && e->lazy.stale_clv[c];
+      for (int s : {op.child1_scaler_index, op.child2_scaler_index})
+        stale |= s >= 0 && (size_t)s < e->lazy.stale_sc.size() && e->lazy.stale_sc[s];
+    }
+    if (stale && !materialize_lazy(p)) return RDK_FAILURE;
+  }
+  for (AncNode &nd : nodes) {
+    const rdk_operation_t &op = ops[nd.op];
+    nd.full = full_row[nd.op];
+    nd.scaled = op.parent_scaler_index != RDK_SCALE_BUFFER_NONE;
+    const unsigned          child[2] = {op.child1_clv_index, op.child2_clv_index};
+    const unsigned          mat[2] = {op.child1_matrix_index, op.child2_matrix_index};
+    const int               scl[2] = {op.child1_scaler_index, op.child2_scaler_index};
+    const double          **tab[2] = {&nd.tab1, &nd.tab2};
+    const void            **clv[2] = {&nd.c1, &nd.c2};
+    const unsigned int    **scp[2] = {&nd.sc1, &nd.sc2};
+    int                    *tip[2] = {&nd.tip1, &nd.tip2};
+    for (int s = 0; s < 2; ++s) {
+      *tab[s] = e->d_pool + (size_t)e->pm_map[mat[s]] * e->K * kSlotDoubles;
+      *tip[s] = child[s] < e->tips;
+      if (child[s] < e->tips) {
+        *clv[s] = e->d_tips + (size_t)child[s] * e->tip_stride;
+      } else {
+        if (!ensure_clv(e, child[s] - e->tips)) return RDK_FAILURE;
+        *clv[s] = e->clv_ptr[child[s] - e->tips];
+      }
+      *scp[s] = nullptr;
+      if (scl[s] != RDK_SCALE_BUFFER_NONE) {
+        if (!ensure_scaler(e, scl[s])) return RDK_FAILURE;
+        *scp[s] = e->sc_ptr[scl[s]];
+      }
+    }
+  }
+  AncPass pass;
+  pass.S = e->S;
+  pass.K = e->K;
+  for (int i = 0; i < 4; ++i) pass.pi[i] = p->frequencies[0][i];
+  for (unsigned k = 0; k < e->K; ++k) pass.w[k] = k < e->Kreal ? p->rate_weights[k] : 0.0;
+  pass.scratch = scratch;
+  pass.count = count;
+  pass.stream = e->stream;
+  if (!ancestral_pass(pass, nodes, out, msg, sizeof(msg)))
+    return fail(RDK_ERROR_CUDA, "rdk_marginal_ancestral_states: %s", msg);
+  e->stats.kernel_launches++;
+  e->stats.d2h_bytes += (unsigned long long)count * e->S * (out->log_norm ? 17 : 9) +
+                        32ull * out->n_full * e->S;
+  return RDK_SUCCESS;
+}
+
 extern "C" int rdk_root_loglikelihood_multi(rdk_partition_t *p, const rdk_operation_t *root_op,
                                             const unsigned int *params_indices,
                                             const unsigned int *freqs_indices,

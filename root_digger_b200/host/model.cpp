@@ -24,6 +24,7 @@
 #include "rdk_support_au.h"  // ... and rdk_rell_support_ms
 #include "rdk_support_genes.h"  // ... and rdk_rell_support_genes
 #include "rdk_sweep_rows.h"   // ... and the row capture of the placement sweep
+#include "rdk_ancestral.h"    // ... and the marginal ancestral states
 #endif
 #include "support_stats.hpp"
 
@@ -101,6 +102,7 @@ model_t::model_t(rooted_tree_t tree, const std::vector<msa_t> &msas,
 
   for (size_t pi = 0; pi < msas.size(); ++pi) {
     auto &msa = msas[pi];
+    _pattern_of_column.push_back(msa.pattern_of_column());
     if (msa.length() > static_cast<size_t>(std::numeric_limits<int>::max()))
       throw std::runtime_error("The length of the MSA is too large to safely cast");
     // the ARCH_* attributes of the reference select coraxlib CPU kernels; the
@@ -1302,6 +1304,132 @@ model_t::placement_support_t model_t::branch_support(checkpoint_t &checkpoint, s
     _tree.annotate_lh(where[q], llh[q]);
     _tree.annotate_ratio(where[q], alpha[q]);
   }
+  return out;
+}
+
+// ---------------------------------------------------------------------------
+// marginal ancestral states (DESIGN.md section 11)
+// ---------------------------------------------------------------------------
+// at the installed parameters: root the tree at `root`, one full traversal, then the pre-order pass
+// of every partition over the CLVs it left
+model_t::ancestral_states_t model_t::ancestral_states_here(const std::string &who, const root_location_t &root,
+                                                           const ancestral_options_t &opts) {
+  for (size_t q = 0; !_tree.can_root_by(root) && q < _tree.root_count(); ++q)  // an unrooted tree: root it elsewhere first
+    if (_tree.can_root_by(_tree.root_location(q))) _tree.root_by(_tree.root_location(q));
+  const traversal_t trav = full_traversal(root);
+  for (size_t p = 0; p < _partitions.size(); ++p) {
+    update_pmatrix_partition(p, trav.pmatrix_indices, trav.branch_lengths);
+    rdk_update_clvs(_partitions[p], trav.ops.data(), (unsigned)trav.ops.size());
+  }
+  const size_t       n = trav.ops.size();
+  ancestral_states_t out;
+  out.root_id = root.id;
+  out.ratio = root.brlen_ratio;
+  out.ops = trav.ops;
+  // the nodes, their parents and clades, from the operations alone
+  std::unordered_map<unsigned, size_t> pos;
+  for (size_t i = 0; i < n; ++i) pos[trav.ops[i].parent_clv_index] = i;
+  std::vector<std::string> tip_label(_tree.tip_count());
+  for (const auto &kv : _tree.label_map()) tip_label.at(kv.second) = kv.first;
+  out.clv_index.resize(n);
+  out.parent.assign(n, -1);
+  out.clade.resize(n);
+  for (size_t i = 0; i < n; ++i) {
+    const rdk_operation_t &op = trav.ops[i];
+    out.clv_index[i] = op.parent_clv_index;
+    for (unsigned c : {op.child1_clv_index, op.child2_clv_index}) {
+      if (c < _tree.tip_count()) {
+        out.clade[i].push_back(tip_label[c]);
+      } else {
+        const size_t j = pos.at(c);
+        out.parent[j] = (int)i;
+        out.clade[i].insert(out.clade[i].end(), out.clade[j].begin(), out.clade[j].end());
+      }
+    }
+  }
+  for (auto &c : out.clade) std::sort(c.begin(), c.end());
+  if (opts.all_full) {
+    for (size_t i = 0; i < n; ++i) out.full.push_back((unsigned)i);
+  } else if (opts.full_nodes.empty()) {
+    out.full.push_back((unsigned)(n - 1));
+  } else {
+    std::vector<char> listed(n, 0);
+    for (unsigned v : opts.full_nodes) {
+      auto it = pos.find(v);
+      if (it == pos.end())
+        throw std::invalid_argument(who + ": node " + std::to_string(v) + " is not an internal node of the rooted tree");
+      if (listed[it->second]++) throw std::invalid_argument(who + ": node " + std::to_string(v) + " is listed twice");
+      out.full.push_back((unsigned)it->second);
+    }
+  }
+  for (size_t p = 0; p < _partitions.size(); ++p) {
+    ancestral_states_t::partition_t part;
+    const size_t                    S = _partitions[p]->sites;
+    part.patterns = (unsigned)S;
+    part.map_state.resize(n * S);
+    part.map_prob.resize(n * S);
+    part.log_norm.resize(n * S);
+    part.posterior.resize(out.full.size() * S * 4);
+    part.pattern_of_column = _pattern_of_column[p];
+    rdk_ancestral_out_t res;
+    std::memset(&res, 0, sizeof(res));
+    res.full_ops = out.full.data();
+    res.n_full = (unsigned)out.full.size();
+    res.map_state = part.map_state.data();
+    res.map_prob = part.map_prob.data();
+    res.posterior = part.posterior.data();
+    res.log_norm = part.log_norm.data();
+    res.threads = opts.threads;
+    res.tile_sites = opts.tile_sites;
+    if (rdk_marginal_ancestral_states(_partitions[p], trav.ops.data(), (unsigned)n, _param_indicies[p].data(), &res) !=
+        RDK_SUCCESS)
+      throw std::runtime_error(who + ": " + engine_error());
+    part.ms = res.ms;
+    part.device_bytes = res.device_bytes;
+    part.scratch = res.scratch;
+    part.tile_sites = res.tile_sites;
+    out.partitions.push_back(std::move(part));
+  }
+  return out;
+}
+
+model_t::ancestral_states_t model_t::ancestral_states(const root_location_t &root, const ancestral_options_t &opts) {
+  const std::string who = "ancestral_states";
+  if (_exchange)
+    throw std::invalid_argument(who + ": a model whose partitions are dealt to several processes is not supported");
+  if (!(root.brlen_ratio >= 0.0 && root.brlen_ratio <= 1.0))
+    throw std::invalid_argument(who + ": root position outside [0, 1]");
+  auto               restore = support_restore_point(true);
+  ancestral_states_t out;
+  try {
+    out = ancestral_states_here(who, root, opts);
+  } catch (...) {
+    restore();
+    throw;
+  }
+  restore();
+  return out;
+}
+
+model_t::ancestral_states_t model_t::ancestral_states(checkpoint_t &checkpoint, const ancestral_options_t &opts) {
+  const std::string who = "ancestral_states";
+  if (_exchange)
+    throw std::invalid_argument(who + ": a model whose partitions are dealt to several processes is not supported");
+  const auto records = checkpoint.read_results();
+  check_support_records(who, records);
+  size_t best = 0;  // highest llh, lowest log index on ties, as branch_support picks it
+  for (size_t r = 1; r < records.size(); ++r)
+    if (records[r].first.llh > records[best].first.llh) best = r;
+  auto               restore = support_restore_point(true);
+  ancestral_states_t out;
+  try {
+    install_record(records[best]);
+    out = ancestral_states_here(who, placement_of(records[best].first).first, opts);
+  } catch (...) {
+    restore();
+    throw;
+  }
+  restore();
   return out;
 }
 

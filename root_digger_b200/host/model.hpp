@@ -239,6 +239,44 @@ public:
   // [record][pattern]
   std::vector<double> site_lnl_rows(size_t partition);
 
+  // ---- marginal ancestral states (DESIGN.md section 11) ------------------------------------------
+  // The posterior of every internal node of the tree rooted at `root` (its ratio included), at the
+  // current parameters: one full traversal, then rdk_marginal_ancestral_states per partition.  Nodes
+  // are the parents of the traversal's operations, in post-order (the root last).  The checkpoint form
+  // installs the parameters and placement of the best record (highest llh, lowest log index on ties).
+  // Both leave the parameters and the rooting as they found them.  Refuses models dealt to several
+  // processes, a ratio outside [0, 1], and full_nodes that are not internal nodes of the rooted tree
+  // or name a node twice.
+  struct ancestral_options_t {
+    std::vector<unsigned> full_nodes;      // CLV indices of the nodes whose full posterior is returned
+    bool                  all_full = false;  // ... or every node; neither: the root
+    unsigned              threads = 0;     // engine launch shape (rdk_ancestral_out_t): 0 = default
+    unsigned              tile_sites = 0;
+  };
+  struct ancestral_states_t {
+    struct partition_t {
+      unsigned                   patterns = 0;
+      std::vector<unsigned char> map_state;                  // [node][pattern], 0..3 = A, C, G, T
+      std::vector<double>        map_prob, log_norm;         // [node][pattern]
+      std::vector<double>        posterior;                  // [full node][pattern][4]
+      std::vector<unsigned>      pattern_of_column;          // [column] -> pattern
+      double                     ms = 0;                     // device time of the pass
+      unsigned long long         device_bytes = 0;
+      unsigned                   scratch = 0, tile_sites = 0;
+    };
+    std::vector<unsigned>                 clv_index;  // [node]
+    std::vector<int>                      parent;     // [node]: position of the parent node, -1 for the root
+    std::vector<std::vector<std::string>> clade;      // [node]: sorted tip labels below it
+    std::vector<unsigned>                 full;       // positions of the nodes with full posteriors
+    std::vector<rdk_operation_t>          ops;        // [node]: the post-order operation that computes it
+    size_t                                root_id = 0;
+    double                                ratio = 0.5;
+    std::vector<partition_t>              partitions;
+  };
+  ancestral_states_t ancestral_states(const root_location_t &root, const ancestral_options_t &opts);
+  ancestral_states_t ancestral_states(checkpoint_t &checkpoint, const ancestral_options_t &opts);
+  const std::vector<unsigned> &pattern_of_column(size_t partition) const { return _pattern_of_column.at(partition); }
+
   rdk_partition_t *partition(size_t i) { return _partitions[i]; }
   size_t           partition_count() const { return _partitions.size(); }
 
@@ -262,6 +300,9 @@ private:
   void annotate_support(placement_support_t &out, const std::vector<root_location_t> &where);
   rooted_tree_t::sweep_schedule_t directed_sweep_schedule(size_t begin, size_t end, const std::vector<double> &ratio,
                                                           std::vector<unsigned int> &chunk_off) const;
+
+  ancestral_states_t ancestral_states_here(const std::string &who, const root_location_t &root,
+                                           const ancestral_options_t &opts);
 
   // ---- parameter plumbing ----------------------------------------------------------------------
   void set_subst_rates_random(size_t, const msa_t &);
@@ -325,6 +366,7 @@ private:
   partition_exchange_fn                  _exchange = nullptr;     // see set_partition_exchange
   void                                  *_exchange_user = nullptr;
   unsigned                               _support_rows = 0;       // rows of the last placement_support
+  std::vector<std::vector<unsigned>>     _pattern_of_column;     // per partition: [column] -> pattern
   std::vector<size_t>                    _global_index;           // global id of each local partition
   size_t                                 _global_partitions = 0;
   static constexpr unsigned int          _submodels = 1;

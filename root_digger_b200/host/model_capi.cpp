@@ -4,6 +4,7 @@
 #include "model.hpp"
 #include "support_stats.hpp"
 
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -18,6 +19,7 @@ struct holder_t {
   std::vector<msa_t>       msa;
   std::unique_ptr<model_t> model;
   checkpoint_t             checkpoint;
+  model_t::ancestral_states_t ancestral;  // the last rdh_model_ancestral_states
 };
 holder_t &H(void *h) { return *reinterpret_cast<holder_t *>(h); }
 }  // namespace
@@ -691,6 +693,127 @@ extern "C" int rdh_model_site_lnl_rows(void *h, unsigned part, double *out, unsi
     std::memcpy(out, rows.data(), sizeof(double) * rows.size());
     std::memcpy(weights, msa.weights(), sizeof(unsigned) * msa.length());
     *n_out = rows.size();
+    return 1;
+  })
+}
+
+// Marginal ancestral states (model_t::ancestral_states, DESIGN.md section 11) of the tree rooted at
+// (root_id, ratio) at the current parameters, or, with from_checkpoint, at the parameters and placement
+// of the best record of "<checkpoint_prefix>.ckp" (NULL: the model's own result log).  full_nodes:
+// CLV indices of the nodes whose full posterior is wanted; n_full = 0: the root, n_full = 0xffffffff
+// (full_nodes ignored): every node.  threads / tile_sites: the engine's launch
+// shape (rdk_ancestral_out_t; 0 = its default).  The result is kept until the next call; n_nodes /
+// n_full_out receive its sizes, rdh_model_ancestral_* read it.
+static const unsigned kAncestralAllNodes = 0xffffffffu;
+extern "C" int rdh_model_ancestral_states(void *h, unsigned root_id, double ratio, const char *checkpoint_prefix,
+                                          int from_checkpoint, unsigned n_full, const unsigned *full_nodes,
+                                          unsigned threads, unsigned tile_sites, unsigned *n_nodes,
+                                          unsigned *n_full_out) {
+  RDH_TRY({
+    model_t::ancestral_options_t opts;
+    opts.all_full = n_full == kAncestralAllNodes;
+    if (!opts.all_full && n_full) {
+      if (!full_nodes) throw std::invalid_argument("ancestral_states: full_nodes is NULL");
+      opts.full_nodes.assign(full_nodes, full_nodes + n_full);
+    }
+    opts.threads = threads;
+    opts.tile_sites = tile_sites;
+    if (from_checkpoint) {
+      checkpoint_t  external;
+      checkpoint_t &ckp = checkpoint_prefix ? (external = checkpoint_t::read_only(checkpoint_prefix)) : H(h).checkpoint;
+      H(h).ancestral = H(h).model->ancestral_states(ckp, opts);
+    } else {
+      if (root_id >= H(h).model->tree().root_count()) throw std::invalid_argument("ancestral_states: root id out of range");
+      H(h).ancestral = H(h).model->ancestral_states(RL(h, root_id, ratio), opts);
+    }
+    *n_nodes = (unsigned)H(h).ancestral.clv_index.size();
+    *n_full_out = (unsigned)H(h).ancestral.full.size();
+    return 1;
+  })
+}
+
+// the nodes of the last rdh_model_ancestral_states (capacities: cap nodes, full_cap full nodes): CLV
+// index and parent position per node (-1: the root), the positions of the nodes with full posteriors,
+// the root id and ratio used, and (ops may be NULL, else 8 * cap ints) each node's post-order
+// operation as 8 ints in the field order of rdk_operation_t
+extern "C" int rdh_model_ancestral_nodes(void *h, unsigned cap, unsigned full_cap, unsigned *clv_index, int *parent,
+                                         unsigned *full, unsigned long long *root_id, double *ratio, int *ops) {
+  RDH_TRY({
+    const auto &a = H(h).ancestral;
+    if (a.clv_index.size() > cap || a.full.size() > full_cap) throw std::runtime_error("output buffers too small");
+    for (size_t i = 0; ops && i < a.ops.size(); ++i) {
+      const rdk_operation_t &o = a.ops[i];
+      int                   *v = ops + 8 * i;
+      v[0] = (int)o.parent_clv_index;
+      v[1] = o.parent_scaler_index;
+      v[2] = (int)o.child1_clv_index;
+      v[3] = (int)o.child1_matrix_index;
+      v[4] = o.child1_scaler_index;
+      v[5] = (int)o.child2_clv_index;
+      v[6] = (int)o.child2_matrix_index;
+      v[7] = o.child2_scaler_index;
+    }
+    std::copy(a.clv_index.begin(), a.clv_index.end(), clv_index);
+    std::copy(a.parent.begin(), a.parent.end(), parent);
+    std::copy(a.full.begin(), a.full.end(), full);
+    *root_id = a.root_id;
+    *ratio = a.ratio;
+    return 1;
+  })
+}
+
+// the sorted tip labels below node `node` of the last rdh_model_ancestral_states, one per line
+// (malloc'd; free with rdh_free), NULL if out of range
+extern "C" char *rdh_model_ancestral_clade(void *h, unsigned node) {
+  const auto &a = H(h).ancestral;
+  if (node >= a.clade.size()) {
+    rdh_set_error("ancestral_clade: node out of range");
+    return nullptr;
+  }
+  std::string s;
+  for (const auto &l : a.clade[node]) s += (s.empty() ? "" : "\n") + l;
+  char *out = (char *)malloc(s.size() + 1);
+  if (!out) {
+    rdh_set_error("ancestral_clade: out of memory");
+    return nullptr;
+  }
+  std::memcpy(out, s.c_str(), s.size() + 1);
+  return out;
+}
+
+// partition `part` of the last rdh_model_ancestral_states: map_state and map_prob [node][pattern],
+// posterior [full node][pattern][4], log_norm [node][pattern]; cap = the capacity of map_state, map_prob
+// and log_norm in entries, full_cap that of posterior in doubles; info = {device ms, device bytes,
+// scratch buffers, patterns per tile}.  Patterns = rdh_model_sites(part).
+extern "C" int rdh_model_ancestral_partition(void *h, unsigned part, unsigned long long cap,
+                                             unsigned long long full_cap, unsigned char *map_state, double *map_prob,
+                                             double *posterior, double *log_norm, double *info) {
+  RDH_TRY({
+    const auto &a = H(h).ancestral;
+    if (part >= a.partitions.size()) throw std::invalid_argument("ancestral_partition: partition out of range");
+    const auto &r = a.partitions[part];
+    if (r.map_state.size() > cap || r.posterior.size() > full_cap) throw std::runtime_error("output buffers too small");
+    std::copy(r.map_state.begin(), r.map_state.end(), map_state);
+    std::copy(r.map_prob.begin(), r.map_prob.end(), map_prob);
+    std::copy(r.posterior.begin(), r.posterior.end(), posterior);
+    std::copy(r.log_norm.begin(), r.log_norm.end(), log_norm);
+    info[0] = r.ms;
+    info[1] = (double)r.device_bytes;
+    info[2] = r.scratch;
+    info[3] = r.tile_sites;
+    return 1;
+  })
+}
+
+// the pattern of every column of partition `part` (its columns in the order of its ranges); capacity
+// cap, n_out = the number of columns
+extern "C" int rdh_model_pattern_of_column(void *h, unsigned part, unsigned *out, unsigned cap, unsigned *n_out) {
+  RDH_TRY({
+    if (part >= H(h).msa.size()) throw std::invalid_argument("pattern_of_column: partition out of range");
+    const auto &m = H(h).model->pattern_of_column(part);
+    *n_out = (unsigned)m.size();
+    if (m.size() > cap) throw std::runtime_error("output buffer too small");
+    std::copy(m.begin(), m.end(), out);
     return 1;
   })
 }

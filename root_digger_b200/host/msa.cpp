@@ -194,6 +194,15 @@ void msa_t::compress() {
       w.push_back(_weights[order[i]]);
     }
   }
+  // column -> pattern: the columns of this alignment first, then those it was compressed from
+  std::vector<unsigned> group(L);
+  for (size_t i = 0, g = 0; i < L; ++i) {
+    if (i && (less(order[i - 1], order[i]) || less(order[i], order[i - 1]))) ++g;
+    group[order[i]] = (unsigned)g;
+  }
+  if (_column_pattern.empty()) _column_pattern.assign(group.begin(), group.end());
+  else
+    for (auto &c : _column_pattern) c = group[c];
   std::vector<std::string> out(n);
   for (size_t r = 0; r < n; ++r) {
     out[r].reserve(keep.size());
@@ -201,6 +210,13 @@ void msa_t::compress() {
   }
   _sequences.swap(out);
   _weights.swap(w);
+}
+
+std::vector<unsigned int> msa_t::pattern_of_column() const {
+  if (!_column_pattern.empty()) return _column_pattern;
+  std::vector<unsigned int> id(length());
+  std::iota(id.begin(), id.end(), 0u);
+  return id;
 }
 
 bool msa_t::constiency_check(std::unordered_set<std::string> labels) const {

@@ -40,12 +40,16 @@ public:
   unsigned int       length() const { return _sequences.empty() ? 0u : (unsigned)_sequences[0].size(); }
 
   void compress();
+  // the pattern each column of the alignment this one was built from became (compress merges
+  // identical columns; a partition's columns are in the order of its ranges): [column] -> pattern
+  std::vector<unsigned int> pattern_of_column() const;
   bool constiency_check(std::unordered_set<std::string> labels) const;
   void valid_data() const;
 
 private:
   std::vector<std::string>  _labels, _sequences;
   std::vector<unsigned int> _weights;
+  std::vector<unsigned int> _column_pattern;  // empty: the identity (never compressed)
   const rdk_state_t        *_map;
   unsigned int              _states;
 };
